@@ -18,7 +18,7 @@ At N = 1 the other configurations are measured beside the headline (bounded, eac
   c5 (configs[4]: one GPU's share -- 2048 poses x 65 536 source points vs a 16M-point model, not L2-resident),
   get_matches (row f4), align_batch (rows a1-a5: AlignPoints family over thousands of neighbourhoods), cpu_baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c3|c2|c2g|c5|small]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c3|c2|c2g|c5|small] [--dump-outputs DIR]
 
 --impl reference times the CPU oracle restatement (the reference is MATLAB; MATLAB/Octave are probed and reported, neither
 exists in this image) on a bounded sample of the same workload.
@@ -253,8 +253,9 @@ def time_steps(torch, fn, steps, flush, sync_all):
 
 
 def gpu_workload(P, torch, w, rank, steps, warmup, dist=None, world=1, T0_override=None, do_e2e=True, do_profile=True, opts_kw=None,
-                 inputs=None):
-    """Measurements of one workload on this rank (collectives included when world > 1)."""
+                 inputs=None, keep_outputs=False):
+    """Measurements of one workload on this rank (collectives included when world > 1).  keep_outputs: r["outputs"] holds
+    what the last timed step returned, copied to the host before any untimed step reuses the buffers."""
     from pcreg_b200 import sharded, torch_ops
     dev = torch.device("cuda", torch.cuda.current_device())
     # PCREG_BENCH_SHARD="r/n": measure on ONE GPU the share that rank r of an n-GPU run would get (work-balance check)
@@ -302,6 +303,11 @@ def gpu_workload(P, torch, w, rank, steps, warmup, dist=None, world=1, T0_overri
     t_wall1 = time.time()
     clocks = sampler.stop(t_wall0, t_wall1)
     launches = P.launch_count() - launches0
+    outputs = None
+    if keep_outputs:
+        # T: [H, 16] column-major 4x4 records as pcreg_icp_batch_dev writes them; best: the step's winner index
+        outputs = {k: v.cpu().numpy().astype(np.float64)
+                   for k, v in dict(T=out.T, rmse=out.rmse, n_used=out.n_used, status=out.status, best=h_best).items()}
     ms = float(sum(per_step))
     ms_ranks = [ms / steps]
     if world > 1:
@@ -312,7 +318,7 @@ def gpu_workload(P, torch, w, rank, steps, warmup, dist=None, world=1, T0_overri
         ms = max(ms_ranks) * steps
     rmse_best = float(out.rmse[int(out.best.item())].item())
     r = dict(ms_per_step=ms / steps, q_per_step=H * ns * (w["iters"] + 1), H=H, ns=ns, launches=launches, clocks=clocks,
-             ms_ranks=ms_ranks, rmse_best=rmse_best, nm=model_h.shape[0], per_step_ms=per_step)
+             ms_ranks=ms_ranks, rmse_best=rmse_best, nm=model_h.shape[0], per_step_ms=per_step, outputs=outputs)
     if do_profile:
         # two extra UNTIMED steps: (2) CUDA-event times of the kernels with nothing added to them, (1) exact device-side work
         # counters (atomics inside the kernels) and the phase clocks of the fused kernel
@@ -680,6 +686,9 @@ def main():
                        ("local", "getLocalPoints (row f2) leg"), ("strong", "strong-scaling leg at N > 1"), ("e2e-multi", "single-process multi-device e2e leg at N > 1")):
         ap.add_argument("--no-" + name, action="store_true", help="skip the " + what)
     ap.add_argument("--only", action="store_true", help="headline only (all side legs off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline's last timed step returned (rank 0's share at N > 1) "
+                         "as DIR/<name>.npy in float64, to compare two builds output for output on the same seeded inputs")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -704,7 +713,11 @@ def main():
     P.init(local_rank)
     warmup = max(3, args.warmup)
 
-    r = gpu_workload(P, torch, w, rank, args.steps, warmup, dist, world, do_e2e=(world == 1))
+    r = gpu_workload(P, torch, w, rank, args.steps, warmup, dist, world, do_e2e=(world == 1), keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in r["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     r["roofline"] = roofline_for(w, r)
     sec = r["ms_per_step"] * 1e-3
     value = r["q_per_step"] * world / sec

@@ -1,11 +1,12 @@
 """The reference's own leaf functions under MATLAB / GNU Octave, when an interpreter AND the reference tree are present
 (SURVEY.md section 8c: the only route from "parity unpinned" to pinned for everything beyond estimateTransform).
 
-Neither exists in the build image nor on the GPU box (probed: matlab, octave, octave-cli), so these tests SKIP there with
-the reason printed.  Where both exist they run the UNMODIFIED .m files (quickTF.m, invertTF.m, estimateTransform.m,
-getLocalPoints.m, AlignPoints.m, AlignPoints_KNN.m, AlignPoints_weighted.m -- the last three need `pca` from the
-statistics package) on seeded inputs exchanged as text files, and compare the oracle restatement (CPU test) and the CUDA
-path (gpu test) with what the interpreter returned.  PCREG_REFERENCE_DIR overrides the location of the reference tree."""
+The reference's .m files are not part of this repository: PCREG_REFERENCE_DIR names a checkout of them.  Without it, or
+without an interpreter (probed: matlab, octave, octave-cli), these tests SKIP with the reason printed.  Where both exist
+they run the UNMODIFIED .m files (quickTF.m, invertTF.m, estimateTransform.m, getLocalPoints.m, AlignPoints.m,
+AlignPoints_KNN.m, AlignPoints_weighted.m -- the last three need `pca` from the statistics package) on seeded inputs
+exchanged as text files, and compare the oracle restatement (CPU test) and the CUDA path (gpu test) with what the
+interpreter returned."""
 import os
 import shutil
 import subprocess
@@ -17,7 +18,7 @@ import pytest
 import oracle
 from pcreg_b200 import synth
 
-REF = os.environ.get("PCREG_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("PCREG_REFERENCE_DIR", "")
 
 
 def _interpreter():
@@ -32,8 +33,8 @@ def _need():
     exe, path = _interpreter()
     if not path:
         pytest.skip("no MATLAB / Octave interpreter on this host (probed: octave-cli, octave, matlab)")
-    if not os.path.isfile(os.path.join(REF, "estimateTransform.m")):
-        pytest.skip("reference tree not present at %s (it does not travel to the GPU box)" % REF)
+    if not REF or not os.path.isfile(os.path.join(REF, "estimateTransform.m")):
+        pytest.skip("no reference tree: set PCREG_REFERENCE_DIR to a checkout of the reference's .m files")
     return exe, path
 
 
