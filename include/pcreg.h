@@ -281,12 +281,48 @@ int  pcreg_icp_batch_dev(const pcreg_model* m, const double* d_src, int64_t ns,
                          double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status,
                          int32_t* d_idx, double* d_rmse_hist, int64_t* d_best, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev} or pcreg_nn_search call,
+/* Convergence tolerance: each hypothesis stops once its pose stops changing.
+ * Poses are row-vector T = [R 0; t 1]; update u (1..iters) takes T_{u-1} to T_u = T_{u-1} dT_u.  Its motion is
+ *   dt_u = |t_u - t_{u-1}|_2                                   (model units)
+ *   dr_u = atan2(|v|, (trace(dR) - 1) / 2) * 180 / pi           (degrees; dR = R_{u-1}' R_u is dT_u's rotation block,
+ *          v = (dR32 - dR23, dR13 - dR31, dR21 - dR12) / 2;  not acos, which is inaccurate at small angles)
+ * After update u >= window the hypothesis STOPS when mean(dt) < tol_t and mean(dr) < tol_r_deg over updates
+ * u-window+1 .. u (each mean a left-to-right FP64 sum divided by window; strict compares: a tolerance of 0 never stops,
+ * +inf switches that criterion off).  The stopping update is applied: T_u is the final pose, n_iter = u, converged = 1.
+ * A stopped hypothesis returns exactly what pcreg_icp_batch with iters = n_iter returns for it (T, rmse, n_used, status,
+ * idx, bit for bit); its rmse_hist columns 0..n_iter are that call's and columns n_iter..iters all hold the final rmse.
+ * A degenerate update (status 1) stops the hypothesis too: n_iter = the updates applied before it, converged = 0.
+ * The rule restates the documented 'Tolerance' of MATLAB's pcregistericp (a translation and a rotation difference averaged
+ * over the three most recent iterations); the toolbox is not available to compare against, so parity is UNPINNED. */
+typedef struct {
+    double tol_t;           /* mean translation change, model units                    */
+    double tol_r_deg;       /* mean rotation change, degrees                           */
+    int    window;          /* updates averaged, 1..16                                 */
+} pcreg_icp_stop;
+void pcreg_icp_stop_default(pcreg_icp_stop* s);        /* {0.01, 0.5, 3} */
+/* pcreg_icp_batch / pcreg_icp_batch_dev with the tolerance stop.  Extra optional outputs: n_iter [nhyp] (pose updates
+ * applied) and converged [nhyp] (1 = stopped by the tolerance).  A negative or NaN tolerance or a window outside [1, 16]
+ * returns PCREG_ERR_ARG.  Results do not depend on the device count. */
+int  pcreg_icp_batch_stop(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld,
+                          const double* w_src, const double* T0_16, int64_t nhyp,
+                          const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                          double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx,
+                          double* rmse_hist, int64_t* best, int32_t* n_iter, int32_t* converged);
+int  pcreg_icp_batch_stop_dev(const pcreg_model* m, const double* d_src, int64_t ns,
+                              const double* d_w_src, const double* d_T0_16, int64_t nhyp,
+                              const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                              double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status,
+                              int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
+                              int32_t* d_n_iter, int32_t* d_converged, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
- *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries,
+ *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
+ *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped
+ *   hypotheses and count every pass),
  *   out[3] = (query, model point) pairs evaluated by brute force,
  *   out[4] = update (select + 17-sum + Kabsch) kernel launches, out[5] = their total ms,
- *   out[6] = correspondences reduced;
+ *   out[6] = correspondences reduced (tolerance stop: of the passes run);
  *   grid NN, exact device-side counts: out[7] = model points / out[8] = cell rows visited by the row scan,
  *   out[9] = pyramid nodes popped, out[10] = queries answered from their candidate list, out[11] = queries walked,
  *   out[12] = queries row-scanned, out[13] = list entries read, out[14] = list points gathered,

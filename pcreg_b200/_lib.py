@@ -51,6 +51,10 @@ class IcpOpts(C.Structure):
                 ("thDist2", C.c_double), ("nn", C.c_int), ("reflection_fix", C.c_int)]
 
 
+class IcpStop(C.Structure):
+    _fields_ = [("tol_t", C.c_double), ("tol_r_deg", C.c_double), ("window", C.c_int)]
+
+
 # name -> (restype, argtypes): every symbol include/pcreg.h declares
 SIGNATURES = {
     "pcreg_init": (C.c_int, [c_i32p, C.c_int]),
@@ -91,6 +95,13 @@ SIGNATURES = {
     "pcreg_icp_batch_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
                                       C.POINTER(IcpOpts), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pcreg_icp_stop_default": (None, [C.POINTER(IcpStop)]),
+    "pcreg_icp_batch_stop": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, c_f64p, c_f64p, C.c_int64,
+                                       C.POINTER(IcpOpts), C.POINTER(IcpStop), c_f64p, c_f64p, c_i32p, c_i32p, c_i32p, c_f64p, c_i64p,
+                                       c_i32p, c_i32p]),
+    "pcreg_icp_batch_stop_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+                                           C.POINTER(IcpOpts), C.POINTER(IcpStop), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pcreg_set_profiling": (C.c_int, [C.c_int]),
     "pcreg_last_profile": (C.c_int, [c_f64p]),
 }

@@ -14,7 +14,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib as L
-from ._lib import AlignOpts, DescOpts, IcpOpts, MatchOpts, ModelOpts, PcregError, RansacOpts  # noqa: F401
+from ._lib import AlignOpts, DescOpts, IcpOpts, IcpStop, MatchOpts, ModelOpts, PcregError, RansacOpts  # noqa: F401
 
 NN_BRUTE, NN_GRID = 0, 1
 ICP_PLAIN, ICP_KNN, ICP_WEIGHTED = 0, 1, 2
@@ -482,10 +482,18 @@ def icp_opts(mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, nn=NN_
     return IcpOpts(int(mode), int(iters), float(k_frac), float(R_w), float(thDist2), int(nn), int(bool(reflection_fix)))
 
 
+def icp_stop(tol_t, tol_r_deg, window=3) -> IcpStop:
+    return IcpStop(float(tol_t), float(tol_r_deg), int(window))
+
+
 def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src=None,
-              nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False):
+              nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3):
     """Multi-start ICP of `src` against the resident `model` from the initial poses T0s [H,4,4].
-    Returns dict(T [H,4,4], rmse [H], n_used [H], status [H], best, idx [H,ns]?, rmse_hist [H,iters+1]?)."""
+    Returns dict(T [H,4,4], rmse [H], n_used [H], status [H], best, idx [H,ns]?, rmse_hist [H,iters+1]?).
+
+    tolerance=(tol_t, tol_r_deg): each hypothesis stops once the mean translation change (model units) and the mean
+    rotation change (degrees) of its last `window` updates are both below these (include/pcreg.h: pcreg_icp_stop); the
+    result then also holds n_iter [H] (pose updates applied) and converged [H] (1 = stopped by the tolerance)."""
     a, is_double, ns = _cm_points(src)
     T0 = _T_to_abi(np.asarray(T0s, dtype=np.float64).reshape(-1, 4, 4))
     H = T0.shape[0]
@@ -498,11 +506,21 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
     idx = np.empty((H, ns), dtype=np.int32) if return_idx else None
     hist = np.empty((H, iters + 1), dtype=np.float64) if return_hist else None
     best = C.c_int64()
-    L.check(L.lib().pcreg_icp_batch(model.handle, a.ctypes.data_as(C.c_void_p), is_double, ns, ns, _ptr(w, L.c_f64p),
-                                    _ptr(T0, L.c_f64p), H, C.byref(o), _ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p),
-                                    _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p),
-                                    _ptr(hist, L.c_f64p), C.byref(best)), "pcreg_icp_batch")
+    args = (model.handle, a.ctypes.data_as(C.c_void_p), is_double, ns, ns, _ptr(w, L.c_f64p), _ptr(T0, L.c_f64p), H, C.byref(o))
+    outs = (_ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p), _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p),
+            _ptr(hist, L.c_f64p), C.byref(best))
+    if tolerance is None:
+        L.check(L.lib().pcreg_icp_batch(*args, *outs), "pcreg_icp_batch")
+    else:
+        n_iter = np.empty(H, dtype=np.int32)
+        converged = np.empty(H, dtype=np.int32)
+        stop = icp_stop(tolerance[0], tolerance[1], window)
+        L.check(L.lib().pcreg_icp_batch_stop(*args, C.byref(stop), *outs, _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)),
+                "pcreg_icp_batch_stop")
     out = dict(T=_T_from_abi(T, H), rmse=rmse, n_used=n_used, status=status, best=int(best.value))
+    if tolerance is not None:
+        out["n_iter"] = n_iter
+        out["converged"] = converged
     if return_idx:
         out["idx"] = idx
     if return_hist:

@@ -33,7 +33,8 @@ struct Pose16 { double t[16]; };      // a row-major row-vector pose as a kernel
 // One block per hypothesis.
 // NT = threads per hypothesis: UPD_THREADS (the fused kernel's count, so that both sum in the same order and agree bit for
 // bit) for sources the fused kernel can take, 512 for large sources (C5: 65 536 correspondences per hypothesis).
-template <int NT>
+// STOP = the tolerance stop (a.stop_iter set); the STOP = false instantiations are the loop without it.
+template <int NT, bool STOP>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __grid_constant__ IcpUpdateArgs a) {
     __shared__ double Ts[16];
     __shared__ double red[KABSCH_NSUMS * 32];
@@ -44,6 +45,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
     const int64_t h = blockIdx.x;
     const int tid = threadIdx.x;
     const int64_t ns = a.ns;
+    if (STOP && a.update && a.stop_iter[h] >= 0) return;       // stopped: intermediate passes leave it alone
     if (tid < 16) Ts[tid] = a.T[h * 16 + tid];
     __syncthreads();
     const int32_t* __restrict__ idx = a.idx + h * ns;
@@ -163,13 +165,23 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
         const double rmse = (sw > 0.0) ? sqrt(s[16] / sw) : nan("");
         a.rmse[h] = rmse;
         a.n_used[h] = (int32_t)n_used;
-        if (a.rmse_hist) a.rmse_hist[h * a.hist_stride + a.hist_col] = rmse;
+        int hist_from = a.hist_col;
+        if (STOP && !a.update) {
+            // final pass: a hypothesis stopped after k updates would have had its final pass at column k (converged) or k + 1
+            // (frozen at pass k); every column from there holds the final rmse
+            const int k = a.stop_iter[h];
+            if (k >= 0) hist_from = k + a.frozen[h];
+            if (a.n_iter) a.n_iter[h] = k >= 0 ? k : a.hist_col;
+            if (a.converged) a.converged[h] = k >= 0 && !a.frozen[h];
+        }
+        if (a.rmse_hist) for (int c = hist_from; c <= a.hist_col; ++c) a.rmse_hist[h * a.hist_stride + c] = rmse;
         float moved = 0.f;
         if (a.update && !a.frozen[h]) {
             double Tn[16], Tc[16];
             for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
             if (!icp_pose_update_call(s, n_used, a.pivot, a.reflection_fix != 0, Tc, Tn)) {
                 a.frozen[h] = 1;
+                if (STOP) a.stop_iter[h] = a.hist_col;
             } else {
                 for (int k = 0; k < 16; ++k) a.T[h * 16 + k] = Tn[k];
                 if (a.delta) {
@@ -186,6 +198,11 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
                     }
                     const double dl = sqrt(fro) * a.src_stats[3] + sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
                     moved = __double2float_ru(dl * (1.0 + 1e-9)) + 1e-30f;
+                }
+                // stopped: the pose no longer moves.  The passes up to the final one compute nothing this hypothesis uses.
+                if (STOP && icp_stop_update(a.stop, Tc, Tn, a.hist_col + 1, a.stop_ring + h * (2 * ICP_STOP_WINDOW_MAX))) {
+                    a.stop_iter[h] = a.hist_col + 1;
+                    moved = 0.f;
                 }
             }
         }
@@ -372,8 +389,10 @@ void transpose16_launch(const double* d_in, double* d_out, int64_t n, cudaStream
     PCREG_LAUNCHED();
 }
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
-    if (a.ns > 20000) k_icp_update<512><<<(unsigned)nhyp, 512, 0, st>>>(a);
-    else              k_icp_update<UPD_THREADS><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    const bool stop = a.stop_iter != nullptr;
+    if (a.ns > 20000) { if (stop) k_icp_update<512, true><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false><<<(unsigned)nhyp, 512, 0, st>>>(a); }
+    else if (stop)    k_icp_update<UPD_THREADS, true><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    else              k_icp_update<UPD_THREADS, false><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
     PCREG_LAUNCHED();
 }
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st) {
@@ -390,7 +409,8 @@ static bool debug_times() { static int v = -1; if (v < 0) { const char* e = gete
 static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3, ld = ns*/, int64_t ns,
                     const double* d_w, const double* d_T0_cm, int64_t nhyp, const pcreg_icp_opts& o,
                     double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
-                    double* d_rmse_hist, int64_t* d_best, cudaStream_t st) {
+                    double* d_rmse_hist, int64_t* d_best, cudaStream_t st,
+                    const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr) {
     PCREG_REQUIRE(m && d_src && d_T0_cm && d_T16_cm, "icp: null pointer");
     PCREG_REQUIRE(ns >= 1 && nhyp >= 1, "icp: need ns >= 1 and nhyp >= 1");
     PCREG_REQUIRE(o.iters >= 0, "icp: iters must be >= 0");
@@ -430,6 +450,22 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     DevBuf<double> rmse_tmp(d_rmse ? 0 : (size_t)nhyp);
     DevBuf<int32_t> nused_tmp(d_n_used ? 0 : (size_t)nhyp);
     DevBuf<unsigned long long> counters(16);
+    IcpStopRule rule{};
+    if (stop) { rule.tol_t = stop->tol_t; rule.tol_r_deg = stop->tol_r_deg; rule.window = stop->window; }
+    // tolerance stop, per-pass path: per-hypothesis stop state (the fused kernel keeps it in shared memory)
+    DevBuf<int32_t> stop_iter(stop && !fused ? (size_t)nhyp : 0);
+    DevBuf<double> stop_ring(stop && !fused ? (size_t)nhyp * 2 * ICP_STOP_WINDOW_MAX : 0);
+    // profiling with the tolerance stop: the passes each hypothesis ran follow from n_iter and status
+    DevBuf<int32_t> n_iter_tmp(stop && prof && !d_n_iter ? (size_t)nhyp : 0);
+    if (n_iter_tmp.p) d_n_iter = n_iter_tmp.p;
+    auto passes_run = [&]() -> double {       // after the stream has drained
+        std::vector<int32_t> ni((size_t)nhyp), fz((size_t)nhyp);
+        PCREG_CUDA(cudaMemcpy(ni.data(), d_n_iter, ni.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        PCREG_CUDA(cudaMemcpy(fz.data(), frozen.p, fz.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+        double n = 0.0;
+        for (int64_t h = 0; h < nhyp; ++h) n += (double)ni[h] + 1.0 + (double)fz[h];   // frozen at pass p: n_iter = p, p + 2 passes
+        return n;
+    };
     // candidate lists (grid NN, nn_grid.cu): built by the full searches once a pose has nearly stopped moving,
     // scanned instead of searching while the query stays inside its list's guarantee.  PCREG_LISTS=0 disables.
     static const bool lists_on = [] { const char* e = getenv("PCREG_LISTS"); return !(e && e[0] == '0'); }();
@@ -478,6 +514,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
 
     PCREG_CUDA(cudaMemsetAsync(frozen.p, 0, frozen.bytes(), st));
     PCREG_CUDA(cudaMemsetAsync(counters.p, 0, counters.bytes(), st));
+    if (stop_iter.p) PCREG_CUDA(cudaMemsetAsync(stop_iter.p, 0xff, stop_iter.bytes(), st));      // -1: running
     transpose16_launch(d_T0_cm, Twork.p, nhyp, st);
 
     std::vector<EventPair> evs;
@@ -520,8 +557,9 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         fa.idx_out = d_idx; fa.perm = sorted ? sperm.p : nullptr; fa.tie_order = sorted ? sinv.p : nullptr;
         fa.mode = o.mode; fa.k_frac = o.k_frac; fa.R_w = o.R_w; fa.thDist2 = o.thDist2; fa.reflection_fix = o.reflection_fix; fa.iters = o.iters;
         fa.counters = (prof && c.profiling_counters) ? counters.p : nullptr;
+        fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged;
         ev_begin(0);
-        icp_fused_launch(fa, nhyp, st);
+        icp_fused_launch(fa, nhyp, stop != nullptr, st);
         ev_end();
         transpose16_launch(Twork.p, d_T16_cm, nhyp, st);
         if (d_status) PCREG_CUDA(cudaMemcpyAsync(d_status, frozen.p, (size_t)nhyp * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
@@ -532,7 +570,8 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
             PCREG_CUDA(cudaEventElapsedTime(&ms, evs[0].a, evs[0].b));
             unsigned long long hcnt[16] = {0};
             PCREG_CUDA(cudaMemcpy(hcnt, counters.p, sizeof hcnt, cudaMemcpyDeviceToHost));
-            const double nq = (double)nhyp * (double)ns * (double)(o.iters + 1);
+            // with the tolerance stop a block runs as many passes as its hypothesis needs
+            const double nq = (double)ns * (stop ? passes_run() : (double)nhyp * (double)(o.iters + 1));
             c.profile[0] = 1; c.profile[1] = ms; c.profile[2] = nq; c.profile[6] = nq;
             c.profile[11] = (double)hcnt[4]; c.profile[10] = nq - (double)hcnt[4];
             c.profile[13] = (double)hcnt[6]; c.profile[14] = (double)hcnt[7];
@@ -594,7 +633,8 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                 else
                     nn_grid_launch(m, sx, sy, sz, ns, Twork.p + h0 * 16, hn, L.have_prev ? L.prev : nullptr, out_idx, L.d2.p,
                                    (prof && c.profiling_counters) ? counters.p : nullptr, L.gscratch, use_lists ? &L.cl : nullptr, it >= 2,
-                                   (lazy_trim && it >= 2 && !last) ? skip_thr.p + h0 : nullptr, ls);
+                                   (lazy_trim && it >= 2 && !last) ? skip_thr.p + h0 : nullptr, ls,
+                                   (stop && !last) ? stop_iter.p + h0 : nullptr);
                 ev_end();
                 nn_launches += 1;
                 IcpUpdateArgs ua{};
@@ -611,6 +651,10 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                 ua.frozen = frozen.p + h0; ua.rmse = rm + h0; ua.n_used = nu + h0;
                 ua.rmse_hist = d_rmse_hist ? d_rmse_hist + h0 * (o.iters + 1) : nullptr;
                 ua.hist_stride = o.iters + 1; ua.hist_col = it;
+                if (stop) {
+                    ua.stop_iter = stop_iter.p + h0; ua.stop_ring = stop_ring.p + h0 * 2 * ICP_STOP_WINDOW_MAX; ua.stop = rule;
+                    ua.n_iter = d_n_iter ? d_n_iter + h0 : nullptr; ua.converged = d_converged ? d_converged + h0 : nullptr;
+                }
                 ev_begin(1);
                 icp_update_launch(ua, hn, ls);
                 ev_end();
@@ -661,9 +705,13 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
             c.profile[20 + marks[k].kind] += 1.0;
         }
         const double nq = (double)nhyp * (double)ns * (double)(o.iters + 1);
-        c.profile[0] = nn_launches; c.profile[1] = nn_ms; c.profile[2] = nq;
+        // with the tolerance stop, the update kernel and the voxel-map NN kernel skip a stopped hypothesis until the final
+        // pass; the brute-force and map-less grid NN kernels still search for it
+        const double nq_run = stop ? (double)ns * passes_run() : nq;
+        const bool vox_nn = o.nn == PCREG_NN_GRID && m->has_vox;
+        c.profile[0] = nn_launches; c.profile[1] = nn_ms; c.profile[2] = vox_nn ? nq_run : nq;
         c.profile[3] = (o.nn == PCREG_NN_BRUTE) ? nq * (double)m->n : 0.0;
-        c.profile[4] = upd_launches; c.profile[5] = upd_ms; c.profile[6] = nq;
+        c.profile[4] = upd_launches; c.profile[5] = upd_ms; c.profile[6] = nq_run;
         c.profile[7] = (double)hcnt[0]; c.profile[8] = (double)hcnt[1]; c.profile[9] = (double)hcnt[2];
         c.profile[26] = (o.nn == PCREG_NN_GRID && m->has_vox) ? 1.0 : 0.0;
     }
@@ -690,6 +738,17 @@ void pcreg_icp_opts_default(pcreg_icp_opts* o) {
     o->nn = PCREG_NN_BRUTE; o->reflection_fix = 0;
 }
 
+void pcreg_icp_stop_default(pcreg_icp_stop* s) {
+    if (!s) return;
+    s->tol_t = 0.01; s->tol_r_deg = 0.5; s->window = 3;
+}
+
+static void check_stop(const pcreg_icp_stop* s) {
+    PCREG_REQUIRE(s, "icp stop: null pointer");
+    PCREG_REQUIRE(s->tol_t >= 0.0 && s->tol_r_deg >= 0.0, "icp stop: tolerances must be >= 0 (NaN is rejected; +inf disables one)");
+    PCREG_REQUIRE(s->window >= 1 && s->window <= ICP_STOP_WINDOW_MAX, "icp stop: window must be in [1, 16]");
+}
+
 int pcreg_icp_batch_dev(const pcreg_model* m, const double* d_src, int64_t ns, const double* d_w_src,
                         const double* d_T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* d_T16,
                         double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist,
@@ -704,34 +763,54 @@ int pcreg_icp_batch_dev(const pcreg_model* m, const double* d_src, int64_t ns, c
     PCREG_API_END
 }
 
+int pcreg_icp_batch_stop_dev(const pcreg_model* m, const double* d_src, int64_t ns, const double* d_w_src,
+                             const double* d_T0_16, int64_t nhyp, const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                             double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
+                             double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    PCREG_REQUIRE(opts, "pcreg_icp_batch_stop_dev: opts is null");
+    check_stop(stop);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    icp_run(m, d_src, ns, d_w_src, d_T0_16, nhyp, *opts, d_T16, d_rmse, d_n_used, d_status, d_idx, d_rmse_hist,
+            d_best, (cudaStream_t)stream, stop, d_n_iter, d_converged);
+    return PCREG_OK;
+    PCREG_API_END
+}
+
 // One device's share [h0, h0 + hn) of a host-buffer batch, on the calling thread's slot.  Output pointers are the caller's
 // arrays (whole batch); every copy lands in its own contiguous slice, which is the "all-gather" of SURVEY.md section 8e.
 static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>& hs, int64_t ns, const double* w_src,
                                  const double* T0_16, int64_t h0, int64_t hn, const pcreg_icp_opts& o, double* T16, double* rmse,
-                                 int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist) {
+                                 int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                                 const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged) {
     PCREG_CUDA(cudaSetDevice(ctx().device));
     cudaStream_t st = 0;
     DevBuf<double> d_src((size_t)ns * 3), d_w(w_src ? (size_t)ns : 0), d_T0((size_t)hn * 16), d_T((size_t)hn * 16);
     DevBuf<double> d_rmse((size_t)hn), d_hist(rmse_hist ? (size_t)hn * (o.iters + 1) : 0);
     DevBuf<int32_t> d_nu((size_t)hn), d_st((size_t)hn), d_idx(idx ? (size_t)hn * ns : 0);
+    DevBuf<int32_t> d_nit(n_iter ? (size_t)hn : 0), d_conv(converged ? (size_t)hn : 0);
     PCREG_CUDA(cudaMemcpyAsync(d_src.p, hs.data(), d_src.bytes(), cudaMemcpyHostToDevice, st));
     if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src, d_w.bytes(), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
     icp_run(m, d_src.p, ns, w_src ? d_w.p : nullptr, d_T0.p, hn, o, d_T.p, d_rmse.p, d_nu.p, d_st.p,
-            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st);
+            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st, stop, d_nit.p, d_conv.p);
     PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
     if (status) PCREG_CUDA(cudaMemcpyAsync(status + h0, d_st.p, d_st.bytes(), cudaMemcpyDeviceToHost, st));
     if (idx) PCREG_CUDA(cudaMemcpyAsync(idx + h0 * ns, d_idx.p, d_idx.bytes(), cudaMemcpyDeviceToHost, st));
     if (rmse_hist) PCREG_CUDA(cudaMemcpyAsync(rmse_hist + h0 * (o.iters + 1), d_hist.p, d_hist.bytes(), cudaMemcpyDeviceToHost, st));
+    if (n_iter) PCREG_CUDA(cudaMemcpyAsync(n_iter + h0, d_nit.p, d_nit.bytes(), cudaMemcpyDeviceToHost, st));
+    if (converged) PCREG_CUDA(cudaMemcpyAsync(converged + h0, d_conv.p, d_conv.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaStreamSynchronize(st));
 }
 
-int pcreg_icp_batch(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
-                    const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* T16, double* rmse,
-                    int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist, int64_t* best) {
-    PCREG_API_BEGIN
+// pcreg_icp_batch and pcreg_icp_batch_stop (stop != nullptr)
+static int icp_batch_host(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
+                          const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* T16, double* rmse,
+                          int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist, int64_t* best,
+                          const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged) {
     require_init();
     PCREG_REQUIRE(m && src && T0_16 && T16 && opts, "pcreg_icp_batch: null pointer");
     PCREG_REQUIRE(ns >= 1 && ld >= ns && nhyp >= 1, "pcreg_icp_batch: bad sizes");
@@ -749,10 +828,12 @@ int pcreg_icp_batch(const pcreg_model* m, const void* src, int is_double, int64_
         const int64_t h0 = k * per, hn = std::min(per, nhyp - h0);
         if (hn <= 0) continue;
         workers.emplace_back([&, k, h0, hn]() {
-            rc[k] = guarded([&]() { use_slot(k); icp_batch_host_slice(m->on_slot(k), hs, ns, w_src, T0_16, h0, hn, *opts, T16, rm, n_used, status, idx, rmse_hist); });
+            rc[k] = guarded([&]() { use_slot(k); icp_batch_host_slice(m->on_slot(k), hs, ns, w_src, T0_16, h0, hn, *opts, T16, rm, n_used, status, idx, rmse_hist,
+                                                                 stop, n_iter, converged); });
         });
     }
-    rc[0] = guarded([&]() { use_slot(0); icp_batch_host_slice(m, hs, ns, w_src, T0_16, 0, std::min(per, nhyp), *opts, T16, rm, n_used, status, idx, rmse_hist); });
+    rc[0] = guarded([&]() { use_slot(0); icp_batch_host_slice(m, hs, ns, w_src, T0_16, 0, std::min(per, nhyp), *opts, T16, rm, n_used, status, idx, rmse_hist,
+                                                         stop, n_iter, converged); });
     for (auto& w : workers) w.join();
     use_slot(0);
     for (int k = 0; k < nd; ++k) if (rc[k] != PCREG_OK) return rc[k];
@@ -762,6 +843,25 @@ int pcreg_icp_batch(const pcreg_model* m, const void* src, int is_double, int64_
         *best = bi;
     }
     return PCREG_OK;
+}
+
+int pcreg_icp_batch(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
+                    const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* T16, double* rmse,
+                    int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist, int64_t* best) {
+    PCREG_API_BEGIN
+    return icp_batch_host(m, src, is_double, ns, ld, w_src, T0_16, nhyp, opts, T16, rmse, n_used, status, idx, rmse_hist, best,
+                          nullptr, nullptr, nullptr);
+    PCREG_API_END
+}
+
+int pcreg_icp_batch_stop(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
+                         const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                         double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                         int64_t* best, int32_t* n_iter, int32_t* converged) {
+    PCREG_API_BEGIN
+    check_stop(stop);
+    return icp_batch_host(m, src, is_double, ns, ld, w_src, T0_16, nhyp, opts, T16, rmse, n_used, status, idx, rmse_hist, best,
+                          stop, n_iter, converged);
     PCREG_API_END
 }
 

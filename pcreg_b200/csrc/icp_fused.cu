@@ -54,9 +54,21 @@ __device__ __noinline__ bool fused_pose_update(const double (&s)[KABSCH_NSUMS], 
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return true;
 }
+// Tolerance stop: the update of pass `it` (update it + 1) and the stop rule.  0: degenerate, pose left alone; 1: pose updated;
+// 2: pose updated and the rule says stop.
+__device__ __noinline__ int fused_pose_update_stop(const double (&s)[KABSCH_NSUMS], long long n_used, const double* pivot, bool reflection_fix,
+                                                   const IcpStopRule& rule, int it, double* ring /*shared*/, double* Ts /*shared*/) {
+    double Tc[16], Tn[16];
+    for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
+    if (!icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
+    for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
+    return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
+}
 
 // KNN = the trimmed mode (its selection scratch -- 18 KB of shared memory -- exists only in that instantiation).
-template <bool KNN>
+// STOP = the tolerance stop (pcreg_icp_batch_stop): a stop -- by the rule or by a degenerate update -- makes the block's next
+// pass its final scoring pass, after which the block exits.  The STOP = false instantiations are the loop without it.
+template <bool KNN, bool STOP>
 __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ FusedArgs a) {
     extern __shared__ __align__(16) unsigned char dyn[];
     __shared__ double Ts[16];
@@ -65,6 +77,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     __shared__ HistSelShared hsel;
     __shared__ unsigned long long red_u64[64];
     __shared__ int s_frozen;
+    __shared__ int s_stop;                                  // STOP: the next pass is the final one
+    __shared__ double s_ring[2 * ICP_STOP_WINDOW_MAX];      // STOP: thread 0's window of update motions
 
     const int ns = a.ns;
     int32_t* __restrict__ idx_s = (int32_t*)dyn;
@@ -82,11 +96,11 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     const bool timing = a.counters != nullptr && tid == 0;
 
     if (tid < 16) Ts[tid] = a.T[h * 16 + tid];
-    if (tid == 0) s_frozen = a.frozen[h];
+    if (tid == 0) { s_frozen = a.frozen[h]; if (STOP) s_stop = 0; }
     __syncthreads();
 
     for (int it = 0; it <= a.iters; ++it) {
-        const bool last = it == a.iters;
+        const bool last = it == a.iters || (STOP && s_stop);     // block-uniform: s_stop was written before the last barrier
         // ---- exact nearest neighbours of the hypothesis' ns queries (two per trip: their header / entry loads overlap) ----
         long long nkept = 0;
         unsigned long long kmin = ~0ull, kmax = 0ull;
@@ -204,14 +218,29 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
         if (tid == 0) {
             const double sw = s[0];
             const double rmse = (sw > 0.0) ? sqrt(s[16] / sw) : nan("");
-            if (a.rmse_hist) a.rmse_hist[h * a.hist_stride + it] = rmse;
+            if (a.rmse_hist) {
+                if (STOP && last) { for (int c = it; c <= a.iters; ++c) a.rmse_hist[h * a.hist_stride + c] = rmse; }
+                else a.rmse_hist[h * a.hist_stride + it] = rmse;
+            }
             if (last) { a.rmse[h] = rmse; a.n_used[h] = (int32_t)n_used; }
+            if (STOP && last) {
+                // a degenerate update at pass p applied p updates and ends the loop with pass p + 1
+                if (a.n_iter) a.n_iter[h] = it - s_frozen;
+                if (a.converged) a.converged[h] = s_stop && !s_frozen;
+            }
             if (!last && !s_frozen) {
-                if (!fused_pose_update(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
+                if (!STOP) {
+                    if (!fused_pose_update(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
+                } else {
+                    const int r = fused_pose_update_stop(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
+                    if (r == 0) s_frozen = 1;
+                    if (r != 1) s_stop = 1;
+                }
             }
         }
         if (timing) { const long long t = clock64(); t_svd += t - t_mark; t_mark = t; }
         __syncthreads();
+        if (STOP && last) break;
     }
     if (tid < 16) a.T[h * 16 + tid] = Ts[tid];
     if (tid == 0) a.frozen[h] = s_frozen;
@@ -250,19 +279,23 @@ bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pc
     if (nhyp < ctx().sm_count) return false;
     if (ns >= ((int64_t)1 << 30)) return false;
     cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, k_icp_fused<true>) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (cudaFuncGetAttributes(&fa, k_icp_fused<true, false>) != cudaSuccess) { cudaGetLastError(); return false; }
     return icp_fused_smem(ns, o.mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
 }
 
-void icp_fused_launch(FusedArgs& a, int64_t nhyp, cudaStream_t st) {
+template <bool KNN, bool STOP>
+static void fused_launch_one(const FusedArgs& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
+    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    k_icp_fused<KNN, STOP><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+}
+
+void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
-    if (a.mode == PCREG_ICP_KNN) {
-        PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-        k_icp_fused<true><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
-    } else {
-        PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-        k_icp_fused<false><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
-    }
+    const bool knn = a.mode == PCREG_ICP_KNN;
+    if (knn && !stop)       fused_launch_one<true, false>(a, nhyp, dyn, st);
+    else if (!knn && !stop) fused_launch_one<false, false>(a, nhyp, dyn, st);
+    else if (knn)           fused_launch_one<true, true>(a, nhyp, dyn, st);
+    else                    fused_launch_one<false, true>(a, nhyp, dyn, st);
     PCREG_LAUNCHED();
 }
 

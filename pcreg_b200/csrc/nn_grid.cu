@@ -768,7 +768,7 @@ __global__ void __launch_bounds__(32 * WW_WARPS, 6) k_nn_grid_walk_warp(const __
 void nn_grid_launch(const pcreg_model* m, const double* d_sx, const double* d_sy, const double* d_sz, int64_t ns,
                     const double* d_T, int64_t nhyp, const int32_t* d_prev, int32_t* d_idx, double* d_d2,
                     unsigned long long* d_counters, GridScratch& sc, const CandView* cl, bool scan_lists, const double* d_skip_thr,
-                    cudaStream_t st) {
+                    cudaStream_t st, const int32_t* d_stop_iter) {
     PCREG_REQUIRE(m->has_grid, "grid NN requested but the model was created without build_grid");
     GridArgs a{};
     a.g = m->grid; a.md = m->md.p;
@@ -801,6 +801,7 @@ void nn_grid_launch(const pcreg_model* m, const double* d_sx, const double* d_sy
         // Voronoi voxel map (nn_vox.cu): one list scan per query; the few queries whose voxel has no list (or that lie outside
         // the padded box) are walked, warm-started by the previous correspondence when there is one.
         a.vox = m->vox;
+        a.stop_iter = d_stop_iter;
         if (sc.worklist.n < (size_t)a.nq) sc.worklist.alloc((size_t)a.nq);
         if (sc.count.n < 2) sc.count.alloc(2);
         PCREG_CUDA(cudaMemsetAsync(sc.count.p, 0, 2 * sizeof(unsigned int), st));

@@ -362,15 +362,20 @@ __global__ void __launch_bounds__(256) k_vox_refine(const __grid_constant__ VoxL
 
 // ---- query --------------------------------------------------------------------------------------------------------------
 // One thread per query.  counters (profiling): [3] queries answered here, [6] entries read, [7] points gathered for the
-// FP64 decision; queries without a list are appended to the work list of the pyramid walk.
+// FP64 decision; queries without a list are appended to the work list of the pyramid walk.  The queries of a hypothesis the
+// tolerance stop has stopped (a.stop_iter[h] >= 0) are neither answered nor handed to the walk: they carry their previous
+// correspondence forward (a stop happens at an update, so every pass after one has a.prev), which keeps every
+// correspondence buffer a valid warm start for the final pass; their d2 stays stale (nothing reads it before the final pass).
 __global__ void __launch_bounds__(256) k_nn_vox(const __grid_constant__ GridArgs a) {
     const VoxView& V = a.vox;
     const int lane = threadIdx.x & 31;
     const int64_t gq = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     bool defer = false;
     unsigned long long n_read = 0, n_gather = 0, n_done = 0;
-    if (gq < a.nq) {
-        const unsigned h = (unsigned)gq / (unsigned)a.ns, i = (unsigned)gq - h * (unsigned)a.ns;
+    const unsigned h = (unsigned)gq / (unsigned)a.ns, i = (unsigned)gq - h * (unsigned)a.ns;
+    if (gq < a.nq && a.stop_iter && a.prev && a.stop_iter[h] >= 0) {
+        a.idx[gq] = a.prev[gq];
+    } else if (gq < a.nq) {
         double qx, qy, qz;
         quick_tf(a.T + (size_t)h * 16, a.sx[i], a.sy[i], a.sz[i], qx, qy, qz);
         uint2 hd;

@@ -18,6 +18,7 @@ struct GridArgs {
     VoxView vox;                    // Voronoi voxel map of the model (nn_vox.cu; vox.hdr == nullptr: none)
     CandView cl;                    // candidate lists of the chunk (cl.cnt == nullptr: disabled)
     const double* skip_thr;         // [nhyp] or null: list kernel skips queries whose previous residual exceeds it (lazy trimming)
+    const int32_t* stop_iter;       // [nhyp] or null: the voxel-map kernel skips the queries of hypotheses with stop_iter >= 0
     const int32_t* in_list;         // direct kernel: the queries to process (nullptr: all nq)
     const unsigned int* in_count;   //                and how many
     int32_t* worklist;              // [nq] query ids handed to the next kernel (list -> direct -> walk)
@@ -49,10 +50,12 @@ struct FusedArgs {
     const int32_t* tie_order;   // [ns] (sorted) position of original index (stable tie rule of the trim), or null
     int mode; double k_frac, R_w, thDist2; int reflection_fix; int iters;
     unsigned long long* counters;           // profiling (may be null): [4] queries walked, [6] list entries read, [7] points gathered
+    IcpStopRule stop;                       // tolerance stop (the k_icp_fused<*, true> instantiations only)
+    int32_t* n_iter; int32_t* converged;    // [nhyp] optional outputs of the tolerance stop
 };
 size_t icp_fused_smem(int64_t ns, int mode);
 bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o);
-void icp_fused_launch(FusedArgs& a, int64_t nhyp, cudaStream_t st);
+void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
 
 __device__ __forceinline__ void flush_counters(unsigned long long* counters, unsigned long long n_pts,
                                                unsigned long long n_cells, unsigned long long n_nodes, int i_pts = 0, int i_cells = 1,

@@ -60,4 +60,29 @@ __device__ __noinline__ static bool icp_pose_update_call(const double (&s)[KABSC
     return icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn);
 }
 
+// Tolerance stop (pcreg_icp_stop, include/pcreg.h).  Update u (1-based) took Tc = T_{u-1} to Tn = T_u = T_{u-1} dT.  Its motion
+//   dt_u = |t_u - t_{u-1}|                                   (translation rows)
+//   dr_u = atan2(|v|, (trace dR - 1) / 2) in degrees,  dR = R_{u-1}' R_u,  v = (dR32 - dR23, dR13 - dR31, dR21 - dR12) / 2
+// goes to slot (u-1) % window of the ring (dt in ring[0..15], dr in ring[16..31]).  Once u >= window, returns true when the
+// means of the last `window` updates (left-to-right FP64 sums over u-window+1 .. u, divided by window) are both strictly below
+// their tolerances.  Both ICP paths call this one function, so the fused and the per-pass kernels stop at the same update.
+__device__ __noinline__ static bool icp_stop_update(const IcpStopRule& r, const double* Tc, const double* Tn, int u, double* ring) {
+    double dR[9];
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j)
+            dR[i * 3 + j] = Tc[0 * 4 + i] * Tn[0 * 4 + j] + Tc[1 * 4 + i] * Tn[1 * 4 + j] + Tc[2 * 4 + i] * Tn[2 * 4 + j];
+    const double v0 = 0.5 * (dR[7] - dR[5]), v1 = 0.5 * (dR[2] - dR[6]), v2 = 0.5 * (dR[3] - dR[1]);
+    const double c = 0.5 * (dR[0] + dR[4] + dR[8] - 1.0);
+    const double dr = atan2(sqrt(v0 * v0 + v1 * v1 + v2 * v2), c) * (180.0 / 3.14159265358979323846);
+    const double x = Tn[12] - Tc[12], y = Tn[13] - Tc[13], z = Tn[14] - Tc[14];
+    const double dt = sqrt(x * x + y * y + z * z);
+    const int w = r.window;
+    ring[(u - 1) % w] = dt;
+    ring[ICP_STOP_WINDOW_MAX + (u - 1) % w] = dr;
+    if (u < w) return false;
+    double st = 0.0, sr = 0.0;
+    for (int k = u - w; k < u; ++k) { st += ring[k % w]; sr += ring[ICP_STOP_WINDOW_MAX + k % w]; }
+    return st / (double)w < r.tol_t && sr / (double)w < r.tol_r_deg;
+}
+
 }  // namespace pcreg

@@ -241,7 +241,12 @@ struct GridScratch {
 void nn_grid_launch(const pcreg_model* m, const double* d_sx, const double* d_sy, const double* d_sz,
                     int64_t ns, const double* d_T, int64_t nhyp, const int32_t* d_prev,
                     int32_t* d_idx, double* d_d2, unsigned long long* d_visit_counters, GridScratch& scratch,
-                    const CandView* cl, bool scan_lists, const double* d_skip_thr /*[nhyp] or null: lazy trimming*/, cudaStream_t st);
+                    const CandView* cl, bool scan_lists, const double* d_skip_thr /*[nhyp] or null: lazy trimming*/, cudaStream_t st,
+                    const int32_t* d_stop_iter = nullptr /*[nhyp] or null: voxel-map path skips hypotheses with stop_iter >= 0*/);
+
+// Tolerance stop of the ICP loop (pcreg_icp_stop; the rule is icp_stop_update in pcreg_icp.cuh)
+constexpr int ICP_STOP_WINDOW_MAX = 16;
+struct IcpStopRule { double tol_t, tol_r_deg; int window; };
 
 // Select / weight / 17 sums / Kabsch / compose, one block per hypothesis.
 struct IcpUpdateArgs {
@@ -260,7 +265,13 @@ struct IcpUpdateArgs {
     int update;                 // 1: apply the pose update; 0: score only (final pass)
     int32_t* frozen;            // [nhyp] status flags (1 = frozen)
     double* rmse; int32_t* n_used;        // [nhyp] written every pass
-    double* rmse_hist; int hist_stride; int hist_col;   // optional
+    double* rmse_hist; int hist_stride; int hist_col;   // optional; hist_col is also the pass index
+    // tolerance stop (stop_iter == nullptr: none, the k_icp_update<*, false> instantiations).  An intermediate pass leaves a
+    // stopped hypothesis alone; the final pass scores it and fills its history from the column its own final pass would have had.
+    int32_t* stop_iter;         // [nhyp] updates applied when the hypothesis stopped (converged or frozen), -1 while it runs
+    double* stop_ring;          // [nhyp][2 * ICP_STOP_WINDOW_MAX] motion of the last `window` updates
+    IcpStopRule stop;
+    int32_t* n_iter; int32_t* converged;   // [nhyp] optional, written by the final pass
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st);

@@ -27,7 +27,7 @@ def src_to_abi_t(src: torch.Tensor) -> torch.Tensor:
 class IcpDeviceBuffers:
     """Output tensors of one batched ICP call, allocated once and reused across steps."""
 
-    def __init__(self, nhyp: int, ns: int, iters: int, device, want_idx=False, want_hist=False):
+    def __init__(self, nhyp: int, ns: int, iters: int, device, want_idx=False, want_hist=False, want_n_iter=False):
         f64, i32 = torch.float64, torch.int32
         self.T = torch.empty((nhyp, 16), dtype=f64, device=device)
         self.rmse = torch.empty(nhyp, dtype=f64, device=device)
@@ -36,6 +36,9 @@ class IcpDeviceBuffers:
         self.idx = torch.empty((nhyp, ns), dtype=i32, device=device) if want_idx else None
         self.hist = torch.empty((nhyp, iters + 1), dtype=f64, device=device) if want_hist else None
         self.best = torch.empty(1, dtype=torch.int64, device=device)
+        # filled by a call with a tolerance stop: pose updates applied, 1 = stopped by the tolerance
+        self.n_iter = torch.empty(nhyp, dtype=i32, device=device) if want_n_iter else None
+        self.converged = torch.empty(nhyp, dtype=i32, device=device) if want_n_iter else None
 
 
 def _p(t):
@@ -43,10 +46,12 @@ def _p(t):
 
 
 def icp_batch_device(model: Model, src_cm: torch.Tensor, w_src, T0_abi: torch.Tensor, opts, out: IcpDeviceBuffers,
-                     stream=None):
+                     stream=None, stop=None):
     """Run pcreg_icp_batch_dev on tensors already resident on the library's device.
 
-    src_cm: float64 [3, ns] (column-major ns x 3); T0_abi: float64 [H,16] column-major records."""
+    src_cm: float64 [3, ns] (column-major ns x 3); T0_abi: float64 [H,16] column-major records.
+    stop: an api.icp_stop(tol_t, tol_r_deg, window) -> pcreg_icp_batch_stop_dev (out.n_iter / out.converged, when allocated,
+    receive the stop outputs)."""
     if not (src_cm.is_cuda and T0_abi.is_cuda):
         raise L.PcregError("icp_batch_device needs CUDA tensors (there is no CPU fallback)")
     assert src_cm.dtype == torch.float64 and src_cm.is_contiguous() and src_cm.shape[0] == 3
@@ -54,8 +59,15 @@ def icp_batch_device(model: Model, src_cm: torch.Tensor, w_src, T0_abi: torch.Te
     ns = src_cm.shape[1]
     nhyp = T0_abi.shape[0]
     st = stream if stream is not None else torch.cuda.current_stream()
-    L.check(L.lib().pcreg_icp_batch_dev(model.handle, _p(src_cm), ns, _p(w_src), _p(T0_abi), nhyp, C.byref(opts),
-                                        _p(out.T), _p(out.rmse), _p(out.n_used), _p(out.status), _p(out.idx),
-                                        _p(out.hist), _p(out.best), C.c_void_p(st.cuda_stream)),
-            "pcreg_icp_batch_dev")
+    if stop is None:
+        L.check(L.lib().pcreg_icp_batch_dev(model.handle, _p(src_cm), ns, _p(w_src), _p(T0_abi), nhyp, C.byref(opts),
+                                            _p(out.T), _p(out.rmse), _p(out.n_used), _p(out.status), _p(out.idx),
+                                            _p(out.hist), _p(out.best), C.c_void_p(st.cuda_stream)),
+                "pcreg_icp_batch_dev")
+    else:
+        L.check(L.lib().pcreg_icp_batch_stop_dev(model.handle, _p(src_cm), ns, _p(w_src), _p(T0_abi), nhyp, C.byref(opts),
+                                                 C.byref(stop), _p(out.T), _p(out.rmse), _p(out.n_used), _p(out.status),
+                                                 _p(out.idx), _p(out.hist), _p(out.best), _p(out.n_iter), _p(out.converged),
+                                                 C.c_void_p(st.cuda_stream)),
+                "pcreg_icp_batch_stop_dev")
     return out
