@@ -315,7 +315,57 @@ int  pcreg_icp_batch_stop_dev(const pcreg_model* m, const double* d_src, int64_t
                               int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
                               int32_t* d_n_iter, int32_t* d_converged, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev} or pcreg_nn_search call,
+/* ---- model normals and the point-to-plane metric --------------------------------------------------------------------
+ * Point-to-point ICP converges only linearly on a smooth, locally planar surface (the CT/MRI models of this project are
+ * meshes); point-to-plane converges in a few updates (Rusinkiewicz & Levoy 2001; Low 2004).  It needs one unit normal per
+ * model point, uploaded or computed on the device.  Normals live with the model (every device replica has its own copy),
+ * in original point order. */
+/* nrm: n x 3 column-major (ld), float (is_double = 0) or double; each row is normalised in FP64 as
+ * n / sqrt((nx*nx + ny*ny) + nz*nz).  A zero or non-finite row returns PCREG_ERR_ARG (and leaves the model's normals alone). */
+int  pcreg_model_set_normals(pcreg_model* m, const void* nrm, int is_double, int64_t ld);
+/* pcnormals(ptCloud, k) semantics, computed on the device; needs a model built with build_grid = 1 (else PCREG_ERR_ARG).
+ * k in [3, 64] and at most the model size (pcnormals' default is 6).  The rule:
+ *   neighbourhood  the k nearest model points of each model point, the point itself included (knnsearch semantics: exact FP64
+ *                  squared distances, ties broken toward the smaller original index);
+ *   normal         the eigenvector of the smallest eigenvalue of the unweighted covariance of those k points about their mean
+ *                  (FP64, symmetric 3x3 Jacobi), normalised as in pcreg_model_set_normals;
+ *   orientation    pcnormals documents none, so this library fixes one: with a viewpoint (double[3]) the normal is flipped so
+ *                  that n . (viewpoint - p) >= 0; with viewpoint == NULL so that n . (p - c) >= 0, c = the centre of the
+ *                  model's bounding box (outward on a closed star-shaped model).  The point-to-plane step does not depend on
+ *                  the sign.
+ * The toolbox is not available to compare against, so parity with pcnormals is UNPINNED. */
+int  pcreg_model_compute_normals(pcreg_model* m, int k, const double* viewpoint);
+/* out: n x 3 column-major doubles (ld = n).  PCREG_ERR_STATE when the model has no normals. */
+int  pcreg_model_get_normals(const pcreg_model* m, double* out);
+
+#define PCREG_ICP_POINT_TO_POINT 0
+#define PCREG_ICP_POINT_TO_PLANE 1
+/* Batched ICP with a choice of metric, plus the optional tolerance stop (stop == NULL: fixed iterations; n_iter and
+ * converged are written only with a stop).  Correspondences, rejection, trimming, weights and rmse (Euclidean,
+ * sqrt(sum w d^2 / sum w)) are those of pcreg_icp_batch; only the minimised metric and the pose update differ.
+ * POINT_TO_POINT: the results equal pcreg_icp_batch / pcreg_icp_batch_stop bit for bit.
+ * POINT_TO_PLANE (needs model normals, else PCREG_ERR_STATE): per pass, for every correspondence with weight w > 0, with
+ * q = quickTF(src, T), m = model point, n = its normal and p = the model's pivot (bounding-box centre),
+ *   q~ = q - p, m~ = m - p, a = (q~ x n, n) in R^6, b = (m~ - q~) . n;
+ * A = sum w a a' and g = sum w a b are FP64 sums; A = L D L' (no pivoting, unknowns (omega, tau) in that order) solves
+ * A x = g.  The update is degenerate (status 1, pose frozen as in pcreg_icp_batch) when fewer than 6 correspondences are
+ * usable, sum w is not > 0, or any D_k <= 1e-12 max_k A_kk (a flat patch).  Otherwise
+ *   R = I + (sin t / t) [omega]x + ((1 - cos t) / t^2) [omega]x^2, t = |omega| (R = I at t = 0),
+ *   dT = [R' 0; p - p R' + tau, 1] (row-vector form) and T <- T dT.
+ * An unknown metric returns PCREG_ERR_ARG.  Results do not depend on the device count. */
+int  pcreg_icp_batch_metric(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld,
+                            const double* w_src, const double* T0_16, int64_t nhyp,
+                            const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                            double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx,
+                            double* rmse_hist, int64_t* best, int32_t* n_iter, int32_t* converged);
+int  pcreg_icp_batch_metric_dev(const pcreg_model* m, const double* d_src, int64_t ns,
+                                const double* d_w_src, const double* d_T0_16, int64_t nhyp,
+                                const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                                double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status,
+                                int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
+                                int32_t* d_n_iter, int32_t* d_converged, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
  *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
  *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped

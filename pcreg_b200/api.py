@@ -18,6 +18,8 @@ from ._lib import AlignOpts, DescOpts, IcpOpts, IcpStop, MatchOpts, ModelOpts, P
 
 NN_BRUTE, NN_GRID = 0, 1
 ICP_PLAIN, ICP_KNN, ICP_WEIGHTED = 0, 1, 2
+ICP_POINT_TO_POINT, ICP_POINT_TO_PLANE = 0, 1
+METRICS = {"point_to_point": ICP_POINT_TO_POINT, "point_to_plane": ICP_POINT_TO_PLANE}
 METRIC_SAD, METRIC_SSD = 0, 1
 ALIGN_PLAIN, ALIGN_KNN_FRAC, ALIGN_KNN_ABS, ALIGN_WEIGHTED, ALIGN_C, ALIGN_KNN_C = range(6)
 
@@ -100,6 +102,27 @@ class Model:
         L.check(L.lib().pcreg_nn_search(self.handle, a.ctypes.data_as(C.c_void_p), is_double, nq, nq, int(nn),
                                         _ptr(idx, L.c_i32p), _ptr(d2, L.c_f64p)), "pcreg_nn_search")
         return idx, d2
+
+    def set_normals(self, nrm):
+        """Upload one normal per model point (N x 3, original order); each row is normalised in FP64.  A zero or non-finite
+        row raises (PCREG_ERR_ARG)."""
+        a, is_double, n = _cm_points(nrm)
+        if n != self.n:
+            raise ValueError("set_normals: need one normal per model point")
+        L.check(L.lib().pcreg_model_set_normals(self.handle, a.ctypes.data_as(C.c_void_p), is_double, n), "pcreg_model_set_normals")
+
+    def compute_normals(self, k: int = 6, viewpoint=None):
+        """pcnormals(ptCloud, k) on the device (include/pcreg.h: pcreg_model_compute_normals): the smallest-eigenvalue direction
+        of the k nearest model points of every point, oriented toward `viewpoint` or, without one, away from the centre of
+        the bounding box.  Needs a model built with grid=True."""
+        vp = None if viewpoint is None else np.ascontiguousarray(np.asarray(viewpoint, dtype=np.float64).reshape(3))
+        L.check(L.lib().pcreg_model_compute_normals(self.handle, int(k), _ptr(vp, L.c_f64p)), "pcreg_model_compute_normals")
+
+    def normals(self):
+        """The model's unit normals, N x 3 float64 (raises when it has none)."""
+        out = np.empty((3, self.n), dtype=np.float64)
+        L.check(L.lib().pcreg_model_get_normals(self.handle, _ptr(out, L.c_f64p)), "pcreg_model_get_normals")
+        return np.ascontiguousarray(out.T)
 
     def destroy(self):
         if self._h is not None:
@@ -487,13 +510,19 @@ def icp_stop(tol_t, tol_r_deg, window=3) -> IcpStop:
 
 
 def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src=None,
-              nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3):
+              nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3,
+              metric="point_to_point"):
     """Multi-start ICP of `src` against the resident `model` from the initial poses T0s [H,4,4].
     Returns dict(T [H,4,4], rmse [H], n_used [H], status [H], best, idx [H,ns]?, rmse_hist [H,iters+1]?).
 
     tolerance=(tol_t, tol_r_deg): each hypothesis stops once the mean translation change (model units) and the mean
     rotation change (degrees) of its last `window` updates are both below these (include/pcreg.h: pcreg_icp_stop); the
-    result then also holds n_iter [H] (pose updates applied) and converged [H] (1 = stopped by the tolerance)."""
+    result then also holds n_iter [H] (pose updates applied) and converged [H] (1 = stopped by the tolerance).
+
+    metric="point_to_plane" minimises the point-to-plane distance with the model's normals (Model.set_normals /
+    Model.compute_normals; include/pcreg.h: pcreg_icp_batch_metric); correspondences, weights and rmse are unchanged."""
+    if metric not in METRICS:
+        raise ValueError("metric must be one of %s" % sorted(METRICS))
     a, is_double, ns = _cm_points(src)
     T0 = _T_to_abi(np.asarray(T0s, dtype=np.float64).reshape(-1, 4, 4))
     H = T0.shape[0]
@@ -509,12 +538,15 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
     args = (model.handle, a.ctypes.data_as(C.c_void_p), is_double, ns, ns, _ptr(w, L.c_f64p), _ptr(T0, L.c_f64p), H, C.byref(o))
     outs = (_ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p), _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p),
             _ptr(hist, L.c_f64p), C.byref(best))
-    if tolerance is None:
+    n_iter = np.empty(H, dtype=np.int32) if tolerance is not None else None
+    converged = np.empty(H, dtype=np.int32) if tolerance is not None else None
+    stop = icp_stop(tolerance[0], tolerance[1], window) if tolerance is not None else None
+    if metric != "point_to_point":
+        L.check(L.lib().pcreg_icp_batch_metric(*args, METRICS[metric], C.byref(stop) if stop is not None else None, *outs,
+                                               _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)), "pcreg_icp_batch_metric")
+    elif tolerance is None:
         L.check(L.lib().pcreg_icp_batch(*args, *outs), "pcreg_icp_batch")
     else:
-        n_iter = np.empty(H, dtype=np.int32)
-        converged = np.empty(H, dtype=np.int32)
-        stop = icp_stop(tolerance[0], tolerance[1], window)
         L.check(L.lib().pcreg_icp_batch_stop(*args, C.byref(stop), *outs, _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)),
                 "pcreg_icp_batch_stop")
     out = dict(T=_T_from_abi(T, H), rmse=rmse, n_used=n_used, status=status, best=int(best.value))

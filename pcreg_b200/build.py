@@ -19,7 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 # for same-session A/B timing with PCREG_LIB=<variant>; the default build ignores both
 LIB = os.environ.get("PCREG_LIB_OUT") or os.path.join(HERE, "libpcreg_b200.so")
 OBJDIR = os.path.join(HERE, "build" if not os.environ.get("PCREG_LIB_OUT") else "build_" + os.path.basename(os.environ["PCREG_LIB_OUT"]))
-SOURCES = ["model.cu", "nn_brute.cu", "nn_grid.cu", "nn_vox.cu", "icp.cu", "icp_fused.cu", "kabsch_ransac.cu", "align.cu", "local_points.cu", "descriptor.cu", "match.cu"]
+SOURCES = ["model.cu", "nn_brute.cu", "nn_grid.cu", "nn_vox.cu", "icp.cu", "icp_fused.cu", "normals.cu", "kabsch_ransac.cu", "align.cu", "local_points.cu", "descriptor.cu", "match.cu"]
 HEADERS = ["pcreg_internal.h", "pcreg_dev.cuh", "pcreg_math.cuh", "pcreg_select.cuh", "pcreg_grid.cuh", "pcreg_vox.cuh", "pcreg_icp.cuh", os.path.join("..", "..", "include", "pcreg.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"] + os.environ.get("PCREG_NVCC_EXTRA", "").split()
@@ -70,12 +70,12 @@ def build_hostmath(force: bool = False) -> str:
     """Host-only build of pcreg_math.cuh behind a tiny C ABI (tests/hostmath): lets the CPU test
     suite check the 3x3 SVD / eigen / Kabsch code that the kernels inline, without a GPU."""
     root = os.path.dirname(HERE)
-    src = os.path.join(root, "tests", "hostmath", "hostmath.cpp")
+    srcs = [os.path.join(root, "tests", "hostmath", f) for f in ("hostmath.cpp", "hostmath_plane.cpp")]
     out = os.path.join(root, "tests", "hostmath", "libhostmath.so")
-    deps = [src, os.path.join(CSRC, "pcreg_math.cuh")]
+    deps = srcs + [os.path.join(CSRC, "pcreg_math.cuh")]
     if not force and os.path.exists(out) and os.path.getmtime(out) >= _newest(deps):
         return out
-    cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-ffp-contract=off", "-x", "c++", src, "-o", out]
+    cmd = ["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-ffp-contract=off", "-x", "c++"] + srcs + ["-o", out]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("g++ failed for hostmath:\n%s\n%s" % (r.stdout, r.stderr))

@@ -34,10 +34,12 @@ struct Pose16 { double t[16]; };      // a row-major row-vector pose as a kernel
 // NT = threads per hypothesis: UPD_THREADS (the fused kernel's count, so that both sum in the same order and agree bit for
 // bit) for sources the fused kernel can take, 512 for large sources (C5: 65 536 correspondences per hypothesis).
 // STOP = the tolerance stop (a.stop_iter set); the STOP = false instantiations are the loop without it.
-template <int NT, bool STOP>
+// PLANE = the point-to-plane metric (a.nrm set): 29 sums, the normals gathered with the model points.
+template <int NT, bool STOP, bool PLANE>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __grid_constant__ IcpUpdateArgs a) {
+    constexpr int NS = icp_nsums<PLANE>;
     __shared__ double Ts[16];
-    __shared__ double red[KABSCH_NSUMS * 32];
+    __shared__ double red[NS * 32];
     __shared__ long long redll[32];
     __shared__ HistSelShared hsel;
     __shared__ unsigned long long red_u64[64];
@@ -99,10 +101,10 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
         if (!reject && K >= 1 && K < nkept && nkept == ns) trim_tau = __longlong_as_double((long long)vK);
     }
 
-    // ---- weights + the 17 sums ----
-    double s[KABSCH_NSUMS];
+    // ---- weights + the 17 (29) sums ----
+    double s[NS];
 #pragma unroll
-    for (int k = 0; k < KABSCH_NSUMS; ++k) s[k] = 0.0;
+    for (int k = 0; k < NS; ++k) s[k] = 0.0;
     long long n_used = 0;
     const double px = a.pivot[0], py = a.pivot[1], pz = a.pivot[2];
     // Branch-free body, four correspondences per trip: the index / residual / source loads and the model gathers
@@ -130,9 +132,12 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
     for (int u = 0; u < UB; ++u) { const int64_t i = (int64_t)tid + (int64_t)u * NT; jn[u] = i < ns ? idx[i] : -1; }
     for (int64_t i0 = tid; i0 < ns; i0 += (int64_t)UB * NT) {
         int32_t jj[UB]; double dd[UB], xs[UB], ys[UB], zs[UB], ww[UB];
-        ModelPointD mm[UB];
+        ModelPointD mm[UB], nv[PLANE ? UB : 1];
 #pragma unroll
-        for (int u = 0; u < UB; ++u) { jj[u] = jn[u]; mm[u] = a.md[jj[u] >= 0 ? jj[u] : 0]; }
+        for (int u = 0; u < UB; ++u) {
+            jj[u] = jn[u]; mm[u] = a.md[jj[u] >= 0 ? jj[u] : 0];
+            if constexpr (PLANE) nv[u] = a.nrm[jj[u] >= 0 ? jj[u] : 0];
+        }
 #pragma unroll
         for (int u = 0; u < UB; ++u) {
             const int64_t i = i0 + (int64_t)u * NT;
@@ -154,15 +159,16 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             if (w > 0.0) ++n_used;
             double qx, qy, qz;
             quick_tf(Ts, xs[u], ys[u], zs[u], qx, qy, qz);
-            icp_accumulate(s, w, d, qx, qy, qz, mm[u], px, py, pz);
+            if constexpr (PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, mm[u], nv[u], px, py, pz);
+            else icp_accumulate(s, w, d, qx, qy, qz, mm[u], px, py, pz);
         }
     }
-    block_sum<KABSCH_NSUMS>(s, red);
+    block_sum<NS>(s, red);
     n_used = block_sum_ll(n_used, redll);
 
     if (tid == 0) {
         const double sw = s[0];
-        const double rmse = (sw > 0.0) ? sqrt(s[16] / sw) : nan("");
+        const double rmse = (sw > 0.0) ? sqrt(s[NS - 1] / sw) : nan("");
         a.rmse[h] = rmse;
         a.n_used[h] = (int32_t)n_used;
         int hist_from = a.hist_col;
@@ -179,7 +185,10 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
         if (a.update && !a.frozen[h]) {
             double Tn[16], Tc[16];
             for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
-            if (!icp_pose_update_call(s, n_used, a.pivot, a.reflection_fix != 0, Tc, Tn)) {
+            bool ok;
+            if constexpr (PLANE) ok = icp_pose_update_plane_call(s, n_used, a.pivot, Tc, Tn);
+            else ok = icp_pose_update_call(s, n_used, a.pivot, a.reflection_fix != 0, Tc, Tn);
+            if (!ok) {
                 a.frozen[h] = 1;
                 if (STOP) a.stop_iter[h] = a.hist_col;
             } else {
@@ -388,11 +397,16 @@ void transpose16_launch(const double* d_in, double* d_out, int64_t n, cudaStream
     k_transpose16<<<(unsigned)((n * 16 + 255) / 256), 256, 0, st>>>(d_in, d_out, n);
     PCREG_LAUNCHED();
 }
-void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
+template <bool PLANE>
+static void icp_update_launch_metric(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
     const bool stop = a.stop_iter != nullptr;
-    if (a.ns > 20000) { if (stop) k_icp_update<512, true><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false><<<(unsigned)nhyp, 512, 0, st>>>(a); }
-    else if (stop)    k_icp_update<UPD_THREADS, true><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
-    else              k_icp_update<UPD_THREADS, false><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    if (a.ns > 20000) { if (stop) k_icp_update<512, true, PLANE><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false, PLANE><<<(unsigned)nhyp, 512, 0, st>>>(a); }
+    else if (stop)    k_icp_update<UPD_THREADS, true, PLANE><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    else              k_icp_update<UPD_THREADS, false, PLANE><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+}
+void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
+    if (a.nrm) icp_update_launch_metric<true>(a, nhyp, st);
+    else       icp_update_launch_metric<false>(a, nhyp, st);
     PCREG_LAUNCHED();
 }
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st) {
@@ -410,8 +424,12 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     const double* d_w, const double* d_T0_cm, int64_t nhyp, const pcreg_icp_opts& o,
                     double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
                     double* d_rmse_hist, int64_t* d_best, cudaStream_t st,
-                    const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr) {
+                    const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr,
+                    int metric = PCREG_ICP_POINT_TO_POINT) {
     PCREG_REQUIRE(m && d_src && d_T0_cm && d_T16_cm, "icp: null pointer");
+    const bool plane = metric == PCREG_ICP_POINT_TO_PLANE;
+    const ModelPointD* nrm = plane ? m->nrm.p : nullptr;
+    if (plane && !nrm) throw StateError{"icp: the point-to-plane metric needs model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
     PCREG_REQUIRE(ns >= 1 && nhyp >= 1, "icp: need ns >= 1 and nhyp >= 1");
     PCREG_REQUIRE(o.iters >= 0, "icp: iters must be >= 0");
     PCREG_REQUIRE(o.mode >= PCREG_ICP_PLAIN && o.mode <= PCREG_ICP_WEIGHTED, "icp: bad mode");
@@ -425,7 +443,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     const double t_enter = now_ms();
     double t_alloc = 0, t_sorted = 0, t_enq = 0;
 
-    const bool fused = icp_fused_eligible(m, ns, nhyp, o);
+    const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop != nullptr, plane);
     // chunk the hypotheses so that the per-correspondence scratch stays bounded
     const size_t total_b = c.total_mem;         // queried once at pcreg_init (cudaMemGetInfo costs up to tens of ms per call)
     const size_t per_hyp = (size_t)ns * (4 + 4 + 8 + (o.mode == PCREG_ICP_KNN ? 8 : 0) + (o.nn == PCREG_NN_GRID ? 8 + (m->has_vox ? 0 : 28 + 4 * 64 + 4 * 448 / 16) : 0));
@@ -557,7 +575,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         fa.idx_out = d_idx; fa.perm = sorted ? sperm.p : nullptr; fa.tie_order = sorted ? sinv.p : nullptr;
         fa.mode = o.mode; fa.k_frac = o.k_frac; fa.R_w = o.R_w; fa.thDist2 = o.thDist2; fa.reflection_fix = o.reflection_fix; fa.iters = o.iters;
         fa.counters = (prof && c.profiling_counters) ? counters.p : nullptr;
-        fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged;
+        fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
         ev_begin(0);
         icp_fused_launch(fa, nhyp, stop != nullptr, st);
         ev_end();
@@ -638,7 +656,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                 ev_end();
                 nn_launches += 1;
                 IcpUpdateArgs ua{};
-                ua.md = m->md.p;
+                ua.md = m->md.p; ua.nrm = nrm;
                 for (int k = 0; k < 3; ++k) ua.pivot[k] = m->pivot[k];
                 ua.sx = sx; ua.sy = sy; ua.sz = sz; ua.w_src = d_w; ua.ns = ns;
                 ua.T = Twork.p + h0 * 16; ua.idx = out_idx; ua.d2 = L.d2.p; ua.keys = L.keys.p;
@@ -783,7 +801,7 @@ int pcreg_icp_batch_stop_dev(const pcreg_model* m, const double* d_src, int64_t 
 static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>& hs, int64_t ns, const double* w_src,
                                  const double* T0_16, int64_t h0, int64_t hn, const pcreg_icp_opts& o, double* T16, double* rmse,
                                  int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
-                                 const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged) {
+                                 const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric) {
     PCREG_CUDA(cudaSetDevice(ctx().device));
     cudaStream_t st = 0;
     DevBuf<double> d_src((size_t)ns * 3), d_w(w_src ? (size_t)ns : 0), d_T0((size_t)hn * 16), d_T((size_t)hn * 16);
@@ -794,7 +812,7 @@ static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>
     if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src, d_w.bytes(), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
     icp_run(m, d_src.p, ns, w_src ? d_w.p : nullptr, d_T0.p, hn, o, d_T.p, d_rmse.p, d_nu.p, d_st.p,
-            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st, stop, d_nit.p, d_conv.p);
+            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st, stop, d_nit.p, d_conv.p, metric);
     PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
@@ -806,11 +824,11 @@ static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>
     PCREG_CUDA(cudaStreamSynchronize(st));
 }
 
-// pcreg_icp_batch and pcreg_icp_batch_stop (stop != nullptr)
+// pcreg_icp_batch, pcreg_icp_batch_stop (stop != nullptr) and pcreg_icp_batch_metric
 static int icp_batch_host(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
                           const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* T16, double* rmse,
                           int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist, int64_t* best,
-                          const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged) {
+                          const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric = PCREG_ICP_POINT_TO_POINT) {
     require_init();
     PCREG_REQUIRE(m && src && T0_16 && T16 && opts, "pcreg_icp_batch: null pointer");
     PCREG_REQUIRE(ns >= 1 && ld >= ns && nhyp >= 1, "pcreg_icp_batch: bad sizes");
@@ -829,11 +847,11 @@ static int icp_batch_host(const pcreg_model* m, const void* src, int is_double, 
         if (hn <= 0) continue;
         workers.emplace_back([&, k, h0, hn]() {
             rc[k] = guarded([&]() { use_slot(k); icp_batch_host_slice(m->on_slot(k), hs, ns, w_src, T0_16, h0, hn, *opts, T16, rm, n_used, status, idx, rmse_hist,
-                                                                 stop, n_iter, converged); });
+                                                                 stop, n_iter, converged, metric); });
         });
     }
     rc[0] = guarded([&]() { use_slot(0); icp_batch_host_slice(m, hs, ns, w_src, T0_16, 0, std::min(per, nhyp), *opts, T16, rm, n_used, status, idx, rmse_hist,
-                                                         stop, n_iter, converged); });
+                                                         stop, n_iter, converged, metric); });
     for (auto& w : workers) w.join();
     use_slot(0);
     for (int k = 0; k < nd; ++k) if (rc[k] != PCREG_OK) return rc[k];
@@ -862,6 +880,37 @@ int pcreg_icp_batch_stop(const pcreg_model* m, const void* src, int is_double, i
     check_stop(stop);
     return icp_batch_host(m, src, is_double, ns, ld, w_src, T0_16, nhyp, opts, T16, rmse, n_used, status, idx, rmse_hist, best,
                           stop, n_iter, converged);
+    PCREG_API_END
+}
+
+static void check_metric(int metric, const pcreg_icp_stop* stop) {
+    PCREG_REQUIRE(metric == PCREG_ICP_POINT_TO_POINT || metric == PCREG_ICP_POINT_TO_PLANE, "icp: unknown metric");
+    if (stop) check_stop(stop);
+}
+
+int pcreg_icp_batch_metric(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
+                           const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                           double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                           int64_t* best, int32_t* n_iter, int32_t* converged) {
+    PCREG_API_BEGIN
+    check_metric(metric, stop);
+    return icp_batch_host(m, src, is_double, ns, ld, w_src, T0_16, nhyp, opts, T16, rmse, n_used, status, idx, rmse_hist, best,
+                          stop, stop ? n_iter : nullptr, stop ? converged : nullptr, metric);
+    PCREG_API_END
+}
+
+int pcreg_icp_batch_metric_dev(const pcreg_model* m, const double* d_src, int64_t ns, const double* d_w_src,
+                               const double* d_T0_16, int64_t nhyp, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                               double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
+                               double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    PCREG_REQUIRE(opts, "pcreg_icp_batch_metric_dev: opts is null");
+    check_metric(metric, stop);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    icp_run(m, d_src, ns, d_w_src, d_T0_16, nhyp, *opts, d_T16, d_rmse, d_n_used, d_status, d_idx, d_rmse_hist,
+            d_best, (cudaStream_t)stream, stop, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, metric);
+    return PCREG_OK;
     PCREG_API_END
 }
 

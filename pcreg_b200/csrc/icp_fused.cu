@@ -46,21 +46,23 @@ __device__ __noinline__ void fused_walk(const GridArgs& a, double qx, double qy,
     walk_search<false>(a, 0, Q, false, lc, ext_slot, thr2, 0.f, n1, n2, n3);
     bidx = Q.bidx; best = Q.best;
 }
-__device__ __noinline__ bool fused_pose_update(const double (&s)[KABSCH_NSUMS], long long n_used, const double* pivot, bool reflection_fix,
+template <bool PLANE>
+__device__ __noinline__ bool fused_pose_update(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot, bool reflection_fix,
                                                double* Ts /*shared, row-major 4x4, updated in place*/) {
     double Tc[16], Tn[16];
     for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
-    if (!icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn)) return false;
+    if (!icp_pose_update_m<PLANE>(s, n_used, pivot, reflection_fix, Tc, Tn)) return false;
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return true;
 }
 // Tolerance stop: the update of pass `it` (update it + 1) and the stop rule.  0: degenerate, pose left alone; 1: pose updated;
 // 2: pose updated and the rule says stop.
-__device__ __noinline__ int fused_pose_update_stop(const double (&s)[KABSCH_NSUMS], long long n_used, const double* pivot, bool reflection_fix,
+template <bool PLANE>
+__device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot, bool reflection_fix,
                                                    const IcpStopRule& rule, int it, double* ring /*shared*/, double* Ts /*shared*/) {
     double Tc[16], Tn[16];
     for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
-    if (!icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
+    if (!icp_pose_update_m<PLANE>(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
 }
@@ -68,11 +70,13 @@ __device__ __noinline__ int fused_pose_update_stop(const double (&s)[KABSCH_NSUM
 // KNN = the trimmed mode (its selection scratch -- 18 KB of shared memory -- exists only in that instantiation).
 // STOP = the tolerance stop (pcreg_icp_batch_stop): a stop -- by the rule or by a degenerate update -- makes the block's next
 // pass its final scoring pass, after which the block exits.  The STOP = false instantiations are the loop without it.
-template <bool KNN, bool STOP>
+// PLANE = the point-to-plane metric (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered there.
+template <bool KNN, bool STOP, bool PLANE>
 __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ FusedArgs a) {
+    constexpr int NS = icp_nsums<PLANE>;
     extern __shared__ __align__(16) unsigned char dyn[];
     __shared__ double Ts[16];
-    __shared__ double red[KABSCH_NSUMS * 32];
+    __shared__ double red[NS * 32];
     __shared__ long long redll[32];
     __shared__ HistSelShared hsel;
     __shared__ unsigned long long red_u64[64];
@@ -89,7 +93,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     const GridPoint* __restrict__ pts = a.g.g.pts;
     const bool reject = a.thDist2 > 0.0;
     constexpr bool knn = KNN;
-    constexpr bool two_pass = KNN || !FUSED_INLINE_SUMS;      // sums in a pass of their own (needed after a trim selection)
+    constexpr bool two_pass = KNN || PLANE || !FUSED_INLINE_SUMS;      // sums in a pass of their own (needed after a trim selection)
     const double px = a.pivot[0], py = a.pivot[1], pz = a.pivot[2];
     unsigned long long c_read = 0, c_gather = 0, c_walk = 0;
     long long t_nn = 0, t_sel = 0, t_sum = 0, t_svd = 0, t_mark = 0;       // phase clocks of thread 0 (profiling only)
@@ -104,9 +108,9 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
         // ---- exact nearest neighbours of the hypothesis' ns queries (two per trip: their header / entry loads overlap) ----
         long long nkept = 0;
         unsigned long long kmin = ~0ull, kmax = 0ull;
-        double s[KABSCH_NSUMS];
+        double s[NS];
 #pragma unroll
-        for (int k = 0; k < KABSCH_NSUMS; ++k) s[k] = 0.0;
+        for (int k = 0; k < NS; ++k) s[k] = 0.0;
         long long n_used = 0;
         unsigned long long vK = 0ull;
         bool all_eq = false;
@@ -143,7 +147,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             }
             idx_s[i0] = b0;
             if (has1) idx_s[i1] = b1;
-            if (!two_pass) {
+            if constexpr (!two_pass) {
                 ModelPointD m;
                 if (ok0) { m.x = w0c[0]; m.y = w0c[1]; m.z = w0c[2]; m.pad = 0.0; } else m = a.g.md[b0 >= 0 ? b0 : 0];
                 const double w0 = weight_of(i0, b0, d0);
@@ -209,15 +213,16 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 const double d = j >= 0 ? dist2_exact(m.x, m.y, m.z, qx, qy, qz) : (double)INFINITY;      // the NN step's d2, bit for bit
                 const double w = weight_of(i, j, d);
                 if (w > 0.0) ++n_used;
-                icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
+                if constexpr (PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
+                else icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
             }
         }
-        block_sum<KABSCH_NSUMS>(s, red);
+        block_sum<NS>(s, red);
         n_used = block_sum_ll(n_used, redll);
         if (timing) { const long long t = clock64(); t_sum += t - t_mark; t_mark = t; }
         if (tid == 0) {
             const double sw = s[0];
-            const double rmse = (sw > 0.0) ? sqrt(s[16] / sw) : nan("");
+            const double rmse = (sw > 0.0) ? sqrt(s[NS - 1] / sw) : nan("");
             if (a.rmse_hist) {
                 if (STOP && last) { for (int c = it; c <= a.iters; ++c) a.rmse_hist[h * a.hist_stride + c] = rmse; }
                 else a.rmse_hist[h * a.hist_stride + it] = rmse;
@@ -230,9 +235,9 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             }
             if (!last && !s_frozen) {
                 if (!STOP) {
-                    if (!fused_pose_update(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
+                    if (!fused_pose_update<PLANE>(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
                 } else {
-                    const int r = fused_pose_update_stop(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
+                    const int r = fused_pose_update_stop<PLANE>(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
                     if (r == 0) s_frozen = 1;
                     if (r != 1) s_stop = 1;
                 }
@@ -271,31 +276,43 @@ size_t icp_fused_smem(int64_t ns, int mode) {
     return (((size_t)ns * 4 + 15) / 16) * 16 + (mode == PCREG_ICP_KNN ? (size_t)ns * 8 : 0);
 }
 
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o) {
+// Point-to-point calls keep the check they always had (the static shared memory of k_icp_fused<true, false, false>); a
+// point-to-plane call checks the instantiation it launches (its reduction buffer is 29 instead of 17 doubles x 32).
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, bool plane) {
     if (!m->has_vox || o.nn != PCREG_NN_GRID) return false;
     if (const char* e = getenv("PCREG_FUSED")) { if (e[0] == '0') return false; if (e[0] == '1') nhyp = (int64_t)1 << 40; }
     // one block per hypothesis: a batch smaller than the SM count leaves SMs idle, the per-pass kernels (all SMs on every
     // pass) are faster there (C2, one hypothesis: 13.9 ms fused vs the per-pass path; PCREG_FUSED=1 forces the fused kernel)
     if (nhyp < ctx().sm_count) return false;
     if (ns >= ((int64_t)1 << 30)) return false;
+    const bool knn = o.mode == PCREG_ICP_KNN;
+    const void* fn = !plane ? (const void*)k_icp_fused<true, false, false>
+                   : knn ? (stop ? (const void*)k_icp_fused<true, true, true> : (const void*)k_icp_fused<true, false, true>)
+                         : (stop ? (const void*)k_icp_fused<false, true, true> : (const void*)k_icp_fused<false, false, true>);
     cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, k_icp_fused<true, false>) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (cudaFuncGetAttributes(&fa, fn) != cudaSuccess) { cudaGetLastError(); return false; }
     return icp_fused_smem(ns, o.mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
 }
 
-template <bool KNN, bool STOP>
+template <bool KNN, bool STOP, bool PLANE>
 static void fused_launch_one(const FusedArgs& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
-    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    k_icp_fused<KNN, STOP><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, PLANE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    k_icp_fused<KNN, STOP, PLANE><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+}
+
+template <bool PLANE>
+static void fused_launch_metric(const FusedArgs& a, int64_t nhyp, bool stop, size_t dyn, cudaStream_t st) {
+    const bool knn = a.mode == PCREG_ICP_KNN;
+    if (knn && !stop)       fused_launch_one<true, false, PLANE>(a, nhyp, dyn, st);
+    else if (!knn && !stop) fused_launch_one<false, false, PLANE>(a, nhyp, dyn, st);
+    else if (knn)           fused_launch_one<true, true, PLANE>(a, nhyp, dyn, st);
+    else                    fused_launch_one<false, true, PLANE>(a, nhyp, dyn, st);
 }
 
 void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
-    const bool knn = a.mode == PCREG_ICP_KNN;
-    if (knn && !stop)       fused_launch_one<true, false>(a, nhyp, dyn, st);
-    else if (!knn && !stop) fused_launch_one<false, false>(a, nhyp, dyn, st);
-    else if (knn)           fused_launch_one<true, true>(a, nhyp, dyn, st);
-    else                    fused_launch_one<false, true>(a, nhyp, dyn, st);
+    if (a.nrm) fused_launch_metric<true>(a, nhyp, stop, dyn, st);
+    else       fused_launch_metric<false>(a, nhyp, stop, dyn, st);
     PCREG_LAUNCHED();
 }
 

@@ -52,9 +52,10 @@ struct FusedArgs {
     unsigned long long* counters;           // profiling (may be null): [4] queries walked, [6] list entries read, [7] points gathered
     IcpStopRule stop;                       // tolerance stop (the k_icp_fused<*, true> instantiations only)
     int32_t* n_iter; int32_t* converged;    // [nhyp] optional outputs of the tolerance stop
+    const ModelPointD* nrm;                 // model normals (original order): the point-to-plane metric; null: point-to-point
 };
 size_t icp_fused_smem(int64_t ns, int mode);
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o);
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, bool plane);
 void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
 
 __device__ __forceinline__ void flush_counters(unsigned long long* counters, unsigned long long n_pts,

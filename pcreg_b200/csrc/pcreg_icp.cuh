@@ -60,6 +60,63 @@ __device__ __noinline__ static bool icp_pose_update_call(const double (&s)[KABSC
     return icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn);
 }
 
+// Point-to-plane metric (PCREG_ICP_POINT_TO_PLANE): with q~ = q - p, m~ = m - p and the model normal n of the correspondence,
+// a = (q~ x n, n), b = (m~ - q~) . n; the 29 sums (pcreg_math.cuh: PLANE_NSUMS) are sw, A = sum w a a' (upper triangle),
+// g = sum w a b and sum w d^2.  The rmse stays Euclidean: s[PLANE_NSUMS - 1] is sum w d^2 as s[16] of the 17 sums.
+__device__ __forceinline__ void icp_accumulate_plane(double (&s)[PLANE_NSUMS], double w, double d, double qx, double qy, double qz,
+                                                     const ModelPointD& m, const ModelPointD& n, double px, double py, double pz) {
+    const double q0 = qx - px, q1 = qy - py, q2 = qz - pz;
+    const double b = ((m.x - px) - q0) * n.x + ((m.y - py) - q1) * n.y + ((m.z - pz) - q2) * n.z;
+    const double a[6] = {q1 * n.z - q2 * n.y, q2 * n.x - q0 * n.z, q0 * n.y - q1 * n.x, n.x, n.y, n.z};
+    s[0] += w;
+    int k = 1;
+#pragma unroll
+    for (int r = 0; r < 6; ++r) {
+        const double wa = w * a[r];
+#pragma unroll
+        for (int c = r; c < 6; ++c) s[k++] += wa * a[c];
+        s[22 + r] += wa * b;
+    }
+    s[28] += w * d;
+}
+
+// Thread 0 after the block reduction: x = (omega, tau) from A x = g, dR = Rodrigues(omega)', dT = [dR 0; p - p dR + tau, 1] and
+// T <- T * dT.  Returns false (pose left alone, hypothesis to be frozen) with fewer than 6 usable correspondences, no weight
+// or a pivot of the LDL' factorisation at or below 1e-12 max A_kk.
+__device__ __forceinline__ bool icp_pose_update_plane(const double (&s)[PLANE_NSUMS], long long n_used, const double* pivot,
+                                                      const double* Tc, double* Tn) {
+    if (n_used < 6 || !(s[0] > 0.0)) return false;
+    double x[6];
+    if (!ldlt6_solve(s + 1, s + 22, x)) return false;
+    double R[9];
+    rodrigues(x, R);
+    double dT[16];
+    for (int r = 0; r < 3; ++r) {
+        for (int c = 0; c < 3; ++c) dT[r * 4 + c] = R[c * 3 + r];
+        dT[r * 4 + 3] = 0.0;
+    }
+    for (int c = 0; c < 3; ++c)
+        dT[12 + c] = (pivot[c] - (pivot[0] * dT[0 * 4 + c] + pivot[1] * dT[1 * 4 + c] + pivot[2] * dT[2 * 4 + c])) + x[3 + c];
+    dT[15] = 1.0;
+    mul4(Tc, dT, Tn);
+    return true;
+}
+
+// out of line for the same reason as icp_pose_update_call
+__device__ __noinline__ static bool icp_pose_update_plane_call(const double (&s)[PLANE_NSUMS], long long n_used, const double* pivot,
+                                                               const double* Tc, double* Tn) {
+    return icp_pose_update_plane(s, n_used, pivot, Tc, Tn);
+}
+
+// sums of one ICP pass: 17 (point-to-point, Kabsch) or 29 (point-to-plane); the last one is sum w d^2 in both
+template <bool PLANE> constexpr int icp_nsums = PLANE ? PLANE_NSUMS : KABSCH_NSUMS;
+template <bool PLANE>
+__device__ __forceinline__ bool icp_pose_update_m(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot,
+                                                  bool reflection_fix, const double* Tc, double* Tn) {
+    if constexpr (PLANE) return icp_pose_update_plane(s, n_used, pivot, Tc, Tn);
+    else return icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn);
+}
+
 // Tolerance stop (pcreg_icp_stop, include/pcreg.h).  Update u (1-based) took Tc = T_{u-1} to Tn = T_u = T_{u-1} dT.  Its motion
 //   dt_u = |t_u - t_{u-1}|                                   (translation rows)
 //   dr_u = atan2(|v|, (trace dR - 1) / 2) in degrees,  dR = R_{u-1}' R_u,  v = (dR32 - dR23, dR13 - dR31, dR21 - dR12) / 2

@@ -34,6 +34,7 @@ void count_launch(int n = 1);
 struct ArgError { std::string msg; };
 #define PCREG_REQUIRE(cond, msg)                                                              \
     do { if (!(cond)) throw ::pcreg::ArgError{msg}; } while (0)
+struct StateError { std::string msg; };     // the handle lacks what the call needs (PCREG_ERR_STATE)
 
 // Every extern "C" body is wrapped in these: no C++ exception crosses the ABI.
 #define PCREG_API_BEGIN try {
@@ -45,6 +46,7 @@ struct ArgError { std::string msg; };
         return PCREG_ERR_CUDA;                                                                                \
     }                                                                                                         \
     catch (const ::pcreg::ArgError& a) { ::pcreg::set_error("%s", a.msg.c_str()); return PCREG_ERR_ARG; }     \
+    catch (const ::pcreg::StateError& a) { ::pcreg::set_error("%s", a.msg.c_str()); return PCREG_ERR_STATE; } \
     catch (const std::bad_alloc&) { ::pcreg::set_error("host allocation failed"); return PCREG_ERR_ALLOC; }   \
     catch (...) { ::pcreg::set_error("unknown C++ exception"); return PCREG_ERR_STATE; }
 
@@ -188,6 +190,7 @@ struct pcreg_model {
     pcreg::DevBuf<float4> m4;               // shuffled scan order: (x,y,z relative to pivot, |.|^2)
     pcreg::DevBuf<int32_t> perm;            // perm[scan position] = original index
     pcreg::DevBuf<pcreg::ModelPointD> md;   // original order, FP64
+    pcreg::DevBuf<pcreg::ModelPointD> nrm;  // unit normals {nx, ny, nz, 0}, original order (empty: none; point-to-plane ICP)
     // grid
     bool has_grid = false;
     pcreg::GridView grid{};
@@ -272,6 +275,7 @@ struct IcpUpdateArgs {
     double* stop_ring;          // [nhyp][2 * ICP_STOP_WINDOW_MAX] motion of the last `window` updates
     IcpStopRule stop;
     int32_t* n_iter; int32_t* converged;   // [nhyp] optional, written by the final pass
+    const pcreg::ModelPointD* nrm;         // model normals (original order): the point-to-plane metric (k_icp_update<*, *, true>)
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st);

@@ -1,7 +1,7 @@
 // pcreg_math.cuh -- small FP64 linear algebra shared by every kernel (host + device).
 //
 // 3x3 one-sided Jacobi SVD, symmetric 3x3 Jacobi eigen-solver, Kabsch pose from the 16 weighted
-// sums, row-vector 4x4 composition.  Matrices are ROW-MAJOR double[9] / double[16] in here
+// sums, row-vector 4x4 composition, the 6x6 LDL' solve and the Rodrigues rotation of the point-to-plane step.  Matrices are ROW-MAJOR double[9] / double[16] in here
 // (element (r,c) at [r*3+c] / [r*4+c]); the C ABI converts to MATLAB column-major at the edge.
 //
 // Reference arithmetic restated (not copied): estimateTransform.m:41-71 (centroids, H = m_c*d_c',
@@ -227,6 +227,62 @@ PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const
         for (int c = 0; c < 3; ++c) dT[r * 4 + c] = R[c * 3 + r];
     dT[0 * 4 + 3] = 0.0; dT[1 * 4 + 3] = 0.0; dT[2 * 4 + 3] = 0.0;
     dT[3 * 4 + 0] = t[0]; dT[3 * 4 + 1] = t[1]; dT[3 * 4 + 2] = t[2]; dT[3 * 4 + 3] = 1.0;
+}
+
+// ---- point-to-plane ICP step (include/pcreg.h: PCREG_ICP_POINT_TO_PLANE) ----
+// 29 running sums: sw, the 21 upper-triangle entries of A = sum w a a' (row-major: (0,0), (0,1), .. (0,5), (1,1), ..), the 6 of
+// g = sum w a b, sum w d^2
+constexpr int PLANE_NSUMS = 29;
+
+// A x = g for a symmetric 6x6 A given by its upper triangle (row-major, 21 entries): A = L D L' without pivoting, unknowns in
+// their natural order.  Returns false (x untouched) when some pivot D_k is not above 1e-12 * max_k A_kk (a flat patch leaves a
+// direction of the pose unconstrained).
+PCREG_HD bool ldlt6_solve(const double* Au, const double* g, double* x) {
+    double A[36];
+    for (int r = 0, k = 0; r < 6; ++r)
+        for (int c = r; c < 6; ++c, ++k) { A[r * 6 + c] = Au[k]; A[c * 6 + r] = Au[k]; }
+    double amax = 0.0;
+    for (int k = 0; k < 6; ++k) amax = fmax(amax, A[k * 7]);
+    const double tiny = 1e-12 * amax;
+    double L[36], D[6];
+    for (int j = 0; j < 6; ++j) {
+        double d = A[j * 7];
+        for (int k = 0; k < j; ++k) d -= L[j * 6 + k] * L[j * 6 + k] * D[k];
+        if (!(d > tiny)) return false;
+        D[j] = d;
+        for (int i = j + 1; i < 6; ++i) {
+            double v = A[i * 6 + j];
+            for (int k = 0; k < j; ++k) v -= L[i * 6 + k] * L[j * 6 + k] * D[k];
+            L[i * 6 + j] = v / d;
+        }
+    }
+    double y[6];
+    for (int i = 0; i < 6; ++i) {
+        double v = g[i];
+        for (int k = 0; k < i; ++k) v -= L[i * 6 + k] * y[k];
+        y[i] = v;
+    }
+    for (int i = 5; i >= 0; --i) {
+        double v = y[i] / D[i];
+        for (int k = i + 1; k < 6; ++k) v -= L[k * 6 + i] * x[k];
+        x[i] = v;
+    }
+    return true;
+}
+
+// Rodrigues: R = I + (sin t / t) [w]x + ((1 - cos t) / t^2) [w]x^2, t = |w|; R = I at t = 0.  Column-vector convention (R v =
+// v + w x v + ...), row-major storage.
+PCREG_HD void rodrigues(const double* w, double* R) {
+    const double t2 = w[0] * w[0] + w[1] * w[1] + w[2] * w[2];
+    const double t = sqrt(t2);
+    for (int i = 0; i < 9; ++i) R[i] = 0.0;
+    R[0] = R[4] = R[8] = 1.0;
+    if (!(t > 0.0)) return;
+    const double a = sin(t) / t, b = (1.0 - cos(t)) / t2;
+    const double K[9] = {0.0, -w[2], w[1], w[2], 0.0, -w[0], -w[1], w[0], 0.0};
+    double K2[9];
+    mul3(K, K, K2);
+    for (int i = 0; i < 9; ++i) R[i] += a * K[i] + b * K2[i];
 }
 
 // MATLAB eps(x) for x >= 0: spacing of doubles at x.
