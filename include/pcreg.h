@@ -365,7 +365,41 @@ int  pcreg_icp_batch_metric_dev(const pcreg_model* m, const double* d_src, int64
                                 int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
                                 int32_t* d_n_iter, int32_t* d_converged, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev} or pcreg_nn_search call,
+/* ---- plane-to-plane metric (generalized ICP; Segal, Haehnel & Thrun 2009) -------------------------------------------
+ * Point-to-point treats the source as exact and point-to-plane uses only the model's surface; plane-to-plane models both clouds
+ * as locally planar, which suits a noisy source (a stereo reconstruction) against a smooth model.  It needs model normals (else
+ * PCREG_ERR_STATE) and one normal per source point.  Per pass, correspondences, rejection, trimming, weights and rmse (Euclidean,
+ * sqrt(sum w d^2 / sum w)) are those of pcreg_icp_batch; only the minimised metric and the update differ.  With q = quickTF(s, T),
+ * R the rotation block of T, p the model's pivot, for every correspondence (s, m) with w > 0:
+ *   n_q = n_s R (the source normal carried with the point), n_m = the model normal of m,
+ *   C = 2I - (1 - eps)(n_m n_m' + n_q n_q')  (the sum of the two plane covariances I - (1 - eps) n n'; eigenvalues in [2 eps, 2]),
+ *   M = C^-1 = adj(C) / det(C) in FP64,  q~ = q - p, m~ = m - p, e = m~ - q~,  J' = [[q~]x; I] (6 x 3),
+ *   A = sum w J' M J (FP64, upper triangle) and g = sum w J' M e = sum w (q~ x Me, Me).
+ * With M = n n' this is the point-to-plane accumulation (J' n = (q~ x n, n) is its a).  The solve, the degenerate case and the update
+ * are those of POINT_TO_PLANE (A x = g by L D L', status 1 and the pose frozen with fewer than 6 usable correspondences, sum w not
+ * > 0 or a pivot <= 1e-12 max A_kk; Rodrigues, dT = [R' 0; p - p R' + tau, 1], T <- T dT).
+ * Consequences: M depends on the normals only through n n', so flipping the sign of any source or model normal changes no bit of
+ * the result; eps = 1 gives M = I/2, i.e. the Gauss-Newton linearised point-to-point step (not the Kabsch one).  This is ONE
+ * Gauss-Newton step per correspondence pass with M frozen for that pass; Segal et al. run an inner optimiser instead.  eps = 1e-3
+ * is their value and the usual default; an eps that is not finite or outside (0, 1] returns PCREG_ERR_ARG.  pcregistericp's
+ * 'planeToPlane' documents no eps, so parity with the toolbox is UNPINNED.
+ * src_nrm: ns x 3 column-major, same type and ld as src; each row is normalised in FP64 as pcreg_model_set_normals does, and a NULL
+ * pointer or a zero or non-finite row returns PCREG_ERR_ARG (checked on the device before any ICP kernel runs).  stop is optional
+ * and checked as in pcreg_icp_batch_stop (n_iter and converged are written only with a stop).  Results do not depend on the device
+ * count: the host entry copies the source normals to every device. */
+int  pcreg_icp_batch_gicp(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld,
+                          const double* w_src, const void* src_nrm, double eps,
+                          const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                          double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx,
+                          double* rmse_hist, int64_t* best, int32_t* n_iter, int32_t* converged);
+/* d_src_nrm: float64 column-major, ld = ns, on the device; synchronous with respect to `stream` as pcreg_icp_batch_dev. */
+int  pcreg_icp_batch_gicp_dev(const pcreg_model* m, const double* d_src, int64_t ns, const double* d_w_src,
+                              const double* d_src_nrm, double eps,
+                              const double* d_T0_16, int64_t nhyp, const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                              double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
+                              double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
  *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
  *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped

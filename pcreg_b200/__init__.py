@@ -5,7 +5,7 @@ this package is only the host-side mirror of the reference's MATLAB interface.  
 """
 from ._lib import PcregError, init, shutdown, load, LIB_PATH  # noqa: F401
 from .api import (  # noqa: F401
-    Model, getLocalPoints, getLocalPoints_batch, getSpacialHistogramDescriptors, spatial_histogram_edges, AlignPoints, AlignPoints_KNN, AlignPoints_knn, AlignPoints_weighted, AlignPoints_c,
+    Model, cloud_normals, getLocalPoints, getLocalPoints_batch, getSpacialHistogramDescriptors, spatial_histogram_edges, AlignPoints, AlignPoints_KNN, AlignPoints_knn, AlignPoints_weighted, AlignPoints_c,
     AlignPoints_KNN_c, align_points_batch, estimateTransform, estimate_transform_batch, ransac, ransac_seeded, ransac_batch,
     getMatches, transfer_colors, quickTF, TF_FORWARD, TF_INVERT, TF_MRDIVIDE, icp_batch, icp_opts, icp_stop, set_profiling, last_profile, launch_count,
     NN_BRUTE, NN_GRID, METRIC_SAD, METRIC_SSD, ICP_PLAIN, ICP_KNN, ICP_WEIGHTED, ICP_POINT_TO_POINT, ICP_POINT_TO_PLANE,

@@ -20,6 +20,9 @@ NN_BRUTE, NN_GRID = 0, 1
 ICP_PLAIN, ICP_KNN, ICP_WEIGHTED = 0, 1, 2
 ICP_POINT_TO_POINT, ICP_POINT_TO_PLANE = 0, 1
 METRICS = {"point_to_point": ICP_POINT_TO_POINT, "point_to_plane": ICP_POINT_TO_PLANE}
+# the plane-to-plane metric has entries of its own (pcreg_icp_batch_gicp{,_dev}); it is no value of pcreg_icp_batch_metric's `metric`
+PLANE_TO_PLANE = "plane_to_plane"
+GICP_EPS = 1e-3
 METRIC_SAD, METRIC_SSD = 0, 1
 ALIGN_PLAIN, ALIGN_KNN_FRAC, ALIGN_KNN_ABS, ALIGN_WEIGHTED, ALIGN_C, ALIGN_KNN_C = range(6)
 
@@ -134,6 +137,18 @@ class Model:
             self.destroy()
         except Exception:
             pass
+
+
+def cloud_normals(pts, k: int = 6, viewpoint=None):
+    """Unit normals of any N x 3 cloud (N x 3 float64), by Model.compute_normals' rule (pcnormals(ptCloud, k) semantics, computed
+    on the device): a temporary grid-only model of the points is built, its normals read back, and the model destroyed.  Meant for
+    the source normals of icp_batch(..., metric="plane_to_plane", src_normals=cloud_normals(src))."""
+    m = Model(pts, grid=True, voxel_map=-1)
+    try:
+        m.compute_normals(k, viewpoint)
+        return m.normals()
+    finally:
+        m.destroy()
 
 
 # ------------------------------------------------------------------------------------------------
@@ -511,7 +526,7 @@ def icp_stop(tol_t, tol_r_deg, window=3) -> IcpStop:
 
 def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src=None,
               nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3,
-              metric="point_to_point"):
+              metric="point_to_point", src_normals=None, gicp_eps=GICP_EPS):
     """Multi-start ICP of `src` against the resident `model` from the initial poses T0s [H,4,4].
     Returns dict(T [H,4,4], rmse [H], n_used [H], status [H], best, idx [H,ns]?, rmse_hist [H,iters+1]?).
 
@@ -520,10 +535,22 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
     result then also holds n_iter [H] (pose updates applied) and converged [H] (1 = stopped by the tolerance).
 
     metric="point_to_plane" minimises the point-to-plane distance with the model's normals (Model.set_normals /
-    Model.compute_normals; include/pcreg.h: pcreg_icp_batch_metric); correspondences, weights and rmse are unchanged."""
-    if metric not in METRICS:
-        raise ValueError("metric must be one of %s" % sorted(METRICS))
+    Model.compute_normals; include/pcreg.h: pcreg_icp_batch_metric); correspondences, weights and rmse are unchanged.
+    metric="plane_to_plane" is generalized ICP (include/pcreg.h: pcreg_icp_batch_gicp): it needs the model's normals and
+    `src_normals` (N x 3, one per source point, e.g. cloud_normals(src)); gicp_eps in (0, 1] is the covariance epsilon.  The C entry
+    takes the normals in the source's type, so with a float32 source they are rounded to float32 before the library normalises
+    them in FP64; pass the source as float64 to keep float64 normals."""
+    if metric not in METRICS and metric != PLANE_TO_PLANE:
+        raise ValueError("metric must be one of %s" % sorted(list(METRICS) + [PLANE_TO_PLANE]))
+    if metric == PLANE_TO_PLANE and src_normals is None:
+        raise ValueError("metric='plane_to_plane' needs src_normals (one normal per source point, e.g. cloud_normals(src))")
+    if metric != PLANE_TO_PLANE and src_normals is not None:
+        raise ValueError("src_normals is used only by metric='plane_to_plane'")
     a, is_double, ns = _cm_points(src)
+    if src_normals is not None:
+        sn = np.asfortranarray(np.asarray(src_normals).astype(a.dtype, copy=False))
+        if sn.shape != (ns, 3):
+            raise ValueError("src_normals must be N x 3, one normal per source point")
     T0 = _T_to_abi(np.asarray(T0s, dtype=np.float64).reshape(-1, 4, 4))
     H = T0.shape[0]
     o = icp_opts(mode, iters, k_frac, R_w, thDist2, nn, reflection_fix)
@@ -541,7 +568,11 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
     n_iter = np.empty(H, dtype=np.int32) if tolerance is not None else None
     converged = np.empty(H, dtype=np.int32) if tolerance is not None else None
     stop = icp_stop(tolerance[0], tolerance[1], window) if tolerance is not None else None
-    if metric != "point_to_point":
+    if metric == PLANE_TO_PLANE:
+        L.check(L.lib().pcreg_icp_batch_gicp(*args[:6], sn.ctypes.data_as(C.c_void_p), float(gicp_eps), *args[6:],
+                                             C.byref(stop) if stop is not None else None, *outs, _ptr(n_iter, L.c_i32p),
+                                             _ptr(converged, L.c_i32p)), "pcreg_icp_batch_gicp")
+    elif metric != "point_to_point":
         L.check(L.lib().pcreg_icp_batch_metric(*args, METRICS[metric], C.byref(stop) if stop is not None else None, *outs,
                                                _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)), "pcreg_icp_batch_metric")
     elif tolerance is None:

@@ -1,6 +1,6 @@
 // icp.cu -- the batched ICP loop: (NN) -> select / weight -> 17 FP64 sums -> Kabsch SVD -> pose
-// compose, for a batch of independent hypotheses, plus the C-ABI entry points pcreg_icp_batch,
-// pcreg_icp_batch_dev and pcreg_nn_search.
+// compose, for a batch of independent hypotheses, plus the C-ABI entry points pcreg_icp_batch{,_stop,_metric,_gicp}{,_dev}
+// and pcreg_nn_search.
 //
 // Composition restated from the reference's primitives (SURVEY.md section 8c, oracle/icp.py):
 //   pose apply    quickTF.m:5-7
@@ -13,6 +13,7 @@
 #include <math.h>
 #include <float.h>
 #include <stdio.h>
+#include <cmath>
 #include <stdlib.h>
 #include <time.h>
 #include <algorithm>
@@ -34,10 +35,12 @@ struct Pose16 { double t[16]; };      // a row-major row-vector pose as a kernel
 // NT = threads per hypothesis: UPD_THREADS (the fused kernel's count, so that both sum in the same order and agree bit for
 // bit) for sources the fused kernel can take, 512 for large sources (C5: 65 536 correspondences per hypothesis).
 // STOP = the tolerance stop (a.stop_iter set); the STOP = false instantiations are the loop without it.
-// PLANE = the point-to-plane metric (a.nrm set): 29 sums, the normals gathered with the model points.
-template <int NT, bool STOP, bool PLANE>
+// METRIC = 1: the point-to-plane metric (a.nrm set): 29 sums, the normals gathered with the model points; 2: plane-to-plane
+// (a.snx set as well): the same, and each correspondence's source normal read with the source point and rotated by the pose.
+template <int NT, bool STOP, int METRIC>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __grid_constant__ IcpUpdateArgs a) {
-    constexpr int NS = icp_nsums<PLANE>;
+    constexpr int NS = icp_nsums<METRIC>;
+    constexpr bool MNRM = METRIC != ICP_M_POINT, SNRM = METRIC == ICP_M_GICP;
     __shared__ double Ts[16];
     __shared__ double red[NS * 32];
     __shared__ long long redll[32];
@@ -132,11 +135,12 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
     for (int u = 0; u < UB; ++u) { const int64_t i = (int64_t)tid + (int64_t)u * NT; jn[u] = i < ns ? idx[i] : -1; }
     for (int64_t i0 = tid; i0 < ns; i0 += (int64_t)UB * NT) {
         int32_t jj[UB]; double dd[UB], xs[UB], ys[UB], zs[UB], ww[UB];
-        ModelPointD mm[UB], nv[PLANE ? UB : 1];
+        ModelPointD mm[UB], nv[MNRM ? UB : 1];
+        double snx[SNRM ? UB : 1], sny[SNRM ? UB : 1], snz[SNRM ? UB : 1];
 #pragma unroll
         for (int u = 0; u < UB; ++u) {
             jj[u] = jn[u]; mm[u] = a.md[jj[u] >= 0 ? jj[u] : 0];
-            if constexpr (PLANE) nv[u] = a.nrm[jj[u] >= 0 ? jj[u] : 0];
+            if constexpr (MNRM) nv[u] = a.nrm[jj[u] >= 0 ? jj[u] : 0];
         }
 #pragma unroll
         for (int u = 0; u < UB; ++u) {
@@ -145,6 +149,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             const int64_t ic = ok ? i : tid;                 // tid < ns is guaranteed inside the loop
             dd[u] = d2[ic];
             xs[u] = a.sx[ic]; ys[u] = a.sy[ic]; zs[u] = a.sz[ic];
+            if constexpr (SNRM) { snx[u] = a.snx[ic]; sny[u] = a.sny[ic]; snz[u] = a.snz[ic]; }
             const int64_t in = i + (int64_t)UB * NT;
             jn[u] = in < ns ? idx[in] : -1;
         }
@@ -159,7 +164,8 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             if (w > 0.0) ++n_used;
             double qx, qy, qz;
             quick_tf(Ts, xs[u], ys[u], zs[u], qx, qy, qz);
-            if constexpr (PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, mm[u], nv[u], px, py, pz);
+            if constexpr (SNRM) icp_accumulate_gicp(s, w, d, qx, qy, qz, mm[u], nv[u], snx[u], sny[u], snz[u], Ts, a.gicp_eps, px, py, pz);
+            else if constexpr (MNRM) icp_accumulate_plane(s, w, d, qx, qy, qz, mm[u], nv[u], px, py, pz);
             else icp_accumulate(s, w, d, qx, qy, qz, mm[u], px, py, pz);
         }
     }
@@ -186,7 +192,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             double Tn[16], Tc[16];
             for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
             bool ok;
-            if constexpr (PLANE) ok = icp_pose_update_plane_call(s, n_used, a.pivot, Tc, Tn);
+            if constexpr (MNRM) ok = icp_pose_update_plane_call(s, n_used, a.pivot, Tc, Tn);
             else ok = icp_pose_update_call(s, n_used, a.pivot, a.reflection_fix != 0, Tc, Tn);
             if (!ok) {
                 a.frozen[h] = 1;
@@ -374,6 +380,20 @@ __global__ void k_unpermute_idx(const int32_t* __restrict__ in, const int32_t* _
     out[g] = in[h * ns + inv[o]];
 }
 
+// Source normals of the plane-to-plane metric, one thread per row: out row r (the order of the sorted source) is input row perm[r]
+// (perm null: r) normalised in FP64 as pcreg_model_set_normals normalises (no contraction into FMA: the same bits as the host
+// loop).  A zero or non-finite row sets *bad.  in, out: ns x 3 column-major, ld = ns.
+__global__ void k_src_normals(const double* __restrict__ in, const int32_t* __restrict__ perm, int64_t ns, double* __restrict__ out,
+                              int* __restrict__ bad) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= ns) return;
+    const int64_t o = perm ? perm[r] : r;
+    const double x = in[o], y = in[ns + o], z = in[2 * ns + o];
+    const double n = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)));
+    if (!(isfinite(n) && n > 0.0)) *bad = 1;
+    out[r] = x / n; out[ns + r] = y / n; out[2 * ns + r] = z / n;
+}
+
 // MATLAB column-major 4x4 <-> internal row-major 4x4 (a transpose), batched
 __global__ void k_transpose16(const double* __restrict__ in, double* __restrict__ out, int64_t n) {
     const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -397,16 +417,17 @@ void transpose16_launch(const double* d_in, double* d_out, int64_t n, cudaStream
     k_transpose16<<<(unsigned)((n * 16 + 255) / 256), 256, 0, st>>>(d_in, d_out, n);
     PCREG_LAUNCHED();
 }
-template <bool PLANE>
+template <int METRIC>
 static void icp_update_launch_metric(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
     const bool stop = a.stop_iter != nullptr;
-    if (a.ns > 20000) { if (stop) k_icp_update<512, true, PLANE><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false, PLANE><<<(unsigned)nhyp, 512, 0, st>>>(a); }
-    else if (stop)    k_icp_update<UPD_THREADS, true, PLANE><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
-    else              k_icp_update<UPD_THREADS, false, PLANE><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    if (a.ns > 20000) { if (stop) k_icp_update<512, true, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); }
+    else if (stop)    k_icp_update<UPD_THREADS, true, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    else              k_icp_update<UPD_THREADS, false, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
 }
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
-    if (a.nrm) icp_update_launch_metric<true>(a, nhyp, st);
-    else       icp_update_launch_metric<false>(a, nhyp, st);
+    if (a.snx)      icp_update_launch_metric<ICP_M_GICP>(a, nhyp, st);
+    else if (a.nrm) icp_update_launch_metric<ICP_M_PLANE>(a, nhyp, st);
+    else            icp_update_launch_metric<ICP_M_POINT>(a, nhyp, st);
     PCREG_LAUNCHED();
 }
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st) {
@@ -425,11 +446,12 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
                     double* d_rmse_hist, int64_t* d_best, cudaStream_t st,
                     const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr,
-                    int metric = PCREG_ICP_POINT_TO_POINT) {
+                    int metric = ICP_M_POINT, const double* d_src_nrm = nullptr /*ICP_M_GICP: col-major ns x 3*/, double gicp_eps = 0.0) {
     PCREG_REQUIRE(m && d_src && d_T0_cm && d_T16_cm, "icp: null pointer");
-    const bool plane = metric == PCREG_ICP_POINT_TO_PLANE;
+    const bool plane = metric != ICP_M_POINT, gicp = metric == ICP_M_GICP;
     const ModelPointD* nrm = plane ? m->nrm.p : nullptr;
-    if (plane && !nrm) throw StateError{"icp: the point-to-plane metric needs model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
+    if (plane && !nrm) throw StateError{"icp: the point-to-plane and plane-to-plane metrics need model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
+    PCREG_REQUIRE(!gicp || d_src_nrm, "icp: the plane-to-plane metric needs source normals");
     PCREG_REQUIRE(ns >= 1 && nhyp >= 1, "icp: need ns >= 1 and nhyp >= 1");
     PCREG_REQUIRE(o.iters >= 0, "icp: iters must be >= 0");
     PCREG_REQUIRE(o.mode >= PCREG_ICP_PLAIN && o.mode <= PCREG_ICP_WEIGHTED, "icp: bad mode");
@@ -443,7 +465,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     const double t_enter = now_ms();
     double t_alloc = 0, t_sorted = 0, t_enq = 0;
 
-    const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop != nullptr, plane);
+    const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop != nullptr, metric);
     // chunk the hypotheses so that the per-correspondence scratch stays bounded
     const size_t total_b = c.total_mem;         // queried once at pcreg_init (cudaMemGetInfo costs up to tens of ms per call)
     const size_t per_hyp = (size_t)ns * (4 + 4 + 8 + (o.mode == PCREG_ICP_KNN ? 8 : 0) + (o.nn == PCREG_NN_GRID ? 8 + (m->has_vox ? 0 : 28 + 4 * 64 + 4 * 448 / 16) : 0));
@@ -562,6 +584,22 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         d_src = src_sorted.p;
         if (d_w) d_w = w_sorted.p;
     }
+    // plane-to-plane: the source normals normalised and checked on the device, in the order of the source arrays.  The flag is read
+    // before any ICP kernel runs, so a bad normal never reaches them.
+    DevBuf<double> snrm(gicp ? (size_t)ns * 3 : 0);
+    if (gicp) {
+        DevBuf<int> bad(1);
+        int h_bad = 0;
+        PCREG_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), st));
+        k_src_normals<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(d_src_nrm, sorted ? sperm.p : nullptr, ns, snrm.p, bad.p);
+        PCREG_LAUNCHED();
+        PCREG_CUDA(cudaMemcpyAsync(&h_bad, bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+        PCREG_CUDA(cudaStreamSynchronize(st));
+        PCREG_REQUIRE(!h_bad, "icp: zero or non-finite source normal");
+    }
+    const double* snx = gicp ? snrm.p : nullptr;
+    const double* sny = gicp ? snrm.p + ns : nullptr;
+    const double* snz = gicp ? snrm.p + 2 * ns : nullptr;
     t_sorted = now_ms();
     const double* sx = d_src; const double* sy = d_src + ns; const double* sz = d_src + 2 * ns;
     if (fused) {
@@ -576,6 +614,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         fa.mode = o.mode; fa.k_frac = o.k_frac; fa.R_w = o.R_w; fa.thDist2 = o.thDist2; fa.reflection_fix = o.reflection_fix; fa.iters = o.iters;
         fa.counters = (prof && c.profiling_counters) ? counters.p : nullptr;
         fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
+        fa.snx = snx; fa.sny = sny; fa.snz = snz; fa.gicp_eps = gicp_eps;
         ev_begin(0);
         icp_fused_launch(fa, nhyp, stop != nullptr, st);
         ev_end();
@@ -657,6 +696,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                 nn_launches += 1;
                 IcpUpdateArgs ua{};
                 ua.md = m->md.p; ua.nrm = nrm;
+                ua.snx = snx; ua.sny = sny; ua.snz = snz; ua.gicp_eps = gicp_eps;
                 for (int k = 0; k < 3; ++k) ua.pivot[k] = m->pivot[k];
                 ua.sx = sx; ua.sy = sy; ua.sz = sz; ua.w_src = d_w; ua.ns = ns;
                 ua.T = Twork.p + h0 * 16; ua.idx = out_idx; ua.d2 = L.d2.p; ua.keys = L.keys.p;
@@ -801,18 +841,21 @@ int pcreg_icp_batch_stop_dev(const pcreg_model* m, const double* d_src, int64_t 
 static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>& hs, int64_t ns, const double* w_src,
                                  const double* T0_16, int64_t h0, int64_t hn, const pcreg_icp_opts& o, double* T16, double* rmse,
                                  int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
-                                 const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric) {
+                                 const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric,
+                                 const std::vector<double>& hnrm, double gicp_eps) {
     PCREG_CUDA(cudaSetDevice(ctx().device));
     cudaStream_t st = 0;
     DevBuf<double> d_src((size_t)ns * 3), d_w(w_src ? (size_t)ns : 0), d_T0((size_t)hn * 16), d_T((size_t)hn * 16);
+    DevBuf<double> d_nrm(hnrm.size());                  // plane-to-plane: the source normals, copied to every device as the source is
     DevBuf<double> d_rmse((size_t)hn), d_hist(rmse_hist ? (size_t)hn * (o.iters + 1) : 0);
     DevBuf<int32_t> d_nu((size_t)hn), d_st((size_t)hn), d_idx(idx ? (size_t)hn * ns : 0);
     DevBuf<int32_t> d_nit(n_iter ? (size_t)hn : 0), d_conv(converged ? (size_t)hn : 0);
     PCREG_CUDA(cudaMemcpyAsync(d_src.p, hs.data(), d_src.bytes(), cudaMemcpyHostToDevice, st));
     if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src, d_w.bytes(), cudaMemcpyHostToDevice, st));
+    if (d_nrm.p) PCREG_CUDA(cudaMemcpyAsync(d_nrm.p, hnrm.data(), d_nrm.bytes(), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
     icp_run(m, d_src.p, ns, w_src ? d_w.p : nullptr, d_T0.p, hn, o, d_T.p, d_rmse.p, d_nu.p, d_st.p,
-            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st, stop, d_nit.p, d_conv.p, metric);
+            idx ? d_idx.p : nullptr, rmse_hist ? d_hist.p : nullptr, nullptr, st, stop, d_nit.p, d_conv.p, metric, d_nrm.p, gicp_eps);
     PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
@@ -824,15 +867,18 @@ static void icp_batch_host_slice(const pcreg_model* m, const std::vector<double>
     PCREG_CUDA(cudaStreamSynchronize(st));
 }
 
-// pcreg_icp_batch, pcreg_icp_batch_stop (stop != nullptr) and pcreg_icp_batch_metric
+// pcreg_icp_batch, pcreg_icp_batch_stop (stop != nullptr), pcreg_icp_batch_metric and pcreg_icp_batch_gicp (src_nrm: the source
+// normals, same type and ld as src)
 static int icp_batch_host(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
                           const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts, double* T16, double* rmse,
                           int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist, int64_t* best,
-                          const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric = PCREG_ICP_POINT_TO_POINT) {
+                          const pcreg_icp_stop* stop, int32_t* n_iter, int32_t* converged, int metric = ICP_M_POINT,
+                          const void* src_nrm = nullptr, double gicp_eps = 0.0) {
     require_init();
     PCREG_REQUIRE(m && src && T0_16 && T16 && opts, "pcreg_icp_batch: null pointer");
     PCREG_REQUIRE(ns >= 1 && ld >= ns && nhyp >= 1, "pcreg_icp_batch: bad sizes");
     const std::vector<double> hs = to_double_cm(src, is_double, ns, ld);
+    const std::vector<double> hnrm = src_nrm ? to_double_cm(src_nrm, is_double, ns, ld) : std::vector<double>();
     std::vector<double> rmse_tmp(rmse ? 0 : (size_t)nhyp);
     double* rm = rmse ? rmse : rmse_tmp.data();
     // Hypotheses are independent (the reference runs them under parfor: slideMatchingWindow_v2.m:178, completeExperiment.m:265):
@@ -847,11 +893,11 @@ static int icp_batch_host(const pcreg_model* m, const void* src, int is_double, 
         if (hn <= 0) continue;
         workers.emplace_back([&, k, h0, hn]() {
             rc[k] = guarded([&]() { use_slot(k); icp_batch_host_slice(m->on_slot(k), hs, ns, w_src, T0_16, h0, hn, *opts, T16, rm, n_used, status, idx, rmse_hist,
-                                                                 stop, n_iter, converged, metric); });
+                                                                 stop, n_iter, converged, metric, hnrm, gicp_eps); });
         });
     }
     rc[0] = guarded([&]() { use_slot(0); icp_batch_host_slice(m, hs, ns, w_src, T0_16, 0, std::min(per, nhyp), *opts, T16, rm, n_used, status, idx, rmse_hist,
-                                                         stop, n_iter, converged, metric); });
+                                                         stop, n_iter, converged, metric, hnrm, gicp_eps); });
     for (auto& w : workers) w.join();
     use_slot(0);
     for (int k = 0; k < nd; ++k) if (rc[k] != PCREG_OK) return rc[k];
@@ -910,6 +956,38 @@ int pcreg_icp_batch_metric_dev(const pcreg_model* m, const double* d_src, int64_
     PCREG_CUDA(cudaSetDevice(ctx().device));
     icp_run(m, d_src, ns, d_w_src, d_T0_16, nhyp, *opts, d_T16, d_rmse, d_n_used, d_status, d_idx, d_rmse_hist,
             d_best, (cudaStream_t)stream, stop, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, metric);
+    return PCREG_OK;
+    PCREG_API_END
+}
+
+static void check_gicp(const void* src_nrm, double eps, const pcreg_icp_stop* stop) {
+    PCREG_REQUIRE(src_nrm, "pcreg_icp_batch_gicp: the source normals are null");
+    PCREG_REQUIRE(std::isfinite(eps) && eps > 0.0 && eps <= 1.0, "pcreg_icp_batch_gicp: eps must be finite and in (0, 1]");
+    if (stop) check_stop(stop);
+}
+
+int pcreg_icp_batch_gicp(const pcreg_model* m, const void* src, int is_double, int64_t ns, int64_t ld, const double* w_src,
+                         const void* src_nrm, double eps, const double* T0_16, int64_t nhyp, const pcreg_icp_opts* opts,
+                         const pcreg_icp_stop* stop, double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx,
+                         double* rmse_hist, int64_t* best, int32_t* n_iter, int32_t* converged) {
+    PCREG_API_BEGIN
+    check_gicp(src_nrm, eps, stop);
+    return icp_batch_host(m, src, is_double, ns, ld, w_src, T0_16, nhyp, opts, T16, rmse, n_used, status, idx, rmse_hist, best,
+                          stop, stop ? n_iter : nullptr, stop ? converged : nullptr, ICP_M_GICP, src_nrm, eps);
+    PCREG_API_END
+}
+
+int pcreg_icp_batch_gicp_dev(const pcreg_model* m, const double* d_src, int64_t ns, const double* d_w_src, const double* d_src_nrm,
+                             double eps, const double* d_T0_16, int64_t nhyp, const pcreg_icp_opts* opts, const pcreg_icp_stop* stop,
+                             double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
+                             double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    PCREG_REQUIRE(opts, "pcreg_icp_batch_gicp_dev: opts is null");
+    check_gicp(d_src_nrm, eps, stop);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    icp_run(m, d_src, ns, d_w_src, d_T0_16, nhyp, *opts, d_T16, d_rmse, d_n_used, d_status, d_idx, d_rmse_hist,
+            d_best, (cudaStream_t)stream, stop, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, ICP_M_GICP, d_src_nrm, eps);
     return PCREG_OK;
     PCREG_API_END
 }

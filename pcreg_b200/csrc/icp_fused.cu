@@ -46,23 +46,23 @@ __device__ __noinline__ void fused_walk(const GridArgs& a, double qx, double qy,
     walk_search<false>(a, 0, Q, false, lc, ext_slot, thr2, 0.f, n1, n2, n3);
     bidx = Q.bidx; best = Q.best;
 }
-template <bool PLANE>
-__device__ __noinline__ bool fused_pose_update(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot, bool reflection_fix,
+template <int METRIC>
+__device__ __noinline__ bool fused_pose_update(const double (&s)[icp_nsums<METRIC>], long long n_used, const double* pivot, bool reflection_fix,
                                                double* Ts /*shared, row-major 4x4, updated in place*/) {
     double Tc[16], Tn[16];
     for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
-    if (!icp_pose_update_m<PLANE>(s, n_used, pivot, reflection_fix, Tc, Tn)) return false;
+    if (!icp_pose_update_m<METRIC>(s, n_used, pivot, reflection_fix, Tc, Tn)) return false;
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return true;
 }
 // Tolerance stop: the update of pass `it` (update it + 1) and the stop rule.  0: degenerate, pose left alone; 1: pose updated;
 // 2: pose updated and the rule says stop.
-template <bool PLANE>
-__device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot, bool reflection_fix,
+template <int METRIC>
+__device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<METRIC>], long long n_used, const double* pivot, bool reflection_fix,
                                                    const IcpStopRule& rule, int it, double* ring /*shared*/, double* Ts /*shared*/) {
     double Tc[16], Tn[16];
     for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
-    if (!icp_pose_update_m<PLANE>(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
+    if (!icp_pose_update_m<METRIC>(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
 }
@@ -70,10 +70,11 @@ __device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<P
 // KNN = the trimmed mode (its selection scratch -- 18 KB of shared memory -- exists only in that instantiation).
 // STOP = the tolerance stop (pcreg_icp_batch_stop): a stop -- by the rule or by a degenerate update -- makes the block's next
 // pass its final scoring pass, after which the block exits.  The STOP = false instantiations are the loop without it.
-// PLANE = the point-to-plane metric (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered there.
-template <bool KNN, bool STOP, bool PLANE>
+// METRIC = 0 point-to-point; 1 point-to-plane (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered
+// there; 2 plane-to-plane (pcreg_icp_batch_gicp): the same, and the source normal of each correspondence rotated by the pose.
+template <bool KNN, bool STOP, int METRIC>
 __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ FusedArgs a) {
-    constexpr int NS = icp_nsums<PLANE>;
+    constexpr int NS = icp_nsums<METRIC>;
     extern __shared__ __align__(16) unsigned char dyn[];
     __shared__ double Ts[16];
     __shared__ double red[NS * 32];
@@ -93,7 +94,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     const GridPoint* __restrict__ pts = a.g.g.pts;
     const bool reject = a.thDist2 > 0.0;
     constexpr bool knn = KNN;
-    constexpr bool two_pass = KNN || PLANE || !FUSED_INLINE_SUMS;      // sums in a pass of their own (needed after a trim selection)
+    constexpr bool two_pass = KNN || METRIC != ICP_M_POINT || !FUSED_INLINE_SUMS;      // sums in a pass of their own (needed after a trim selection)
     const double px = a.pivot[0], py = a.pivot[1], pz = a.pivot[2];
     unsigned long long c_read = 0, c_gather = 0, c_walk = 0;
     long long t_nn = 0, t_sel = 0, t_sum = 0, t_svd = 0, t_mark = 0;       // phase clocks of thread 0 (profiling only)
@@ -213,7 +214,9 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 const double d = j >= 0 ? dist2_exact(m.x, m.y, m.z, qx, qy, qz) : (double)INFINITY;      // the NN step's d2, bit for bit
                 const double w = weight_of(i, j, d);
                 if (w > 0.0) ++n_used;
-                if constexpr (PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
+                if constexpr (METRIC == ICP_M_GICP)
+                    icp_accumulate_gicp(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], a.snx[i], a.sny[i], a.snz[i], Ts, a.gicp_eps, px, py, pz);
+                else if constexpr (METRIC == ICP_M_PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
                 else icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
             }
         }
@@ -235,9 +238,9 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             }
             if (!last && !s_frozen) {
                 if (!STOP) {
-                    if (!fused_pose_update<PLANE>(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
+                    if (!fused_pose_update<METRIC>(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
                 } else {
-                    const int r = fused_pose_update_stop<PLANE>(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
+                    const int r = fused_pose_update_stop<METRIC>(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
                     if (r == 0) s_frozen = 1;
                     if (r != 1) s_stop = 1;
                 }
@@ -276,9 +279,15 @@ size_t icp_fused_smem(int64_t ns, int mode) {
     return (((size_t)ns * 4 + 15) / 16) * 16 + (mode == PCREG_ICP_KNN ? (size_t)ns * 8 : 0);
 }
 
-// Point-to-point calls keep the check they always had (the static shared memory of k_icp_fused<true, false, false>); a
-// point-to-plane call checks the instantiation it launches (its reduction buffer is 29 instead of 17 doubles x 32).
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, bool plane) {
+template <int METRIC>
+static const void* fused_kernel(bool knn, bool stop) {
+    return knn ? (stop ? (const void*)k_icp_fused<true, true, METRIC> : (const void*)k_icp_fused<true, false, METRIC>)
+               : (stop ? (const void*)k_icp_fused<false, true, METRIC> : (const void*)k_icp_fused<false, false, METRIC>);
+}
+
+// Point-to-point calls keep the check they always had (the static shared memory of k_icp_fused<true, false, 0>); the other metrics
+// check the instantiation they launch (their reduction buffer is 29 instead of 17 doubles x 32).
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, int metric) {
     if (!m->has_vox || o.nn != PCREG_NN_GRID) return false;
     if (const char* e = getenv("PCREG_FUSED")) { if (e[0] == '0') return false; if (e[0] == '1') nhyp = (int64_t)1 << 40; }
     // one block per hypothesis: a batch smaller than the SM count leaves SMs idle, the per-pass kernels (all SMs on every
@@ -286,33 +295,33 @@ bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pc
     if (nhyp < ctx().sm_count) return false;
     if (ns >= ((int64_t)1 << 30)) return false;
     const bool knn = o.mode == PCREG_ICP_KNN;
-    const void* fn = !plane ? (const void*)k_icp_fused<true, false, false>
-                   : knn ? (stop ? (const void*)k_icp_fused<true, true, true> : (const void*)k_icp_fused<true, false, true>)
-                         : (stop ? (const void*)k_icp_fused<false, true, true> : (const void*)k_icp_fused<false, false, true>);
+    const void* fn = metric == ICP_M_POINT ? (const void*)k_icp_fused<true, false, ICP_M_POINT>
+                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE>(knn, stop) : fused_kernel<ICP_M_GICP>(knn, stop);
     cudaFuncAttributes fa;
     if (cudaFuncGetAttributes(&fa, fn) != cudaSuccess) { cudaGetLastError(); return false; }
     return icp_fused_smem(ns, o.mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
 }
 
-template <bool KNN, bool STOP, bool PLANE>
+template <bool KNN, bool STOP, int METRIC>
 static void fused_launch_one(const FusedArgs& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
-    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, PLANE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    k_icp_fused<KNN, STOP, PLANE><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    k_icp_fused<KNN, STOP, METRIC><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
 }
 
-template <bool PLANE>
+template <int METRIC>
 static void fused_launch_metric(const FusedArgs& a, int64_t nhyp, bool stop, size_t dyn, cudaStream_t st) {
     const bool knn = a.mode == PCREG_ICP_KNN;
-    if (knn && !stop)       fused_launch_one<true, false, PLANE>(a, nhyp, dyn, st);
-    else if (!knn && !stop) fused_launch_one<false, false, PLANE>(a, nhyp, dyn, st);
-    else if (knn)           fused_launch_one<true, true, PLANE>(a, nhyp, dyn, st);
-    else                    fused_launch_one<false, true, PLANE>(a, nhyp, dyn, st);
+    if (knn && !stop)       fused_launch_one<true, false, METRIC>(a, nhyp, dyn, st);
+    else if (!knn && !stop) fused_launch_one<false, false, METRIC>(a, nhyp, dyn, st);
+    else if (knn)           fused_launch_one<true, true, METRIC>(a, nhyp, dyn, st);
+    else                    fused_launch_one<false, true, METRIC>(a, nhyp, dyn, st);
 }
 
 void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
-    if (a.nrm) fused_launch_metric<true>(a, nhyp, stop, dyn, st);
-    else       fused_launch_metric<false>(a, nhyp, stop, dyn, st);
+    if (a.snx)      fused_launch_metric<ICP_M_GICP>(a, nhyp, stop, dyn, st);
+    else if (a.nrm) fused_launch_metric<ICP_M_PLANE>(a, nhyp, stop, dyn, st);
+    else            fused_launch_metric<ICP_M_POINT>(a, nhyp, stop, dyn, st);
     PCREG_LAUNCHED();
 }
 

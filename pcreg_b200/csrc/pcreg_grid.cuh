@@ -53,9 +53,11 @@ struct FusedArgs {
     IcpStopRule stop;                       // tolerance stop (the k_icp_fused<*, true> instantiations only)
     int32_t* n_iter; int32_t* converged;    // [nhyp] optional outputs of the tolerance stop
     const ModelPointD* nrm;                 // model normals (original order): the point-to-plane metric; null: point-to-point
+    // plane-to-plane metric (null: the other two): unit source normals in the order of sx / sy / sz, and the covariance epsilon
+    const double* snx; const double* sny; const double* snz; double gicp_eps;
 };
 size_t icp_fused_smem(int64_t ns, int mode);
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, bool plane);
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, int metric);
 void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
 
 __device__ __forceinline__ void flush_counters(unsigned long long* counters, unsigned long long n_pts,

@@ -108,12 +108,28 @@ __device__ __noinline__ static bool icp_pose_update_plane_call(const double (&s)
     return icp_pose_update_plane(s, n_used, pivot, Tc, Tn);
 }
 
-// sums of one ICP pass: 17 (point-to-point, Kabsch) or 29 (point-to-plane); the last one is sum w d^2 in both
-template <bool PLANE> constexpr int icp_nsums = PLANE ? PLANE_NSUMS : KABSCH_NSUMS;
-template <bool PLANE>
-__device__ __forceinline__ bool icp_pose_update_m(const double (&s)[icp_nsums<PLANE>], long long n_used, const double* pivot,
+// Plane-to-plane metric (pcreg_icp_batch_gicp): sn = the source normal of the correspondence's source point, carried by the
+// current pose Ts (row-major, row-vector: n_q = n_s R); the arithmetic is gicp_accumulate (pcreg_math.cuh), which both kernels call
+// in the same thread order.
+__device__ __forceinline__ void icp_accumulate_gicp(double (&s)[PLANE_NSUMS], double w, double d, double qx, double qy, double qz,
+                                                    const ModelPointD& m, const ModelPointD& n, double snx, double sny, double snz,
+                                                    const double* Ts, double eps, double px, double py, double pz) {
+    const double qt[3] = {qx - px, qy - py, qz - pz}, mt[3] = {m.x - px, m.y - py, m.z - pz};
+    const double nm[3] = {n.x, n.y, n.z};
+    double nq[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) nq[c] = snx * Ts[0 * 4 + c] + sny * Ts[1 * 4 + c] + snz * Ts[2 * 4 + c];
+    gicp_accumulate(s, w, d, qt, mt, nq, nm, eps);
+}
+
+// ICP metrics of the kernels' METRIC template parameter: 0 point-to-point (17 sums, Kabsch), 1 point-to-plane and 2 plane-to-plane
+// (29 sums, the LDL' step); the last sum is sum w d^2 in all of them
+constexpr int ICP_M_POINT = 0, ICP_M_PLANE = 1, ICP_M_GICP = 2;
+template <int METRIC> constexpr int icp_nsums = METRIC != ICP_M_POINT ? PLANE_NSUMS : KABSCH_NSUMS;
+template <int METRIC>
+__device__ __forceinline__ bool icp_pose_update_m(const double (&s)[icp_nsums<METRIC>], long long n_used, const double* pivot,
                                                   bool reflection_fix, const double* Tc, double* Tn) {
-    if constexpr (PLANE) return icp_pose_update_plane(s, n_used, pivot, Tc, Tn);
+    if constexpr (METRIC != ICP_M_POINT) return icp_pose_update_plane(s, n_used, pivot, Tc, Tn);
     else return icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn);
 }
 

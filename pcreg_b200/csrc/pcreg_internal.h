@@ -275,7 +275,9 @@ struct IcpUpdateArgs {
     double* stop_ring;          // [nhyp][2 * ICP_STOP_WINDOW_MAX] motion of the last `window` updates
     IcpStopRule stop;
     int32_t* n_iter; int32_t* converged;   // [nhyp] optional, written by the final pass
-    const pcreg::ModelPointD* nrm;         // model normals (original order): the point-to-plane metric (k_icp_update<*, *, true>)
+    const pcreg::ModelPointD* nrm;         // model normals (original order): the point-to-plane metric (k_icp_update<*, *, 1>)
+    // plane-to-plane metric (k_icp_update<*, *, 2>; null otherwise): unit source normals in the order of sx / sy / sz, covariance epsilon
+    const double* snx; const double* sny; const double* snz; double gicp_eps;
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
 void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st);

@@ -285,6 +285,48 @@ PCREG_HD void rodrigues(const double* w, double* R) {
     for (int i = 0; i < 9; ++i) R[i] += a * K[i] + b * K2[i];
 }
 
+// ---- plane-to-plane (generalized ICP) step (include/pcreg.h: pcreg_icp_batch_gicp) ----
+// One correspondence of weight w into the 29 sums of the point-to-plane layout.  qt = q - p, mt = m - p (p the pivot), nq the
+// source normal carried by the pose, nm the model normal, eps in (0, 1]:
+//   C = 2I - (1 - eps)(nm nm' + nq nq'),  M = C^-1 = adj(C) / det(C),  e = mt - qt,  J' = [[qt]x; I]  (6 x 3),
+//   A += w J' M J = w [[qt]x M [qt]x', [qt]x M; M [qt]x', M]  (upper triangle, row-major),  g += w J' M e = w (qt x Me, Me).
+// With M = n n' this is the point-to-plane accumulation: J' n = (qt x n, n) is its a and n' e its b.  C enters only through the
+// products n_i n_j, so the sign of either normal changes no bit.  s[0] += w and s[28] += w d as in the other metrics.
+PCREG_HD void gicp_accumulate(double* s, double w, double d, const double* qt, const double* mt, const double* nq, const double* nm,
+                              double eps) {
+    const double a = 1.0 - eps;
+    const double c00 = 2.0 - a * (nm[0] * nm[0] + nq[0] * nq[0]), c11 = 2.0 - a * (nm[1] * nm[1] + nq[1] * nq[1]);
+    const double c22 = 2.0 - a * (nm[2] * nm[2] + nq[2] * nq[2]);
+    const double c01 = -a * (nm[0] * nm[1] + nq[0] * nq[1]), c02 = -a * (nm[0] * nm[2] + nq[0] * nq[2]);
+    const double c12 = -a * (nm[1] * nm[2] + nq[1] * nq[2]);
+    const double a00 = c11 * c22 - c12 * c12, a01 = c02 * c12 - c01 * c22, a02 = c01 * c12 - c02 * c11;
+    const double a11 = c00 * c22 - c02 * c02, a12 = c01 * c02 - c00 * c12, a22 = c00 * c11 - c01 * c01;
+    const double f = w / (c00 * a00 + c01 * a01 + c02 * a02);              // w / det(C): w M = f adj(C)
+    const double M[9] = {f * a00, f * a01, f * a02, f * a01, f * a11, f * a12, f * a02, f * a12, f * a22};
+    const double e[3] = {mt[0] - qt[0], mt[1] - qt[1], mt[2] - qt[2]};
+    double Me[3], P[9];                                                    // w M e and P = [qt]x w M (row-major)
+    for (int r = 0; r < 3; ++r) Me[r] = M[r * 3 + 0] * e[0] + M[r * 3 + 1] * e[1] + M[r * 3 + 2] * e[2];
+    for (int c = 0; c < 3; ++c) {
+        P[0 * 3 + c] = qt[1] * M[2 * 3 + c] - qt[2] * M[1 * 3 + c];
+        P[1 * 3 + c] = qt[2] * M[0 * 3 + c] - qt[0] * M[2 * 3 + c];
+        P[2 * 3 + c] = qt[0] * M[1 * 3 + c] - qt[1] * M[0 * 3 + c];
+    }
+    // [qt]x w M [qt]x' = P [qt]x': entry (r, c) is (qt x row r of P)_c
+    const double T00 = qt[1] * P[2] - qt[2] * P[1], T01 = qt[2] * P[0] - qt[0] * P[2], T02 = qt[0] * P[1] - qt[1] * P[0];
+    const double T11 = qt[2] * P[3] - qt[0] * P[5], T12 = qt[0] * P[4] - qt[1] * P[3];
+    const double T22 = qt[0] * P[7] - qt[1] * P[6];
+    s[0] += w;
+    s[1] += T00; s[2] += T01; s[3] += T02; s[4] += P[0]; s[5] += P[1]; s[6] += P[2];
+    s[7] += T11; s[8] += T12; s[9] += P[3]; s[10] += P[4]; s[11] += P[5];
+    s[12] += T22; s[13] += P[6]; s[14] += P[7]; s[15] += P[8];
+    s[16] += M[0]; s[17] += M[1]; s[18] += M[2];
+    s[19] += M[4]; s[20] += M[5];
+    s[21] += M[8];
+    s[22] += qt[1] * Me[2] - qt[2] * Me[1]; s[23] += qt[2] * Me[0] - qt[0] * Me[2]; s[24] += qt[0] * Me[1] - qt[1] * Me[0];
+    s[25] += Me[0]; s[26] += Me[1]; s[27] += Me[2];
+    s[28] += w * d;
+}
+
 // MATLAB eps(x) for x >= 0: spacing of doubles at x.
 PCREG_HD double spacing(double x) {
     if (!(x > 0.0)) return 4.9406564584124654e-324;

@@ -7,7 +7,7 @@ import ctypes as C
 import torch
 
 from . import _lib as L
-from .api import METRICS, Model, icp_opts
+from .api import GICP_EPS, METRICS, PLANE_TO_PLANE, Model, icp_opts
 
 
 def T_to_abi_t(T: torch.Tensor) -> torch.Tensor:
@@ -46,12 +46,13 @@ def _p(t):
 
 
 def icp_batch_device(model: Model, src_cm: torch.Tensor, w_src, T0_abi: torch.Tensor, opts, out: IcpDeviceBuffers,
-                     stream=None, stop=None, metric="point_to_point"):
+                     stream=None, stop=None, metric="point_to_point", src_normals=None, gicp_eps=GICP_EPS):
     """Run pcreg_icp_batch_dev on tensors already resident on the library's device.
 
     src_cm: float64 [3, ns] (column-major ns x 3); T0_abi: float64 [H,16] column-major records.
     stop: an api.icp_stop(tol_t, tol_r_deg, window) -> pcreg_icp_batch_stop_dev (out.n_iter / out.converged, when allocated,
-    receive the stop outputs).  metric="point_to_plane" -> pcreg_icp_batch_metric_dev (needs model normals)."""
+    receive the stop outputs).  metric="point_to_plane" -> pcreg_icp_batch_metric_dev (needs model normals).
+    metric="plane_to_plane" -> pcreg_icp_batch_gicp_dev: needs model normals and src_normals, a CUDA float64 [ns, 3] tensor."""
     if not (src_cm.is_cuda and T0_abi.is_cuda):
         raise L.PcregError("icp_batch_device needs CUDA tensors (there is no CPU fallback)")
     assert src_cm.dtype == torch.float64 and src_cm.is_contiguous() and src_cm.shape[0] == 3
@@ -59,7 +60,18 @@ def icp_batch_device(model: Model, src_cm: torch.Tensor, w_src, T0_abi: torch.Te
     ns = src_cm.shape[1]
     nhyp = T0_abi.shape[0]
     st = stream if stream is not None else torch.cuda.current_stream()
-    if metric != "point_to_point":
+    if metric == PLANE_TO_PLANE:
+        if src_normals is None:
+            raise ValueError("metric='plane_to_plane' needs src_normals (a CUDA float64 [ns, 3] tensor)")
+        if not (src_normals.is_cuda and src_normals.dtype == torch.float64 and tuple(src_normals.shape) == (ns, 3)):
+            raise ValueError("src_normals must be a CUDA float64 [ns, 3] tensor")
+        sn_cm = src_normals.t().contiguous()                   # column-major ns x 3, ld = ns
+        L.check(L.lib().pcreg_icp_batch_gicp_dev(model.handle, _p(src_cm), ns, _p(w_src), _p(sn_cm), float(gicp_eps), _p(T0_abi), nhyp,
+                                                 C.byref(opts), C.byref(stop) if stop is not None else None, _p(out.T),
+                                                 _p(out.rmse), _p(out.n_used), _p(out.status), _p(out.idx), _p(out.hist),
+                                                 _p(out.best), _p(out.n_iter), _p(out.converged), C.c_void_p(st.cuda_stream)),
+                "pcreg_icp_batch_gicp_dev")
+    elif metric != "point_to_point":
         L.check(L.lib().pcreg_icp_batch_metric_dev(model.handle, _p(src_cm), ns, _p(w_src), _p(T0_abi), nhyp, C.byref(opts),
                                                    METRICS[metric], C.byref(stop) if stop is not None else None, _p(out.T),
                                                    _p(out.rmse), _p(out.n_used), _p(out.status), _p(out.idx), _p(out.hist),
