@@ -42,7 +42,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
     constexpr int NS = icp_nsums<METRIC>;
     constexpr bool MNRM = METRIC != ICP_M_POINT, SNRM = METRIC == ICP_M_GICP;
     __shared__ double Ts[16];
-    __shared__ double red[NS * 32];
+    __shared__ double red[(NS + 1) * 32];
     __shared__ long long redll[32];
     __shared__ HistSelShared hsel;
     __shared__ unsigned long long red_u64[64];
@@ -169,8 +169,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             else icp_accumulate(s, w, d, qx, qy, qz, mm[u], px, py, pz);
         }
     }
-    block_sum<NS>(s, red);
-    n_used = block_sum_ll(n_used, redll);
+    n_used = block_sum_count<NS>(s, n_used, red);
 
     if (tid == 0) {
         const double sw = s[0];

@@ -77,10 +77,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     constexpr int NS = icp_nsums<METRIC>;
     extern __shared__ __align__(16) unsigned char dyn[];
     __shared__ double Ts[16];
-    __shared__ double red[NS * 32];
-    __shared__ long long redll[32];
+    __shared__ double red[(NS + 1) * 32];
     __shared__ HistSelShared hsel;
-    __shared__ unsigned long long red_u64[64];
     __shared__ int s_frozen;
     __shared__ int s_stop;                                  // STOP: the next pass is the final one
     __shared__ double s_ring[2 * ICP_STOP_WINDOW_MAX];      // STOP: thread 0's window of update motions
@@ -102,19 +100,23 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
 
     if (tid < 16) Ts[tid] = a.T[h * 16 + tid];
     if (tid == 0) { s_frozen = a.frozen[h]; if (STOP) s_stop = 0; }
+    if (KNN) for (int b = tid; b < SEL_BINS; b += UPD_THREADS) hsel.hist[b] = 0;     // block_hist_finish leaves it zero after
     __syncthreads();
+    // trimmed mode: the K-th residual key of the last pass (0: none yet, or nothing selected); the next pass centres its
+    // histogram window on it
+    unsigned long long vK = 0ull;
+    bool all_eq = false;
 
     for (int it = 0; it <= a.iters; ++it) {
         const bool last = it == a.iters || (STOP && s_stop);     // block-uniform: s_stop was written before the last barrier
         // ---- exact nearest neighbours of the hypothesis' ns queries (two per trip: their header / entry loads overlap) ----
-        long long nkept = 0;
-        unsigned long long kmin = ~0ull, kmax = 0ull;
         double s[NS];
 #pragma unroll
         for (int k = 0; k < NS; ++k) s[k] = 0.0;
         long long n_used = 0;
-        unsigned long long vK = 0ull;
-        bool all_eq = false;
+        // trim histogram, filled where the keys are produced: a range-free monotone bin map (exact at any scale; the window
+        // only decides how many keys share the boundary bin)
+        const SelBinsShift bins = SelBinsShift::around(vK);
         auto weight_of = [&](int i, int32_t j, double d) -> double {
             const bool keep = j >= 0 && (!reject || d < a.thDist2);
             double w = 0.0;
@@ -165,38 +167,25 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 const bool keep0 = b0 >= 0 && (!reject || d0 < a.thDist2);
                 const unsigned long long key0 = keep0 ? dbits(__dsqrt_rn(d0)) : KEY_NOSEL;
                 keys_s[i0] = key0;
-                if (keep0) { ++nkept; kmin = key0 < kmin ? key0 : kmin; kmax = key0 > kmax ? key0 : kmax; }
+                if (keep0) atomicAdd(&hsel.hist[bins(key0)], 1);
                 if (has1) {
                     const bool keep1 = b1 >= 0 && (!reject || d1 < a.thDist2);
                     const unsigned long long key1 = keep1 ? dbits(__dsqrt_rn(d1)) : KEY_NOSEL;
                     keys_s[i1] = key1;
-                    if (keep1) { ++nkept; kmin = key1 < kmin ? key1 : kmin; kmax = key1 > kmax ? key1 : kmax; }
+                    if (keep1) atomicAdd(&hsel.hist[bins(key1)], 1);
                 }
             }
         }
         __syncthreads();
         if (timing) { const long long t = clock64(); t_nn += t - t_mark; t_mark = t; }
         // ---- trim: the round(k_frac * kept) smallest residuals, stable tie rule (AlignPoints_KNN.m:20-26) ----
+        // (the histogram's total is the number of kept residuals)
         if (knn) {
-            nkept = block_sum_ll(nkept, redll);
-            const int lane = tid & 31, warp = tid >> 5;
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                const unsigned long long a0 = __shfl_xor_sync(0xffffffffu, kmin, o), a1 = __shfl_xor_sync(0xffffffffu, kmax, o);
-                kmin = a0 < kmin ? a0 : kmin;
-                kmax = a1 > kmax ? a1 : kmax;
-            }
-            if (lane == 0) { red_u64[warp] = kmin; red_u64[32 + warp] = kmax; }
-            __syncthreads();
-            kmin = ~0ull; kmax = 0ull;
-            for (int w = 0; w < UPD_THREADS / 32; ++w) {
-                kmin = red_u64[w] < kmin ? red_u64[w] : kmin;
-                kmax = red_u64[32 + w] > kmax ? red_u64[32 + w] : kmax;
-            }
-            __syncthreads();
-            long long K = (long long)floor(a.k_frac * (double)nkept + 0.5);     // MATLAB round (AlignPoints_KNN.m:21)
-            if (K > nkept) K = nkept;
-            block_hist_select(keys_s, ns, K, kmin, kmax, hsel, vK, all_eq, a.tie_order);
+            const auto k_of_kept = [&](long long nkept) {
+                const long long K = (long long)floor(a.k_frac * (double)nkept + 0.5);     // MATLAB round (AlignPoints_KNN.m:21)
+                return K > nkept ? nkept : K;
+            };
+            block_hist_finish(keys_s, ns, bins, k_of_kept, hsel, vK, all_eq, a.tie_order);
         }
         if (timing) { const long long t = clock64(); t_sel += t - t_mark; t_mark = t; }
         // ---- weights + the 17 sums (thread t: correspondences t, t + UPD_THREADS, ... in this order, as k_icp_update) ----
@@ -220,8 +209,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 else icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
             }
         }
-        block_sum<NS>(s, red);
-        n_used = block_sum_ll(n_used, redll);
+        n_used = block_sum_count<NS>(s, n_used, red);
         if (timing) { const long long t = clock64(); t_sum += t - t_mark; t_mark = t; }
         if (tid == 0) {
             const double sw = s[0];

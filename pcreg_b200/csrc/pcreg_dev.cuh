@@ -66,6 +66,21 @@ __device__ __forceinline__ void block_sum(double (&v)[NV], double* scratch) {
     __syncthreads();
 }
 
+// block_sum of NV doubles and one per-thread count, reduced as one more double in the same pass (exact: a count is an
+// integer far below 2^53).  Every sum goes through the same tree as in block_sum<NV>.  `scratch` must hold (NV + 1) * 32
+// doubles.  Returns the block's count in every thread.
+template <int NV>
+__device__ __forceinline__ long long block_sum_count(double (&v)[NV], long long count, double* scratch) {
+    double x[NV + 1];
+#pragma unroll
+    for (int k = 0; k < NV; ++k) x[k] = v[k];
+    x[NV] = (double)count;
+    block_sum<NV + 1>(x, scratch);
+#pragma unroll
+    for (int k = 0; k < NV; ++k) v[k] = x[k];
+    return (long long)x[NV];
+}
+
 __device__ __forceinline__ long long block_sum_ll(long long v, long long* scratch /*[32]*/) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = (blockDim.x + 31) >> 5;
 #pragma unroll
