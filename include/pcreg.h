@@ -399,7 +399,44 @@ int  pcreg_icp_batch_gicp_dev(const pcreg_model* m, const double* d_src, int64_t
                               double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
                               double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev} or pcreg_nn_search call,
+/* ---- many matching windows in one call ----------------------------------------------------------------------------------
+ * The reference registers each matching window of a surface separately (slideMatchingWindow_v2.m:178-198 under parfor,
+ * completeExperiment.m:265); pcreg_ransac_batch runs every window's RANSAC in one call, and this entry polishes every window's
+ * hypotheses against that window's own source cloud in one call.  A call holds nwin >= 1 windows:
+ *   window w has source rows src_offsets[w] .. src_offsets[w + 1] - 1 of src (ns_total x 3 column-major, ns_total =
+ *   src_offsets[nwin], same type and ld for src_nrm), its own rows of w_src and src_nrm, and hypotheses hyp_offsets[w] ..
+ *   hyp_offsets[w + 1] - 1 of T0_16 (hypotheses grouped by window, as in pcreg_ransac_batch);
+ *   the model, opts, metric, gicp_eps and stop are shared.
+ * Window w's results equal, bit for bit, what pcreg_icp_batch_metric (metric 0 or 1) / pcreg_icp_batch_gicp (metric 2) returns
+ * for its rows, weights, normals and poses alone: T16, rmse, n_used, status, idx, rmse_hist, n_iter and converged.  Results do not
+ * depend on the device count.
+ * metric: PCREG_ICP_POINT_TO_POINT, _POINT_TO_PLANE or _PLANE_TO_PLANE; src_nrm (and gicp_eps) only with PLANE_TO_PLANE, ignored
+ * otherwise.  stop optional (n_iter and converged are written only with a stop).  Per-hypothesis outputs are indexed by the global
+ * hypothesis h; idx is ragged and window-major: window w's [H_w][ns_w] block (original source order relative to the window) starts at
+ * sum_{v<w} H_v ns_v.  best [nwin]: per window, the first-index arg-min of rmse relative to the window, -1 when the window has no
+ * hypothesis or all its rmse are NaN.
+ * PCREG_ERR_ARG: null offsets, offsets[0] != 0 or decreasing offsets, nwin < 1, a window with hypotheses but no source rows, an unknown
+ * metric, a bad eps or stop, a zero or non-finite source normal.  PCREG_ERR_STATE: metric 1 or 2 on a model without normals.
+ * The batch runs as ONE launch of the fused per-hypothesis kernel when the model has a voxel map, opts.nn is the grid and the largest
+ * window fits its shared memory (DESIGN.md section 3.3 gives the rule); otherwise, or with PCREG_FUSED=0, it loops over the windows
+ * through the single-source path.  pcreg_last_profile then reports out[27] = 1 (fused) or 0 (loop: launches, times and counts summed
+ * over the windows). */
+#define PCREG_ICP_PLANE_TO_PLANE 2
+int  pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                             const double* w_src, const void* src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
+                             const double* T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                             double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                             int64_t* best, int32_t* n_iter, int32_t* converged);
+/* The same on device arrays (src, w_src, src_nrm float64 column-major with ld = ns_total), launched on `stream` and synchronous
+ * with respect to it as pcreg_icp_batch_dev.  src_offsets and hyp_offsets are HOST arrays (the host sizes the launch from them);
+ * d_best is a device int64[nwin]. */
+int  pcreg_icp_batch_windows_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                                 const double* d_src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
+                                 const double* d_T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                                 double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
+                                 double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev,_windows,_windows_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
  *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
  *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped

@@ -117,6 +117,13 @@ SIGNATURES = {
     "pcreg_icp_batch_gicp_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_int64,
                                            C.POINTER(IcpOpts), C.POINTER(IcpStop), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pcreg_icp_batch_windows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, c_i64p, c_f64p, C.c_void_p, C.c_double, c_i64p,
+                                          C.c_int64, c_f64p, C.POINTER(IcpOpts), C.c_int, C.POINTER(IcpStop), c_f64p, c_f64p, c_i32p,
+                                          c_i32p, c_i32p, c_f64p, c_i64p, c_i32p, c_i32p]),
+    "pcreg_icp_batch_windows_dev": (C.c_int, [C.c_void_p, C.c_void_p, c_i64p, C.c_void_p, C.c_void_p, C.c_double, c_i64p, C.c_int64,
+                                              C.c_void_p, C.POINTER(IcpOpts), C.c_int, C.POINTER(IcpStop), C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p]),
     "pcreg_set_profiling": (C.c_int, [C.c_int]),
     "pcreg_last_profile": (C.c_int, [c_f64p]),
 }

@@ -18,9 +18,10 @@ from ._lib import AlignOpts, DescOpts, IcpOpts, IcpStop, MatchOpts, ModelOpts, P
 
 NN_BRUTE, NN_GRID = 0, 1
 ICP_PLAIN, ICP_KNN, ICP_WEIGHTED = 0, 1, 2
-ICP_POINT_TO_POINT, ICP_POINT_TO_PLANE = 0, 1
+ICP_POINT_TO_POINT, ICP_POINT_TO_PLANE, ICP_PLANE_TO_PLANE = 0, 1, 2
 METRICS = {"point_to_point": ICP_POINT_TO_POINT, "point_to_plane": ICP_POINT_TO_PLANE}
 # the plane-to-plane metric has entries of its own (pcreg_icp_batch_gicp{,_dev}); it is no value of pcreg_icp_batch_metric's `metric`
+# (pcreg_icp_batch_windows{,_dev} take all three: ICP_PLANE_TO_PLANE)
 PLANE_TO_PLANE = "plane_to_plane"
 GICP_EPS = 1e-3
 METRIC_SAD, METRIC_SSD = 0, 1
@@ -588,6 +589,86 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
         out["idx"] = idx
     if return_hist:
         out["rmse_hist"] = hist
+    return out
+
+
+def icp_batch_windows(model: Model, src_list, T0_list, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src_list=None,
+                      nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3,
+                      metric="point_to_point", src_normals_list=None, gicp_eps=GICP_EPS):
+    """icp_batch for many matching windows in ONE call (include/pcreg.h: pcreg_icp_batch_windows): window w polishes the poses
+    T0_list[w] [H_w,4,4] (H_w may be 0) against its own source cloud src_list[w] [ns_w,3], with w_src_list[w] / src_normals_list[w]
+    when given; the model and every other keyword (as icp_batch) are shared.  Returns one dict per window, each what
+    icp_batch(model, src_list[w], T0_list[w], ...) returns (best relative to the window, -1 without hypotheses), bit for bit.
+    The windows' sources are passed as float32 only when all of them are float32."""
+    if metric not in METRICS and metric != PLANE_TO_PLANE:
+        raise ValueError("metric must be one of %s" % sorted(list(METRICS) + [PLANE_TO_PLANE]))
+    if metric == PLANE_TO_PLANE and src_normals_list is None:
+        raise ValueError("metric='plane_to_plane' needs src_normals_list (one N x 3 array of normals per window)")
+    if metric != PLANE_TO_PLANE and src_normals_list is not None:
+        raise ValueError("src_normals_list is used only by metric='plane_to_plane'")
+    nw = len(src_list)
+    if len(T0_list) != nw or (w_src_list is not None and len(w_src_list) != nw) or (src_normals_list is not None and len(src_normals_list) != nw):
+        raise ValueError("one source, one pose array (and one w_src / normals array, when given) per window")
+    srcs = [np.asarray(p).reshape(-1, 3) for p in src_list]
+    dt = np.float32 if all(p.dtype == np.float32 for p in srcs) else np.float64
+    ns = np.array([p.shape[0] for p in srcs], dtype=np.int64)
+    soff = np.zeros(nw + 1, dtype=np.int64)
+    np.cumsum(ns, out=soff[1:])
+    nt = int(soff[-1])
+    cat = np.asfortranarray(np.concatenate([p.astype(dt, copy=False) for p in srcs], axis=0)) if nt else np.zeros((1, 3), dtype=dt, order="F")
+    sn = None
+    if src_normals_list is not None:
+        nrm = [np.asarray(x).reshape(-1, 3) for x in src_normals_list]
+        if any(x.shape[0] != n for x, n in zip(nrm, ns)):
+            raise ValueError("src_normals_list[w] must be N_w x 3, one normal per source point of window w")
+        sn = np.asfortranarray(np.concatenate([x.astype(dt, copy=False) for x in nrm], axis=0)) if nt else np.zeros((1, 3), dtype=dt, order="F")
+    T0s = [np.asarray(t, dtype=np.float64).reshape(-1, 4, 4) for t in T0_list]
+    H = np.array([t.shape[0] for t in T0s], dtype=np.int64)
+    hoff = np.zeros(nw + 1, dtype=np.int64)
+    np.cumsum(H, out=hoff[1:])
+    nh = int(hoff[-1])
+    T0 = _T_to_abi(np.concatenate(T0s, axis=0)) if nh else np.zeros((1, 4, 4))
+    w = None
+    if w_src_list is not None:
+        ws = [np.asarray(x, dtype=np.float64).reshape(-1) for x in w_src_list]
+        if any(x.shape[0] != n for x, n in zip(ws, ns)):
+            raise ValueError("w_src_list[w] must hold one weight per source point of window w")
+        w = np.ascontiguousarray(np.concatenate(ws)) if nt else np.zeros(1)
+    o = icp_opts(mode, iters, k_frac, R_w, thDist2, nn, reflection_fix)
+    ioff = np.zeros(nw + 1, dtype=np.int64)
+    np.cumsum(H * ns, out=ioff[1:])
+    T = np.empty((max(nh, 1), 16), dtype=np.float64)
+    rmse = np.empty(max(nh, 1), dtype=np.float64)
+    n_used = np.empty(max(nh, 1), dtype=np.int32)
+    status = np.empty(max(nh, 1), dtype=np.int32)
+    idx = np.empty(max(int(ioff[-1]), 1), dtype=np.int32) if return_idx else None
+    hist = np.empty((max(nh, 1), iters + 1), dtype=np.float64) if return_hist else None
+    best = np.empty(nw, dtype=np.int64)
+    stop = icp_stop(tolerance[0], tolerance[1], window) if tolerance is not None else None
+    n_iter = np.empty(max(nh, 1), dtype=np.int32) if tolerance is not None else None
+    converged = np.empty(max(nh, 1), dtype=np.int32) if tolerance is not None else None
+    mcode = ICP_PLANE_TO_PLANE if metric == PLANE_TO_PLANE else METRICS[metric]
+    L.check(L.lib().pcreg_icp_batch_windows(model.handle, cat.ctypes.data_as(C.c_void_p), int(dt == np.float64), cat.shape[0],
+                                            _ptr(soff, L.c_i64p), _ptr(w, L.c_f64p),
+                                            sn.ctypes.data_as(C.c_void_p) if sn is not None else None, float(gicp_eps),
+                                            _ptr(hoff, L.c_i64p), nw, _ptr(T0, L.c_f64p), C.byref(o), mcode,
+                                            C.byref(stop) if stop is not None else None, _ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p),
+                                            _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p), _ptr(hist, L.c_f64p),
+                                            _ptr(best, L.c_i64p), _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)),
+            "pcreg_icp_batch_windows")
+    Ts = _T_from_abi(T, T.shape[0])
+    out = []
+    for k in range(nw):
+        a, b = int(hoff[k]), int(hoff[k + 1])
+        r = dict(T=Ts[a:b].copy(), rmse=rmse[a:b].copy(), n_used=n_used[a:b].copy(), status=status[a:b].copy(), best=int(best[k]))
+        if tolerance is not None:
+            r["n_iter"] = n_iter[a:b].copy()
+            r["converged"] = converged[a:b].copy()
+        if return_idx:
+            r["idx"] = idx[int(ioff[k]):int(ioff[k + 1])].reshape(b - a, int(ns[k])).copy()
+        if return_hist:
+            r["rmse_hist"] = hist[a:b].copy()
+        out.append(r)
     return out
 
 

@@ -268,8 +268,11 @@ __global__ void __launch_bounds__(1024) k_src_stats(const double* __restrict__ s
     }
 }
 
-// first-index arg-min over hypotheses, NaN never wins; one block.
-__global__ void __launch_bounds__(1024) k_icp_argmin(const double* __restrict__ rmse, int64_t n, int64_t* __restrict__ best) {
+// first-index arg-min over hypotheses, NaN never wins (-1: none); one block per segment: block b takes rmse[seg[b] .. seg[b + 1] - 1]
+// and writes best[b] relative to seg[b] (seg null: one segment of n).
+__global__ void __launch_bounds__(1024) k_icp_argmin(const double* __restrict__ rmse, const int64_t* __restrict__ seg, int64_t n,
+                                                     int64_t* __restrict__ best) {
+    if (seg) { rmse += seg[blockIdx.x]; n = seg[blockIdx.x + 1] - seg[blockIdx.x]; }
     __shared__ double sv[32];
     __shared__ long long si[32];
     double bv = INFINITY;
@@ -302,7 +305,7 @@ __global__ void __launch_bounds__(1024) k_icp_argmin(const double* __restrict__ 
             const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
             if (better(bv, bi, ov, oi)) { bv = ov; bi = oi; }
         }
-        if (lane == 0) *best = bi;
+        if (lane == 0) best[blockIdx.x] = bi;
     }
 }
 
@@ -318,14 +321,36 @@ __device__ __forceinline__ unsigned spread10(unsigned v) {
     v = (v | (v << 2)) & 0x09249249u;
     return v;
 }
-__global__ void __launch_bounds__(1024) k_src_sort(const double* __restrict__ src, const double* __restrict__ w, int64_t ns,
-                                                   int npow2, unsigned long long* __restrict__ keys, double* __restrict__ out_src,
-                                                   double* __restrict__ out_w, int32_t* __restrict__ perm, int32_t* __restrict__ inv) {
+// One block per window: window b is rows off[b] .. off[b + 1] - 1 of src (column stride ld; off null: one window of ns rows).  A window
+// of 64 .. 2^17 rows is sorted as the single-block sort is sized; any other gets the identity order (the single-source call does not
+// launch the sort for those).  perm / inv are relative to the window's first row; keys: scratch of 2 ld entries (a window's power of
+// two stays below twice its row count).
+__global__ void __launch_bounds__(1024) k_src_sort(const double* __restrict__ src, const double* __restrict__ w, int64_t ld,
+                                                   const int64_t* __restrict__ off, int64_t ns, unsigned long long* __restrict__ keys,
+                                                   double* __restrict__ out_src, double* __restrict__ out_w, int32_t* __restrict__ perm,
+                                                   int32_t* __restrict__ inv) {
     __shared__ double red[6 * 32];
     const int tid = threadIdx.x;
+    if (off) {
+        const int64_t r0 = off[blockIdx.x];
+        ns = off[blockIdx.x + 1] - r0;
+        src += r0; out_src += r0; perm += r0; inv += r0; keys += 2 * r0;
+        if (w) { w += r0; out_w += r0; }
+    }
+    if (ns < 64 || ns > (1 << 17)) {
+        for (int64_t r = tid; r < ns; r += blockDim.x) {
+            perm[r] = (int32_t)r;
+            inv[r] = (int32_t)r;
+            out_src[r] = src[r]; out_src[ld + r] = src[ld + r]; out_src[2 * ld + r] = src[2 * ld + r];
+            if (w) out_w[r] = w[r];
+        }
+        return;
+    }
+    int npow2 = 1;
+    while (npow2 < ns) npow2 <<= 1;
     double mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
     for (int64_t i = tid; i < ns; i += blockDim.x)
-        for (int a = 0; a < 3; ++a) { const double v = src[a * ns + i]; mn[a] = fmin(mn[a], v); mx[a] = fmax(mx[a], v); }
+        for (int a = 0; a < 3; ++a) { const double v = src[a * ld + i]; mn[a] = fmin(mn[a], v); mx[a] = fmax(mx[a], v); }
     for (int a = 0; a < 3; ++a) {
         for (int o = 16; o > 0; o >>= 1) { mn[a] = fmin(mn[a], __shfl_xor_sync(0xffffffffu, mn[a], o)); mx[a] = fmax(mx[a], __shfl_xor_sync(0xffffffffu, mx[a], o)); }
         if ((tid & 31) == 0) { red[a * 32 + (tid >> 5)] = mn[a]; red[(3 + a) * 32 + (tid >> 5)] = mx[a]; }
@@ -342,8 +367,8 @@ __global__ void __launch_bounds__(1024) k_src_sort(const double* __restrict__ sr
     for (int i = tid; i < npow2; i += blockDim.x) {
         unsigned long long k = ~0ull;
         if (i < ns) {
-            const unsigned cx = (unsigned)((src[i] - mn[0]) * scale), cy = (unsigned)((src[ns + i] - mn[1]) * scale),
-                           cz = (unsigned)((src[2 * ns + i] - mn[2]) * scale);
+            const unsigned cx = (unsigned)((src[i] - mn[0]) * scale), cy = (unsigned)((src[ld + i] - mn[1]) * scale),
+                           cz = (unsigned)((src[2 * ld + i] - mn[2]) * scale);
             const unsigned code = spread10(cx) | (spread10(cy) << 1) | (spread10(cz) << 2);
             k = ((unsigned long long)code << 32) | (unsigned long long)(unsigned)i;
         }
@@ -366,7 +391,7 @@ __global__ void __launch_bounds__(1024) k_src_sort(const double* __restrict__ sr
         const int32_t o = (int32_t)(unsigned)(keys[r] & 0xffffffffull);
         perm[r] = o;
         inv[o] = (int32_t)r;
-        out_src[r] = src[o]; out_src[ns + r] = src[ns + o]; out_src[2 * ns + r] = src[2 * ns + o];
+        out_src[r] = src[o]; out_src[ld + r] = src[ld + o]; out_src[2 * ld + r] = src[2 * ld + o];
         if (w) out_w[r] = w[o];
     }
 }
@@ -381,16 +406,19 @@ __global__ void k_unpermute_idx(const int32_t* __restrict__ in, const int32_t* _
 
 // Source normals of the plane-to-plane metric, one thread per row: out row r (the order of the sorted source) is input row perm[r]
 // (perm null: r) normalised in FP64 as pcreg_model_set_normals normalises (no contraction into FMA: the same bits as the host
-// loop).  A zero or non-finite row sets *bad.  in, out: ns x 3 column-major, ld = ns.
-__global__ void k_src_normals(const double* __restrict__ in, const int32_t* __restrict__ perm, int64_t ns, double* __restrict__ out,
-                              int* __restrict__ bad) {
+// loop).  A zero or non-finite row sets *bad.  in, out: column-major, column stride ld.  Windowed calls: blockIdx.y is the window,
+// rows off[y] .. off[y + 1] - 1, perm relative to the window's first row (off null: one window of ns rows).
+__global__ void k_src_normals(const double* __restrict__ in, const int32_t* __restrict__ perm, int64_t ld, const int64_t* __restrict__ off,
+                              int64_t ns, double* __restrict__ out, int* __restrict__ bad) {
+    const int64_t r0 = off ? off[blockIdx.y] : 0;
+    if (off) ns = off[blockIdx.y + 1] - r0;
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= ns) return;
-    const int64_t o = perm ? perm[r] : r;
-    const double x = in[o], y = in[ns + o], z = in[2 * ns + o];
+    const int64_t o = r0 + (perm ? perm[r0 + r] : r);
+    const double x = in[o], y = in[ld + o], z = in[2 * ld + o];
     const double n = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)));
     if (!(isfinite(n) && n > 0.0)) *bad = 1;
-    out[r] = x / n; out[ns + r] = y / n; out[2 * ns + r] = z / n;
+    out[r0 + r] = x / n; out[ld + r0 + r] = y / n; out[2 * ld + r0 + r] = z / n;
 }
 
 // MATLAB column-major 4x4 <-> internal row-major 4x4 (a transpose), batched
@@ -429,8 +457,8 @@ void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
     else            icp_update_launch_metric<ICP_M_POINT>(a, nhyp, st);
     PCREG_LAUNCHED();
 }
-void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st) {
-    k_icp_argmin<<<1, 1024, 0, st>>>(d_rmse, nhyp, d_best);
+void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st, const int64_t* d_seg, int64_t nseg) {
+    k_icp_argmin<<<(unsigned)nseg, 1024, 0, st>>>(d_rmse, d_seg, nhyp, d_best);
     PCREG_LAUNCHED();
 }
 
@@ -577,7 +605,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         int npow2 = 1;
         while (npow2 < ns) npow2 <<= 1;
         DevBuf<unsigned long long> skeys((size_t)npow2);
-        k_src_sort<<<1, 1024, 0, st>>>(d_src, d_w, ns, npow2, skeys.p, src_sorted.p, d_w ? w_sorted.p : nullptr, sperm.p, sinv.p);
+        k_src_sort<<<1, 1024, 0, st>>>(d_src, d_w, ns, nullptr, ns, skeys.p, src_sorted.p, d_w ? w_sorted.p : nullptr, sperm.p, sinv.p);
         PCREG_LAUNCHED();
         PCREG_CUDA(cudaStreamSynchronize(st));      // skeys is released here
         d_src = src_sorted.p;
@@ -590,7 +618,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         DevBuf<int> bad(1);
         int h_bad = 0;
         PCREG_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), st));
-        k_src_normals<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(d_src_nrm, sorted ? sperm.p : nullptr, ns, snrm.p, bad.p);
+        k_src_normals<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(d_src_nrm, sorted ? sperm.p : nullptr, ns, nullptr, ns, snrm.p, bad.p);
         PCREG_LAUNCHED();
         PCREG_CUDA(cudaMemcpyAsync(&h_bad, bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
         PCREG_CUDA(cudaStreamSynchronize(st));
@@ -771,6 +799,172 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         c.profile[4] = upd_launches; c.profile[5] = upd_ms; c.profile[6] = nq_run;
         c.profile[7] = (double)hcnt[0]; c.profile[8] = (double)hcnt[1]; c.profile[9] = (double)hcnt[2];
         c.profile[26] = (o.nn == PCREG_NN_GRID && m->has_vox) ? 1.0 : 0.0;
+    }
+}
+
+// ---- windowed calls (pcreg_icp_batch_windows{,_dev}) ----------------------------------------------------------------------
+// Host-side layout of a windowed call: window w owns source rows src_off[w] .. src_off[w + 1] - 1 and hypotheses hyp_off[w] ..
+// hyp_off[w + 1] - 1; its [H_w][ns_w] block of idx starts at idx_off[w].
+struct WindowLayout {
+    int64_t nwin = 0, nrows = 0, nhyp = 0, ns_max = 0;
+    std::vector<int64_t> src_off, hyp_off, idx_off;
+    WindowLayout(const int64_t* so, const int64_t* ho, int64_t nw) : nwin(nw), src_off(so, so + nw + 1), hyp_off(ho, ho + nw + 1), idx_off((size_t)nw + 1, 0) {
+        for (int64_t w = 0; w < nw; ++w) {
+            const int64_t ns = src_off[w + 1] - src_off[w];
+            ns_max = std::max(ns_max, ns);
+            idx_off[w + 1] = idx_off[w] + (hyp_off[w + 1] - hyp_off[w]) * ns;
+        }
+        nrows = src_off[nw]; nhyp = hyp_off[nw];
+    }
+    int64_t ns(int64_t w) const { return src_off[w + 1] - src_off[w]; }
+    int64_t nh(int64_t w) const { return hyp_off[w + 1] - hyp_off[w]; }
+    int64_t window_of(int64_t h) const {       // the window that holds hypothesis h
+        return (int64_t)(std::upper_bound(hyp_off.begin(), hyp_off.end(), h) - hyp_off.begin()) - 1;
+    }
+    int64_t idx_at(int64_t h) const { const int64_t w = window_of(h); return idx_off[w] + (h - hyp_off[w]) * ns(w); }
+};
+
+// When a windowed call runs as one launch of the fused kernel.  The alternative is a loop over the windows through icp_run, each
+// window at least an NN and an update launch per pass plus host synchronisations (DESIGN.md section 3.3 has the measurements).
+static bool windows_use_fused(const pcreg_model* m, const WindowLayout& L, const pcreg_icp_opts& o, bool stop, int metric) {
+    if (!icp_fused_windows_fit(m, L.ns_max, o, stop, metric)) return false;
+    if (const char* e = getenv("PCREG_FUSED")) { if (e[0] == '0') return false; if (e[0] == '1') return true; }
+    int64_t busy = 0;                          // windows with hypotheses
+    for (int64_t w = 0; w < L.nwin; ++w) busy += L.nh(w) > 0;
+    return busy >= 2 || L.nhyp >= ctx().sm_count;
+}
+
+// One device: d_src column-major with column stride L.nrows (the windows' rows one after the other), d_w / d_src_nrm at the same
+// rows, d_T0_cm / outputs indexed by hypothesis as in icp_run, d_idx in the ragged window-major layout, d_best [nwin] (relative).
+static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const double* d_src, const double* d_w, const double* d_src_nrm,
+                            const double* d_T0_cm, const pcreg_icp_opts& o, const pcreg_icp_stop* stop, int metric, double gicp_eps,
+                            double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist,
+                            int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, cudaStream_t st) {
+    PCREG_REQUIRE(m && d_T16_cm && (L.nrows == 0 || d_src) && (L.nhyp == 0 || d_T0_cm), "icp windows: null pointer");
+    const bool gicp = metric == ICP_M_GICP;
+    const ModelPointD* nrm = metric != ICP_M_POINT ? m->nrm.p : nullptr;
+    if (metric != ICP_M_POINT && !nrm) throw StateError{"icp: the point-to-plane and plane-to-plane metrics need model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
+    PCREG_REQUIRE(!gicp || d_src_nrm, "icp: the plane-to-plane metric needs source normals");
+    PCREG_REQUIRE(o.iters >= 0, "icp: iters must be >= 0");
+    PCREG_REQUIRE(o.mode >= PCREG_ICP_PLAIN && o.mode <= PCREG_ICP_WEIGHTED, "icp: bad mode");
+    PCREG_REQUIRE(o.nn == PCREG_NN_BRUTE || o.nn == PCREG_NN_GRID, "icp: bad nn kind");
+    if (o.nn == PCREG_NN_GRID) PCREG_REQUIRE(m->has_grid, "icp: grid NN requested but the model has no grid");
+    Context& c = ctx();
+    const bool prof = c.profiling;
+    const int64_t nrows = L.nrows, nhyp = L.nhyp;
+    DevBuf<int64_t> offs((size_t)(3 * L.nwin + 2));            // src_off [nwin + 1], hyp_off [nwin + 1], idx_off [nwin]
+    int64_t* d_soff = offs.p; int64_t* d_hoff = offs.p + L.nwin + 1; int64_t* d_ioff = offs.p + 2 * (L.nwin + 1);
+    PCREG_CUDA(cudaMemcpyAsync(d_soff, L.src_off.data(), (size_t)(L.nwin + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    PCREG_CUDA(cudaMemcpyAsync(d_hoff, L.hyp_off.data(), (size_t)(L.nwin + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    PCREG_CUDA(cudaMemcpyAsync(d_ioff, L.idx_off.data(), (size_t)L.nwin * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    const bool fused = nhyp > 0 && windows_use_fused(m, L, o, stop != nullptr, metric);
+    // plane-to-plane: every window's source normals normalised and checked before any ICP kernel runs (in the windows' sorted order
+    // on the fused path; the loop normalises each window again inside icp_run, from the caller's rows)
+    DevBuf<int32_t> sperm(fused ? (size_t)nrows : 0), sinv(fused ? (size_t)nrows : 0);
+    DevBuf<double> src_sorted(fused ? (size_t)nrows * 3 : 0), w_sorted(fused && d_w ? (size_t)nrows : 0);
+    if (fused && nrows > 0) {
+        DevBuf<unsigned long long> skeys((size_t)nrows * 2);
+        k_src_sort<<<(unsigned)L.nwin, 1024, 0, st>>>(d_src, d_w, nrows, d_soff, 0, skeys.p, src_sorted.p, d_w ? w_sorted.p : nullptr, sperm.p, sinv.p);
+        PCREG_LAUNCHED();
+        PCREG_CUDA(cudaStreamSynchronize(st));      // skeys is released here
+    }
+    DevBuf<double> snrm(gicp ? (size_t)nrows * 3 : 0);
+    if (gicp && nrows > 0) {
+        DevBuf<int> bad(1);
+        int h_bad = 0;
+        PCREG_CUDA(cudaMemsetAsync(bad.p, 0, sizeof(int), st));
+        for (int64_t w0 = 0; w0 < L.nwin; w0 += 65535) {         // grid.y: at most 65 535 windows per launch
+            const dim3 grid((unsigned)((L.ns_max + 255) / 256), (unsigned)std::min<int64_t>(65535, L.nwin - w0));
+            k_src_normals<<<grid, 256, 0, st>>>(d_src_nrm, fused ? sperm.p : nullptr, nrows, d_soff + w0, 0, snrm.p, bad.p);
+            PCREG_LAUNCHED();
+        }
+        PCREG_CUDA(cudaMemcpyAsync(&h_bad, bad.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+        PCREG_CUDA(cudaStreamSynchronize(st));
+        PCREG_REQUIRE(!h_bad, "icp: zero or non-finite source normal");
+    }
+    if (d_best) PCREG_CUDA(cudaMemsetAsync(d_best, 0xff, (size_t)L.nwin * sizeof(int64_t), st));     // -1: no hypothesis
+    if (!fused) {
+        // one icp_run per window with hypotheses, on its rows copied out of the concatenation and its slices of every output
+        double prof_sum[32] = {0};
+        const size_t hs = (size_t)o.iters + 1;
+        for (int64_t w = 0; w < L.nwin; ++w) {
+            const int64_t ns = L.ns(w), nh = L.nh(w), r0 = L.src_off[w], h0 = L.hyp_off[w];
+            if (nh == 0) continue;
+            DevBuf<double> src_w((size_t)ns * 3), nrm_w(gicp ? (size_t)ns * 3 : 0);
+            for (int a = 0; a < 3; ++a) {
+                PCREG_CUDA(cudaMemcpyAsync(src_w.p + a * ns, d_src + a * nrows + r0, (size_t)ns * sizeof(double), cudaMemcpyDeviceToDevice, st));
+                if (gicp) PCREG_CUDA(cudaMemcpyAsync(nrm_w.p + a * ns, d_src_nrm + a * nrows + r0, (size_t)ns * sizeof(double), cudaMemcpyDeviceToDevice, st));
+            }
+            icp_run(m, src_w.p, ns, d_w ? d_w + r0 : nullptr, d_T0_cm + h0 * 16, nh, o, d_T16_cm + h0 * 16, d_rmse ? d_rmse + h0 : nullptr,
+                    d_n_used ? d_n_used + h0 : nullptr, d_status ? d_status + h0 : nullptr, d_idx ? d_idx + L.idx_off[w] : nullptr,
+                    d_rmse_hist ? d_rmse_hist + h0 * hs : nullptr, d_best ? d_best + w : nullptr, st, stop,
+                    d_n_iter ? d_n_iter + h0 : nullptr, d_converged ? d_converged + h0 : nullptr, metric, gicp ? nrm_w.p : nullptr, gicp_eps);
+            if (prof) {
+                for (int k = 0; k < 26; ++k) prof_sum[k] += c.profile[k];
+                prof_sum[26] = std::max(prof_sum[26], c.profile[26]);
+            }
+        }
+        PCREG_CUDA(cudaStreamSynchronize(st));
+        for (int k = 0; k < 32; ++k) c.profile[k] = prof_sum[k];       // out[27] = 0: the loop ran
+        return;
+    }
+    for (int i = 0; i < 32; ++i) c.profile[i] = 0.0;
+    // one launch of the fused kernel for every hypothesis of every window (k_icp_fused<*, *, *, true>)
+    DevBuf<double> Twork((size_t)nhyp * 16);
+    DevBuf<int32_t> frozen((size_t)nhyp);
+    DevBuf<double> rmse_tmp(d_rmse ? 0 : (size_t)nhyp);
+    DevBuf<int32_t> nused_tmp(d_n_used ? 0 : (size_t)nhyp);
+    DevBuf<unsigned long long> counters(16);
+    DevBuf<int32_t> n_iter_tmp(stop && prof && !d_n_iter ? (size_t)nhyp : 0);
+    if (n_iter_tmp.p) d_n_iter = n_iter_tmp.p;
+    double* rm = d_rmse ? d_rmse : rmse_tmp.p;
+    PCREG_CUDA(cudaMemsetAsync(frozen.p, 0, frozen.bytes(), st));
+    PCREG_CUDA(cudaMemsetAsync(counters.p, 0, counters.bytes(), st));
+    transpose16_launch(d_T0_cm, Twork.p, nhyp, st);
+    FusedWinArgs fa{};
+    fa.g.g = m->grid; fa.g.md = m->md.p; fa.g.vox = m->vox;
+    fa.sx = src_sorted.p; fa.sy = src_sorted.p + nrows; fa.sz = src_sorted.p + 2 * nrows; fa.w_src = d_w ? w_sorted.p : nullptr;
+    fa.ns = (int32_t)L.ns_max;
+    for (int k = 0; k < 3; ++k) fa.pivot[k] = m->pivot[k];
+    fa.T = Twork.p; fa.frozen = frozen.p; fa.rmse = rm; fa.n_used = d_n_used ? d_n_used : nused_tmp.p;
+    fa.rmse_hist = d_rmse_hist; fa.hist_stride = o.iters + 1;
+    fa.idx_out = d_idx; fa.perm = sperm.p; fa.tie_order = sinv.p;
+    fa.mode = o.mode; fa.k_frac = o.k_frac; fa.R_w = o.R_w; fa.thDist2 = o.thDist2; fa.reflection_fix = o.reflection_fix; fa.iters = o.iters;
+    fa.counters = (prof && c.profiling_counters) ? counters.p : nullptr;
+    if (stop) { fa.stop.tol_t = stop->tol_t; fa.stop.tol_r_deg = stop->tol_r_deg; fa.stop.window = stop->window; }
+    fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
+    fa.snx = gicp ? snrm.p : nullptr; fa.sny = gicp ? snrm.p + nrows : nullptr; fa.snz = gicp ? snrm.p + 2 * nrows : nullptr; fa.gicp_eps = gicp_eps;
+    fa.win_src = d_soff; fa.win_hyp = d_hoff; fa.win_idx = d_ioff; fa.nwin = (int32_t)L.nwin;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    if (prof) { e0 = pooled_event(0); e1 = pooled_event(1); PCREG_CUDA(cudaEventRecord(e0, st)); }
+    icp_fused_windows_launch(fa, nhyp, stop != nullptr, st);
+    if (prof) PCREG_CUDA(cudaEventRecord(e1, st));
+    transpose16_launch(Twork.p, d_T16_cm, nhyp, st);
+    if (d_status) PCREG_CUDA(cudaMemcpyAsync(d_status, frozen.p, (size_t)nhyp * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    if (d_best) icp_argmin_launch(rm, nhyp, d_best, st, d_hoff, L.nwin);
+    PCREG_CUDA(cudaStreamSynchronize(st));
+    if (prof) {
+        float ms = 0.f;
+        PCREG_CUDA(cudaEventElapsedTime(&ms, e0, e1));
+        unsigned long long hcnt[16] = {0};
+        PCREG_CUDA(cudaMemcpy(hcnt, counters.p, sizeof hcnt, cudaMemcpyDeviceToHost));
+        // queries of the passes each hypothesis ran (with the tolerance stop: n_iter + 1, one more after a freeze)
+        double nq = 0.0;
+        if (stop) {
+            std::vector<int32_t> ni((size_t)nhyp), fz((size_t)nhyp);
+            PCREG_CUDA(cudaMemcpy(ni.data(), d_n_iter, ni.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+            PCREG_CUDA(cudaMemcpy(fz.data(), frozen.p, fz.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+            for (int64_t h = 0; h < nhyp; ++h) nq += (double)L.ns(L.window_of(h)) * ((double)ni[h] + 1.0 + (double)fz[h]);
+        } else {
+            for (int64_t w = 0; w < L.nwin; ++w) nq += (double)L.nh(w) * (double)L.ns(w) * (double)(o.iters + 1);
+        }
+        c.profile[0] = 1; c.profile[1] = ms; c.profile[2] = nq; c.profile[6] = nq;
+        c.profile[11] = (double)hcnt[4]; c.profile[10] = nq - (double)hcnt[4];
+        c.profile[13] = (double)hcnt[6]; c.profile[14] = (double)hcnt[7];
+        c.profile[17] = ms; c.profile[20] = 1;
+        c.profile[26] = 1.0; c.profile[27] = 1.0;
+        const double tot = (double)hcnt[11] + (double)hcnt[12] + (double)hcnt[13] + (double)hcnt[14];
+        for (int k = 0; k < 4; ++k) c.profile[28 + k] = tot > 0.0 ? (double)hcnt[11 + k] / tot : 0.0;
     }
 }
 
@@ -987,6 +1181,131 @@ int pcreg_icp_batch_gicp_dev(const pcreg_model* m, const double* d_src, int64_t 
     PCREG_CUDA(cudaSetDevice(ctx().device));
     icp_run(m, d_src, ns, d_w_src, d_T0_16, nhyp, *opts, d_T16, d_rmse, d_n_used, d_status, d_idx, d_rmse_hist,
             d_best, (cudaStream_t)stream, stop, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, ICP_M_GICP, d_src_nrm, eps);
+    return PCREG_OK;
+    PCREG_API_END
+}
+
+static void check_windows(const pcreg_model* m, const int64_t* src_off, const int64_t* hyp_off, int64_t nwin, const pcreg_icp_opts* opts,
+                               int metric, const void* src_nrm, double eps, const pcreg_icp_stop* stop) {
+    PCREG_REQUIRE(m && opts, "pcreg_icp_batch_windows: null pointer");
+    PCREG_REQUIRE(nwin >= 1, "icp windows: need nwin >= 1");
+    PCREG_REQUIRE(src_off && hyp_off, "icp windows: null offsets");
+    PCREG_REQUIRE(src_off[0] == 0 && hyp_off[0] == 0, "icp windows: offsets must start at 0");
+    for (int64_t w = 0; w < nwin; ++w) {
+        PCREG_REQUIRE(src_off[w + 1] >= src_off[w] && hyp_off[w + 1] >= hyp_off[w], "icp windows: decreasing offsets");
+        PCREG_REQUIRE(hyp_off[w + 1] == hyp_off[w] || src_off[w + 1] > src_off[w], "icp windows: a window with hypotheses has no source rows");
+        PCREG_REQUIRE(src_off[w + 1] - src_off[w] < ((int64_t)1 << 31), "icp windows: a window holds at most 2^31 - 1 source rows");
+    }
+    PCREG_REQUIRE(metric >= PCREG_ICP_POINT_TO_POINT && metric <= PCREG_ICP_PLANE_TO_PLANE, "icp: unknown metric");
+    if (metric == PCREG_ICP_PLANE_TO_PLANE) check_gicp(src_nrm, eps, nullptr);
+    if (stop) check_stop(stop);
+    if (metric != PCREG_ICP_POINT_TO_POINT && !m->nrm.p)
+        throw StateError{"icp: the point-to-plane and plane-to-plane metrics need model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
+}
+
+// One device's share [h0, h1) of a windowed host call: the windows it touches (a share may start or end inside a window), their rows
+// and rebased offsets; every output lands in its own slice of the caller's arrays.
+static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, const std::vector<double>& hs, const double* w_src,
+                                   const std::vector<double>& hnrm, const double* T0_16, int64_t h0, int64_t h1, const pcreg_icp_opts& o,
+                                   const pcreg_icp_stop* stop, int metric, double eps, double* T16, double* rmse, int32_t* n_used,
+                                   int32_t* status, int32_t* idx, double* rmse_hist, int32_t* n_iter, int32_t* converged) {
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    cudaStream_t st = 0;
+    const int64_t wa = L.window_of(h0), wb = L.window_of(h1 - 1), nw = wb - wa + 1;
+    const int64_t ra = L.src_off[wa], nr = L.src_off[wb + 1] - ra, hn = h1 - h0;
+    std::vector<int64_t> so((size_t)nw + 1), ho((size_t)nw + 1);
+    for (int64_t k = 0; k <= nw; ++k) {
+        so[k] = L.src_off[wa + k] - ra;
+        ho[k] = std::min(std::max(L.hyp_off[wa + k], h0), h1) - h0;
+    }
+    const WindowLayout S(so.data(), ho.data(), nw);
+    const int64_t i0 = L.idx_at(h0), ni = S.idx_off[nw];
+    DevBuf<double> d_src((size_t)nr * 3), d_w(w_src ? (size_t)nr : 0), d_nrm(hnrm.empty() ? 0 : (size_t)nr * 3);
+    DevBuf<double> d_T0((size_t)hn * 16), d_T((size_t)hn * 16), d_rmse((size_t)hn), d_hist(rmse_hist ? (size_t)hn * (o.iters + 1) : 0);
+    DevBuf<int32_t> d_nu((size_t)hn), d_st((size_t)hn), d_idx(idx ? (size_t)ni : 0);
+    DevBuf<int32_t> d_nit(n_iter ? (size_t)hn : 0), d_conv(converged ? (size_t)hn : 0);
+    for (int a = 0; a < 3; ++a) {
+        PCREG_CUDA(cudaMemcpyAsync(d_src.p + a * nr, hs.data() + a * L.nrows + ra, (size_t)nr * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (d_nrm.p) PCREG_CUDA(cudaMemcpyAsync(d_nrm.p + a * nr, hnrm.data() + a * L.nrows + ra, (size_t)nr * sizeof(double), cudaMemcpyHostToDevice, st));
+    }
+    if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src + ra, d_w.bytes(), cudaMemcpyHostToDevice, st));
+    PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
+    icp_windows_run(m, S, d_src.p, d_w.p, d_nrm.p, d_T0.p, o, stop, metric, eps, d_T.p, d_rmse.p, d_nu.p, d_st.p, d_idx.p, d_hist.p,
+                    nullptr, d_nit.p, d_conv.p, st);
+    PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
+    PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
+    if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
+    if (status) PCREG_CUDA(cudaMemcpyAsync(status + h0, d_st.p, d_st.bytes(), cudaMemcpyDeviceToHost, st));
+    if (idx) PCREG_CUDA(cudaMemcpyAsync(idx + i0, d_idx.p, d_idx.bytes(), cudaMemcpyDeviceToHost, st));
+    if (rmse_hist) PCREG_CUDA(cudaMemcpyAsync(rmse_hist + h0 * (o.iters + 1), d_hist.p, d_hist.bytes(), cudaMemcpyDeviceToHost, st));
+    if (n_iter) PCREG_CUDA(cudaMemcpyAsync(n_iter + h0, d_nit.p, d_nit.bytes(), cudaMemcpyDeviceToHost, st));
+    if (converged) PCREG_CUDA(cudaMemcpyAsync(converged + h0, d_conv.p, d_conv.bytes(), cudaMemcpyDeviceToHost, st));
+    PCREG_CUDA(cudaStreamSynchronize(st));
+}
+
+int pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                            const double* w_src, const void* src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
+                            const double* T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                            double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                            int64_t* best, int32_t* n_iter, int32_t* converged) {
+    PCREG_API_BEGIN
+    require_init();
+    check_windows(m, src_offsets, hyp_offsets, nwin, opts, metric, src_nrm, gicp_eps, stop);
+    const WindowLayout L(src_offsets, hyp_offsets, nwin);
+    PCREG_REQUIRE((L.nrows == 0 || src) && (L.nhyp == 0 || (T0_16 && T16)) && ld >= L.nrows, "pcreg_icp_batch_windows: null pointer or bad ld");
+    const bool gicp = metric == PCREG_ICP_PLANE_TO_PLANE;
+    const std::vector<double> hs = to_double_cm(src, is_double, L.nrows, ld);
+    const std::vector<double> hnrm = gicp ? to_double_cm(src_nrm, is_double, L.nrows, ld) : std::vector<double>();
+    for (size_t i = 0; i < (size_t)L.nrows && gicp; ++i) {    // every window's normals, also those of windows no device runs
+        const double x = hnrm[i], y = hnrm[L.nrows + i], z = hnrm[2 * L.nrows + i];
+        const double n = std::sqrt((x * x + y * y) + z * z);
+        PCREG_REQUIRE(std::isfinite(n) && n > 0.0, "icp: zero or non-finite source normal");
+    }
+    if (!stop) { n_iter = nullptr; converged = nullptr; }
+    std::vector<double> rmse_tmp(rmse ? 0 : (size_t)L.nhyp);
+    double* rm = rmse ? rmse : rmse_tmp.data();
+    // contiguous shares of the hypotheses, one host thread + stream per selected device, as icp_batch_host
+    const int nd = (int)std::min<int64_t>(num_slots(), std::min<int64_t>(L.nhyp, (int64_t)m->replicas.size() + 1));
+    if (nd >= 1) {
+        const int64_t per = (L.nhyp + nd - 1) / nd;
+        std::vector<int> rc((size_t)nd, PCREG_OK);
+        std::vector<std::thread> workers;
+        auto run = [&](int k) {
+            const int64_t h0 = k * per, h1 = std::min(L.nhyp, h0 + per);
+            if (h1 <= h0) return;
+            rc[k] = guarded([&]() { use_slot(k); icp_windows_host_slice(m->on_slot(k), L, hs, w_src, hnrm, T0_16, h0, h1, *opts, stop, metric, gicp_eps,
+                                                                      T16, rm, n_used, status, idx, rmse_hist, n_iter, converged); });
+        };
+        for (int k = 1; k < nd; ++k) workers.emplace_back(run, k);
+        run(0);
+        for (auto& w : workers) w.join();
+        use_slot(0);
+        for (int k = 0; k < nd; ++k) if (rc[k] != PCREG_OK) return rc[k];
+    }
+    if (best) {                                           // per window: first-index arg-min, NaN never wins, relative to the window
+        for (int64_t w = 0; w < nwin; ++w) {
+            int64_t bi = -1;
+            for (int64_t h = L.hyp_off[w]; h < L.hyp_off[w + 1]; ++h)
+                if (rm[h] == rm[h] && (bi < 0 || rm[h] < rm[L.hyp_off[w] + bi])) bi = h - L.hyp_off[w];
+            best[w] = bi;
+        }
+    }
+    return PCREG_OK;
+    PCREG_API_END
+}
+
+int pcreg_icp_batch_windows_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                                const double* d_src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin, const double* d_T0_16,
+                                const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop, double* d_T16, double* d_rmse,
+                                int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
+                                int32_t* d_n_iter, int32_t* d_converged, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    check_windows(m, src_offsets, hyp_offsets, nwin, opts, metric, d_src_nrm, gicp_eps, stop);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    const WindowLayout L(src_offsets, hyp_offsets, nwin);
+    icp_windows_run(m, L, d_src, d_w_src, d_src_nrm, d_T0_16, *opts, stop, metric, gicp_eps, d_T16, d_rmse, d_n_used, d_status, d_idx,
+                    d_rmse_hist, d_best, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, (cudaStream_t)stream);
     return PCREG_OK;
     PCREG_API_END
 }

@@ -18,6 +18,7 @@
 #include <float.h>
 #include <stdlib.h>
 #include <algorithm>
+#include <type_traits>
 
 #include "pcreg_internal.h"
 #include "pcreg_dev.cuh"
@@ -67,13 +68,30 @@ __device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<M
     return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
 }
 
+// The source rows of a block's hypothesis: rows r0 .. r0 + ns - 1 of the source arrays, its idx_out block at idx_base (windowed calls).
+struct FusedWindow { int64_t r0, idx_base; int ns; };
+template <bool WIN, class Args>
+__device__ __forceinline__ FusedWindow fused_window(const Args& a, int64_t h) {
+    if constexpr (WIN) {
+        int lo = 0, hi = a.nwin - 1;            // the last window w with win_hyp[w] <= h (windows without hypotheses are skipped)
+        while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (a.win_hyp[mid] <= h) lo = mid; else hi = mid - 1; }
+        const int64_t r0 = a.win_src[lo];
+        const int ns = (int)(a.win_src[lo + 1] - r0);
+        return FusedWindow{r0, a.win_idx[lo] + (h - a.win_hyp[lo]) * (int64_t)ns, ns};
+    } else {
+        return FusedWindow{0, 0, a.ns};
+    }
+}
+
 // KNN = the trimmed mode (its selection scratch -- 18 KB of shared memory -- exists only in that instantiation).
 // STOP = the tolerance stop (pcreg_icp_batch_stop): a stop -- by the rule or by a degenerate update -- makes the block's next
 // pass its final scoring pass, after which the block exits.  The STOP = false instantiations are the loop without it.
 // METRIC = 0 point-to-point; 1 point-to-plane (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered
 // there; 2 plane-to-plane (pcreg_icp_batch_gicp): the same, and the source normal of each correspondence rotated by the pose.
-template <bool KNN, bool STOP, int METRIC>
-__global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ FusedArgs a) {
+// WIN = a windowed call (pcreg_icp_batch_windows, FusedWinArgs): a prologue finds the block's window; from there on the block runs
+// exactly as in a call on that window alone (its rows, ns, perm / tie_order entries and idx_out block).
+template <bool KNN, bool STOP, int METRIC, bool WIN = false>
+__global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ std::conditional_t<WIN, FusedWinArgs, FusedArgs> a) {
     constexpr int NS = icp_nsums<METRIC>;
     extern __shared__ __align__(16) unsigned char dyn[];
     __shared__ double Ts[16];
@@ -83,7 +101,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     __shared__ int s_stop;                                  // STOP: the next pass is the final one
     __shared__ double s_ring[2 * ICP_STOP_WINDOW_MAX];      // STOP: thread 0's window of update motions
 
-    const int ns = a.ns;
+    const FusedWindow W = fused_window<WIN>(a, blockIdx.x);
+    const int ns = W.ns;
     int32_t* __restrict__ idx_s = (int32_t*)dyn;
     unsigned long long* __restrict__ keys_s = (unsigned long long*)(dyn + (((size_t)ns * 4 + 15) / 16) * 16);    // KNN mode only
     const int64_t h = blockIdx.x;
@@ -123,7 +142,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             if (knn) w = (j >= 0 && key_selected(keys_s[i], vK, all_eq)) ? 1.0 : 0.0;
             else if (a.mode == PCREG_ICP_PLAIN) w = keep ? 1.0 : 0.0;
             else if (keep) w = fmax(__dsub_rn(a.R_w, __dsqrt_rn(d)), 0.0);
-            if (a.w_src) w = __dmul_rn(w, a.w_src[i]);
+            if (a.w_src) w = __dmul_rn(w, a.w_src[W.r0 + i]);
             return w;
         };
         if (timing) t_mark = clock64();
@@ -132,8 +151,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             const bool has1 = i1 < ns;
             const int i1c = has1 ? i1 : i0;
             double q0x, q0y, q0z, q1x, q1y, q1z;
-            quick_tf(Ts, a.sx[i0], a.sy[i0], a.sz[i0], q0x, q0y, q0z);
-            quick_tf(Ts, a.sx[i1c], a.sy[i1c], a.sz[i1c], q1x, q1y, q1z);
+            quick_tf(Ts, a.sx[W.r0 + i0], a.sy[W.r0 + i0], a.sz[W.r0 + i0], q0x, q0y, q0z);
+            quick_tf(Ts, a.sx[W.r0 + i1c], a.sy[W.r0 + i1c], a.sz[W.r0 + i1c], q1x, q1y, q1z);
             uint2 hd0 = make_uint2(0u, 0u), hd1 = make_uint2(0u, 0u);
             float x0, y0, z0, x1, y1, z1;
             const bool ok0 = vox_lookup(V, q0x, q0y, q0z, hd0, x0, y0, z0);
@@ -185,7 +204,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 const long long K = (long long)floor(a.k_frac * (double)nkept + 0.5);     // MATLAB round (AlignPoints_KNN.m:21)
                 return K > nkept ? nkept : K;
             };
-            block_hist_finish(keys_s, ns, bins, k_of_kept, hsel, vK, all_eq, a.tie_order);
+            block_hist_finish(keys_s, ns, bins, k_of_kept, hsel, vK, all_eq, WIN ? a.tie_order + W.r0 : a.tie_order);
         }
         if (timing) { const long long t = clock64(); t_sel += t - t_mark; t_mark = t; }
         // ---- weights + the 17 sums (thread t: correspondences t, t + UPD_THREADS, ... in this order, as k_icp_update) ----
@@ -198,13 +217,13 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 if (knn && !(j >= 0 && key_selected(keys_s[i], vK, all_eq))) continue;
 #endif
                 double qx, qy, qz;
-                quick_tf(Ts, a.sx[i], a.sy[i], a.sz[i], qx, qy, qz);
+                quick_tf(Ts, a.sx[W.r0 + i], a.sy[W.r0 + i], a.sz[W.r0 + i], qx, qy, qz);
                 const ModelPointD m = a.g.md[j >= 0 ? j : 0];
                 const double d = j >= 0 ? dist2_exact(m.x, m.y, m.z, qx, qy, qz) : (double)INFINITY;      // the NN step's d2, bit for bit
                 const double w = weight_of(i, j, d);
                 if (w > 0.0) ++n_used;
                 if constexpr (METRIC == ICP_M_GICP)
-                    icp_accumulate_gicp(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], a.snx[i], a.sny[i], a.snz[i], Ts, a.gicp_eps, px, py, pz);
+                    icp_accumulate_gicp(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], a.snx[W.r0 + i], a.sny[W.r0 + i], a.snz[W.r0 + i], Ts, a.gicp_eps, px, py, pz);
                 else if constexpr (METRIC == ICP_M_PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
                 else icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
             }
@@ -241,8 +260,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     if (tid < 16) a.T[h * 16 + tid] = Ts[tid];
     if (tid == 0) a.frozen[h] = s_frozen;
     if (a.idx_out) {
-        int32_t* __restrict__ out = a.idx_out + h * (int64_t)ns;
-        for (int r = tid; r < ns; r += UPD_THREADS) out[a.perm ? a.perm[r] : r] = idx_s[r];
+        int32_t* __restrict__ out = a.idx_out + (WIN ? W.idx_base : h * (int64_t)ns);
+        for (int r = tid; r < ns; r += UPD_THREADS) out[a.perm ? a.perm[W.r0 + r] : r] = idx_s[r];
     }
     if (a.counters) {
 #pragma unroll
@@ -267,10 +286,16 @@ size_t icp_fused_smem(int64_t ns, int mode) {
     return (((size_t)ns * 4 + 15) / 16) * 16 + (mode == PCREG_ICP_KNN ? (size_t)ns * 8 : 0);
 }
 
-template <int METRIC>
+template <int METRIC, bool WIN = false>
 static const void* fused_kernel(bool knn, bool stop) {
-    return knn ? (stop ? (const void*)k_icp_fused<true, true, METRIC> : (const void*)k_icp_fused<true, false, METRIC>)
-               : (stop ? (const void*)k_icp_fused<false, true, METRIC> : (const void*)k_icp_fused<false, false, METRIC>);
+    return knn ? (stop ? (const void*)k_icp_fused<true, true, METRIC, WIN> : (const void*)k_icp_fused<true, false, METRIC, WIN>)
+               : (stop ? (const void*)k_icp_fused<false, true, METRIC, WIN> : (const void*)k_icp_fused<false, false, METRIC, WIN>);
+}
+
+static bool fused_fits(const void* fn, int64_t ns, int mode) {
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, fn) != cudaSuccess) { cudaGetLastError(); return false; }
+    return icp_fused_smem(ns, mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
 }
 
 // Point-to-point calls keep the check they always had (the static shared memory of k_icp_fused<true, false, 0>); the other metrics
@@ -285,32 +310,42 @@ bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pc
     const bool knn = o.mode == PCREG_ICP_KNN;
     const void* fn = metric == ICP_M_POINT ? (const void*)k_icp_fused<true, false, ICP_M_POINT>
                    : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE>(knn, stop) : fused_kernel<ICP_M_GICP>(knn, stop);
-    cudaFuncAttributes fa;
-    if (cudaFuncGetAttributes(&fa, fn) != cudaSuccess) { cudaGetLastError(); return false; }
-    return icp_fused_smem(ns, o.mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
+    return fused_fits(fn, ns, o.mode);
 }
 
-template <bool KNN, bool STOP, int METRIC>
-static void fused_launch_one(const FusedArgs& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
-    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, METRIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
-    k_icp_fused<KNN, STOP, METRIC><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, bool stop, int metric) {
+    if (!m->has_vox || o.nn != PCREG_NN_GRID || ns_max >= ((int64_t)1 << 30)) return false;
+    const bool knn = o.mode == PCREG_ICP_KNN;
+    const void* fn = metric == ICP_M_POINT ? fused_kernel<ICP_M_POINT, true>(knn, stop)
+                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE, true>(knn, stop) : fused_kernel<ICP_M_GICP, true>(knn, stop);
+    return fused_fits(fn, ns_max, o.mode);
 }
 
-template <int METRIC>
-static void fused_launch_metric(const FusedArgs& a, int64_t nhyp, bool stop, size_t dyn, cudaStream_t st) {
+template <bool KNN, bool STOP, int METRIC, bool WIN, class Args>
+static void fused_launch_one(const Args& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
+    PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, METRIC, WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+    k_icp_fused<KNN, STOP, METRIC, WIN><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
+}
+
+template <int METRIC, bool WIN, class Args>
+static void fused_launch_metric(const Args& a, int64_t nhyp, bool stop, size_t dyn, cudaStream_t st) {
     const bool knn = a.mode == PCREG_ICP_KNN;
-    if (knn && !stop)       fused_launch_one<true, false, METRIC>(a, nhyp, dyn, st);
-    else if (!knn && !stop) fused_launch_one<false, false, METRIC>(a, nhyp, dyn, st);
-    else if (knn)           fused_launch_one<true, true, METRIC>(a, nhyp, dyn, st);
-    else                    fused_launch_one<false, true, METRIC>(a, nhyp, dyn, st);
+    if (knn && !stop)       fused_launch_one<true, false, METRIC, WIN>(a, nhyp, dyn, st);
+    else if (!knn && !stop) fused_launch_one<false, false, METRIC, WIN>(a, nhyp, dyn, st);
+    else if (knn)           fused_launch_one<true, true, METRIC, WIN>(a, nhyp, dyn, st);
+    else                    fused_launch_one<false, true, METRIC, WIN>(a, nhyp, dyn, st);
 }
 
-void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) {
+template <bool WIN, class Args>
+static void fused_launch(const Args& a, int64_t nhyp, bool stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
-    if (a.snx)      fused_launch_metric<ICP_M_GICP>(a, nhyp, stop, dyn, st);
-    else if (a.nrm) fused_launch_metric<ICP_M_PLANE>(a, nhyp, stop, dyn, st);
-    else            fused_launch_metric<ICP_M_POINT>(a, nhyp, stop, dyn, st);
+    if (a.snx)      fused_launch_metric<ICP_M_GICP, WIN>(a, nhyp, stop, dyn, st);
+    else if (a.nrm) fused_launch_metric<ICP_M_PLANE, WIN>(a, nhyp, stop, dyn, st);
+    else            fused_launch_metric<ICP_M_POINT, WIN>(a, nhyp, stop, dyn, st);
     PCREG_LAUNCHED();
 }
+
+void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) { fused_launch<false>(a, nhyp, stop, st); }
+void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, bool stop, cudaStream_t st) { fused_launch<true>(a, nhyp, stop, st); }
 
 }  // namespace pcreg

@@ -56,9 +56,21 @@ struct FusedArgs {
     // plane-to-plane metric (null: the other two): unit source normals in the order of sx / sy / sz, and the covariance epsilon
     const double* snx; const double* sny; const double* snz; double gicp_eps;
 };
+// Windowed calls (pcreg_icp_batch_windows; the k_icp_fused<*, *, *, true> instantiations): the source arrays, w_src, the source
+// normals, perm and tie_order are the concatenation of nwin windows (column stride of sx / sy / sz: the total row count), and
+// ns is the largest window's row count.  Window w owns rows win_src[w] .. win_src[w + 1] - 1 and hypotheses win_hyp[w] ..
+// win_hyp[w + 1] - 1; its perm / tie_order entries are relative to its first row, and its [H_w][ns_w] block of idx_out starts at
+// win_idx[w].
+struct FusedWinArgs : FusedArgs {
+    const int64_t* win_src; const int64_t* win_hyp; const int64_t* win_idx;   // device, [nwin + 1], [nwin + 1], [nwin]
+    int32_t nwin;
+};
 size_t icp_fused_smem(int64_t ns, int mode);
 bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, int metric);
 void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
+// windowed calls: the instantiation they launch fits the largest window (ns_max) in shared memory on the model's voxel map
+bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, bool stop, int metric);
+void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
 
 __device__ __forceinline__ void flush_counters(unsigned long long* counters, unsigned long long n_pts,
                                                unsigned long long n_cells, unsigned long long n_nodes, int i_pts = 0, int i_cells = 1,

@@ -280,7 +280,8 @@ struct IcpUpdateArgs {
     const double* snx; const double* sny; const double* snz; double gicp_eps;
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
-void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st);
+// d_seg (optional, device [nseg + 1]): one arg-min per segment of the rmse array, each relative to its segment
+void icp_argmin_launch(const double* d_rmse, int64_t nhyp, int64_t* d_best, cudaStream_t st, const int64_t* d_seg = nullptr, int64_t nseg = 1);
 
 // getLocalPoints.m batched over centres with the neighbourhoods left on the device (local_points.cu)
 struct LocalPointsDev {

@@ -32,12 +32,14 @@
 //                                                      -> matches (Px2 uint32, 1-based), matchMetric (Px1)   (getMatches.m)
 //   'icp', handle, src(Nx3), T0(4x4xH), opts(struct)[, w_src]
 //                                                      -> T(4x4xH), rmse(Hx1), n_used, status, best(1-based), idx(NxH)
+// The ICP of many matching windows in one call has a gateway of its own (pcreg_mex_windows.cpp).
 #include <string.h>
 #include <string>
 #include <vector>
 
 #include "mex.h"
 #include "../../include/pcreg.h"
+#include "pcreg_mex_util.h"
 
 namespace {
 
@@ -63,17 +65,7 @@ bool ensure_init(const mxArray* devices) {
     return true;
 }
 
-bool is_pts(const mxArray* a) { return a && (mxIsDouble(a) || mxIsSingle(a)) && !mxIsComplex(a) && mxGetN(a) == 3; }
 mxArray* empty() { return mxCreateDoubleMatrix(0, 0, mxREAL); }
-double field_or(const mxArray* s, const char* name, double dflt) {
-    if (!s || !mxIsStruct(s)) return dflt;
-    const mxArray* f = mxGetField(s, 0, name);
-    return (f && !mxIsEmpty(f)) ? mxGetScalar(f) : dflt;
-}
-pcreg_model* handle_of(const mxArray* a) {
-    if (!a || mxGetClassID(a) != mxUINT64_CLASS || mxGetNumberOfElements(a) != 1) return nullptr;
-    return (pcreg_model*)(uintptr_t)(*(const uint64_t*)mxGetData(a));
-}
 
 // ---- commands: each returns false with g_fail set on error ----
 bool cmd_model_create(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
@@ -382,15 +374,7 @@ bool cmd_icp(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         g_fail = "icp: need (handle, src Nx3, T0 4x4xH double, opts struct[, w_src])";
         return false;
     }
-    pcreg_icp_opts o;
-    pcreg_icp_opts_default(&o);
-    o.mode = (int)field_or(prhs[4], "mode", o.mode);
-    o.iters = (int)field_or(prhs[4], "iters", o.iters);
-    o.k_frac = field_or(prhs[4], "k_frac", o.k_frac);
-    o.R_w = field_or(prhs[4], "R_w", o.R_w);
-    o.thDist2 = field_or(prhs[4], "thDist2", o.thDist2);
-    o.nn = (int)field_or(prhs[4], "nn", o.nn);
-    o.reflection_fix = (int)field_or(prhs[4], "reflection_fix", 0);
+    const pcreg_icp_opts o = icp_opts_of(prhs[4]);
     const int64_t ns = (int64_t)mxGetM(prhs[2]);
     const int64_t H = (int64_t)(mxGetNumberOfElements(prhs[3]) / 16);
     const double* w = (nrhs > 5 && mxIsDouble(prhs[5]) && (int64_t)mxGetNumberOfElements(prhs[5]) == ns) ? mxGetPr(prhs[5]) : nullptr;

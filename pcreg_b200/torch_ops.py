@@ -4,10 +4,11 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import _lib as L
-from .api import GICP_EPS, METRICS, PLANE_TO_PLANE, Model, icp_opts
+from .api import GICP_EPS, ICP_PLANE_TO_PLANE, METRICS, PLANE_TO_PLANE, Model, icp_opts
 
 
 def T_to_abi_t(T: torch.Tensor) -> torch.Tensor:
@@ -39,6 +40,16 @@ class IcpDeviceBuffers:
         # filled by a call with a tolerance stop: pose updates applied, 1 = stopped by the tolerance
         self.n_iter = torch.empty(nhyp, dtype=i32, device=device) if want_n_iter else None
         self.converged = torch.empty(nhyp, dtype=i32, device=device) if want_n_iter else None
+
+
+class IcpWindowsDeviceBuffers(IcpDeviceBuffers):
+    """Output tensors of one windowed call (icp_windows_device): per-hypothesis outputs as IcpDeviceBuffers, idx ragged (n_idx =
+    sum over the windows of H_w * ns_w, window-major) and best [nwin]."""
+
+    def __init__(self, nhyp: int, n_idx: int, nwin: int, iters: int, device, want_idx=False, want_hist=False, want_n_iter=False):
+        super().__init__(nhyp, 0, iters, device, False, want_hist, want_n_iter)
+        self.idx = torch.empty(n_idx, dtype=torch.int32, device=device) if want_idx else None
+        self.best = torch.empty(nwin, dtype=torch.int64, device=device)
 
 
 def _p(t):
@@ -88,4 +99,36 @@ def icp_batch_device(model: Model, src_cm: torch.Tensor, w_src, T0_abi: torch.Te
                                                  _p(out.idx), _p(out.hist), _p(out.best), _p(out.n_iter), _p(out.converged),
                                                  C.c_void_p(st.cuda_stream)),
                 "pcreg_icp_batch_stop_dev")
+    return out
+
+
+def icp_windows_device(model: Model, src_cm: torch.Tensor, src_offsets, w_src, T0_abi: torch.Tensor, hyp_offsets, opts,
+                       out: IcpWindowsDeviceBuffers, stream=None, stop=None, metric="point_to_point", src_normals=None, gicp_eps=GICP_EPS):
+    """Run pcreg_icp_batch_windows_dev on tensors already resident on the library's device.
+
+    src_cm: float64 [3, ns_total], the windows' sources one after the other (column-major ns_total x 3); src_offsets / hyp_offsets:
+    HOST sequences of nwin + 1 row / hypothesis offsets; T0_abi: float64 [H,16] column-major records grouped by window; w_src: CUDA
+    float64 [ns_total] or None.  metric="plane_to_plane" needs src_normals, a CUDA float64 [ns_total, 3] tensor."""
+    if not (src_cm.is_cuda and T0_abi.is_cuda):
+        raise L.PcregError("icp_windows_device needs CUDA tensors (there is no CPU fallback)")
+    assert src_cm.dtype == torch.float64 and src_cm.is_contiguous() and src_cm.shape[0] == 3
+    assert T0_abi.dtype == torch.float64 and T0_abi.is_contiguous()
+    soff = np.ascontiguousarray(np.asarray(src_offsets, dtype=np.int64))
+    hoff = np.ascontiguousarray(np.asarray(hyp_offsets, dtype=np.int64))
+    nwin = soff.shape[0] - 1
+    if hoff.shape[0] != nwin + 1 or soff[-1] != src_cm.shape[1] or hoff[-1] != T0_abi.shape[0]:
+        raise ValueError("src_offsets / hyp_offsets must be nwin + 1 offsets ending at ns_total / the number of poses")
+    sn_cm = None
+    if metric == PLANE_TO_PLANE:
+        if src_normals is None or not (src_normals.is_cuda and src_normals.dtype == torch.float64 and tuple(src_normals.shape) == (src_cm.shape[1], 3)):
+            raise ValueError("metric='plane_to_plane' needs src_normals, a CUDA float64 [ns_total, 3] tensor")
+        sn_cm = src_normals.t().contiguous()
+    mcode = ICP_PLANE_TO_PLANE if metric == PLANE_TO_PLANE else METRICS[metric]
+    st = stream if stream is not None else torch.cuda.current_stream()
+    L.check(L.lib().pcreg_icp_batch_windows_dev(model.handle, _p(src_cm), soff.ctypes.data_as(L.c_i64p), _p(w_src), _p(sn_cm),
+                                                float(gicp_eps), hoff.ctypes.data_as(L.c_i64p), nwin, _p(T0_abi), C.byref(opts), mcode,
+                                                C.byref(stop) if stop is not None else None, _p(out.T), _p(out.rmse), _p(out.n_used),
+                                                _p(out.status), _p(out.idx), _p(out.hist), _p(out.best), _p(out.n_iter), _p(out.converged),
+                                                C.c_void_p(st.cuda_stream)),
+            "pcreg_icp_batch_windows_dev")
     return out
