@@ -436,7 +436,49 @@ int  pcreg_icp_batch_windows_dev(const pcreg_model* m, const double* d_src, cons
                                  double* d_T16, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
                                  double* d_rmse_hist, int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev,_windows,_windows_dev} or pcreg_nn_search call,
+/* ---- pose extrapolation (accelerated ICP; Besl & McKay 1992, section IV; pcregistericp's 'Extrapolate') ------------------------
+ * When the last updates of a hypothesis keep pointing the same way, the pose jumps further along that direction, by a step from a
+ * line fit and a parabola fit of the error against the distance travelled.  Point-to-point only.  The rule (parity with the toolbox is
+ * UNPINNED):
+ *   c: the hypothesis's source centroid, the unweighted FP64 mean of its window's rows (one fixed-order device reduction per window).
+ *   State of a pose T = [R 0; t 1]: x(T) = (qR, qT) in R^7, qR = the unit quaternion (w, x, y, z) of R (Shepperd's largest-diagonal
+ *   branch), qT = c R + t (the image of the centroid: moving both clouds by a common rigid motion leaves the rule unchanged).  Sign of
+ *   qR: for T_0 w >= 0 (at w = 0 the first nonzero component positive); for every later state the one with qR . qR_prev >= 0.
+ *   d(T) = sum w |m - quickTF(s, T)|^2 / sum w over update u's correspondences and weights (the paper's d_k; a closed form of the
+ *   update's 17 sums, centred so that a source far from the model's pivot loses no accuracy).
+ *   Update u (1-based, not degenerate), K_u = T_{u-1} dT the Kabsch pose: Delta_u = x(K_u) - x_{u-1} (x_{u-1} the stored state),
+ *   n_u = |Delta_u|, theta_u = acos(clamp(cos angle(Delta_{u-1}, Delta_u), -1, 1)) in degrees, undefined for u < 2 or a zero norm.
+ *   It extrapolates when u >= 3 and theta_u, theta_{u-1} are both defined and < angle_deg: with v = (0, -n_u, -n_u - n_{u-1}) and
+ *   D = (d(K_u), d_{u-1}, d_{u-2}), v1 = the zero of the least-squares line through (v_i, D_i), v2 = -b / (2a) the vertex of the
+ *   parabola through them, vmax = vmax_scale n_u; dv = v2 if 0 < v2 < v1 < vmax or 0 < v2 < vmax < v1; v1 if 0 < v1 < v2 < vmax,
+ *   0 < v1 < vmax < v2 or (v2 < 0 and 0 < v1 < vmax); vmax if v1 > vmax and v2 > vmax; else 0 (strict compares, NaN fails each).
+ *   With dv > 0: x' = x(K_u) + dv Delta_u / n_u, qR' renormalised, T_u = [R(qR') 0; qT' - c R' 1]; otherwise T_u = K_u.
+ *   Stored: x_u = x' or x(K_u), d_u = d(T_u), Delta_u and n_u as before the jump; n_extrap counts the updates with dv > 0.
+ * Correspondences, rejection, trimming, weights, rmse, the degenerate freeze and the winner are unchanged.  The tolerance stop
+ * measures the motion from T_{u-1} to the pose written, T_u.  The rule is causal: a hypothesis stopped after k updates returns exactly
+ * what the same call with iters = k returns.  Defaults {10, 25} are the paper's; angle_deg outside (0, 180] or a vmax_scale that is not
+ * finite and > 0 returns PCREG_ERR_ARG. */
+typedef struct {
+    double angle_deg;       /* both of the last two direction changes below this: extrapolate  */
+    double vmax_scale;      /* the step is at most vmax_scale n_u                              */
+} pcreg_icp_extrap;
+void pcreg_icp_extrap_default(pcreg_icp_extrap* e);   /* {10, 25} */
+/* Point-to-point batched ICP with pose extrapolation, in the windows layout of pcreg_icp_batch_windows (nwin = 1: one source for every
+ * hypothesis; arguments, outputs, errors and sharding over the devices as there, metric 0).  stop is optional; ex == NULL returns the
+ * bits of pcreg_icp_batch_windows with metric 0.  n_extrap [nhyp] (optional, written only with ex): updates extrapolated. */
+int  pcreg_icp_batch_extrap(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                            const double* w_src, const int64_t* hyp_offsets, int64_t nwin, const double* T0_16,
+                            const pcreg_icp_opts* opts, const pcreg_icp_stop* stop, const pcreg_icp_extrap* ex,
+                            double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                            int64_t* best, int32_t* n_iter, int32_t* converged, int32_t* n_extrap);
+/* The same on device arrays, synchronous with respect to `stream` as pcreg_icp_batch_windows_dev (offsets on the host). */
+int  pcreg_icp_batch_extrap_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                                const int64_t* hyp_offsets, int64_t nwin, const double* d_T0_16, const pcreg_icp_opts* opts,
+                                const pcreg_icp_stop* stop, const pcreg_icp_extrap* ex, double* d_T16, double* d_rmse,
+                                int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
+                                int32_t* d_n_iter, int32_t* d_converged, int32_t* d_n_extrap, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev,_windows,_windows_dev,_extrap,_extrap_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
  *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
  *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped

@@ -55,6 +55,10 @@ class IcpStop(C.Structure):
     _fields_ = [("tol_t", C.c_double), ("tol_r_deg", C.c_double), ("window", C.c_int)]
 
 
+class IcpExtrap(C.Structure):
+    _fields_ = [("angle_deg", C.c_double), ("vmax_scale", C.c_double)]
+
+
 # name -> (restype, argtypes): every symbol include/pcreg.h declares
 SIGNATURES = {
     "pcreg_init": (C.c_int, [c_i32p, C.c_int]),
@@ -124,6 +128,14 @@ SIGNATURES = {
                                               C.c_void_p, C.POINTER(IcpOpts), C.c_int, C.POINTER(IcpStop), C.c_void_p, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p]),
+    "pcreg_icp_extrap_default": (None, [C.POINTER(IcpExtrap)]),
+    "pcreg_icp_batch_extrap": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, c_i64p, c_f64p, c_i64p, C.c_int64, c_f64p,
+                                         C.POINTER(IcpOpts), C.POINTER(IcpStop), C.POINTER(IcpExtrap), c_f64p, c_f64p, c_i32p, c_i32p,
+                                         c_i32p, c_f64p, c_i64p, c_i32p, c_i32p, c_i32p]),
+    "pcreg_icp_batch_extrap_dev": (C.c_int, [C.c_void_p, C.c_void_p, c_i64p, C.c_void_p, c_i64p, C.c_int64, C.c_void_p,
+                                             C.POINTER(IcpOpts), C.POINTER(IcpStop), C.POINTER(IcpExtrap), C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p]),
     "pcreg_set_profiling": (C.c_int, [C.c_int]),
     "pcreg_last_profile": (C.c_int, [c_f64p]),
 }

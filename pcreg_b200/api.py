@@ -14,7 +14,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib as L
-from ._lib import AlignOpts, DescOpts, IcpOpts, IcpStop, MatchOpts, ModelOpts, PcregError, RansacOpts  # noqa: F401
+from ._lib import AlignOpts, DescOpts, IcpExtrap, IcpOpts, IcpStop, MatchOpts, ModelOpts, PcregError, RansacOpts  # noqa: F401
 
 NN_BRUTE, NN_GRID = 0, 1
 ICP_PLAIN, ICP_KNN, ICP_WEIGHTED = 0, 1, 2
@@ -525,9 +525,22 @@ def icp_stop(tol_t, tol_r_deg, window=3) -> IcpStop:
     return IcpStop(float(tol_t), float(tol_r_deg), int(window))
 
 
+def icp_extrap(angle_deg=10.0, vmax_scale=25.0) -> IcpExtrap:
+    return IcpExtrap(float(angle_deg), float(vmax_scale))
+
+
+def _extrap_of(extrapolate, metric):
+    """The `extrapolate` keyword -> an IcpExtrap or None: False / None off, True the defaults (10 deg, 25), or (angle_deg, vmax_scale)."""
+    if extrapolate is None or extrapolate is False:
+        return None
+    if metric != "point_to_point":
+        raise ValueError("extrapolate is defined for metric='point_to_point' only")
+    return icp_extrap() if extrapolate is True else icp_extrap(*extrapolate)
+
+
 def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src=None,
               nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3,
-              metric="point_to_point", src_normals=None, gicp_eps=GICP_EPS):
+              metric="point_to_point", src_normals=None, gicp_eps=GICP_EPS, extrapolate=False):
     """Multi-start ICP of `src` against the resident `model` from the initial poses T0s [H,4,4].
     Returns dict(T [H,4,4], rmse [H], n_used [H], status [H], best, idx [H,ns]?, rmse_hist [H,iters+1]?).
 
@@ -540,7 +553,14 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
     metric="plane_to_plane" is generalized ICP (include/pcreg.h: pcreg_icp_batch_gicp): it needs the model's normals and
     `src_normals` (N x 3, one per source point, e.g. cloud_normals(src)); gicp_eps in (0, 1] is the covariance epsilon.  The C entry
     takes the normals in the source's type, so with a float32 source they are rounded to float32 before the library normalises
-    them in FP64; pass the source as float64 to keep float64 normals."""
+    them in FP64; pass the source as float64 to keep float64 normals.
+
+    extrapolate=True or (angle_deg, vmax_scale) (point-to-point only; default (10, 25)): each hypothesis's pose jumps ahead along its
+    recent path when the last updates keep pointing the same way (Besl & McKay's accelerated ICP; include/pcreg.h: pcreg_icp_extrap).
+    The result then also holds n_extrap [H], the updates that extrapolated."""
+    if _extrap_of(extrapolate, metric) is not None:
+        return icp_batch_windows(model, [src], [T0s], mode, iters, k_frac, R_w, thDist2, None if w_src is None else [w_src], nn,
+                                 reflection_fix, return_idx, return_hist, tolerance, window, extrapolate=extrapolate)[0]
     if metric not in METRICS and metric != PLANE_TO_PLANE:
         raise ValueError("metric must be one of %s" % sorted(list(METRICS) + [PLANE_TO_PLANE]))
     if metric == PLANE_TO_PLANE and src_normals is None:
@@ -594,12 +614,14 @@ def icp_batch(model: Model, src, T0s, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w
 
 def icp_batch_windows(model: Model, src_list, T0_list, mode=ICP_PLAIN, iters=50, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src_list=None,
                       nn=NN_BRUTE, reflection_fix=False, return_idx=False, return_hist=False, tolerance=None, window=3,
-                      metric="point_to_point", src_normals_list=None, gicp_eps=GICP_EPS):
+                      metric="point_to_point", src_normals_list=None, gicp_eps=GICP_EPS, extrapolate=False):
     """icp_batch for many matching windows in ONE call (include/pcreg.h: pcreg_icp_batch_windows): window w polishes the poses
     T0_list[w] [H_w,4,4] (H_w may be 0) against its own source cloud src_list[w] [ns_w,3], with w_src_list[w] / src_normals_list[w]
     when given; the model and every other keyword (as icp_batch) are shared.  Returns one dict per window, each what
     icp_batch(model, src_list[w], T0_list[w], ...) returns (best relative to the window, -1 without hypotheses), bit for bit.
-    The windows' sources are passed as float32 only when all of them are float32."""
+    The windows' sources are passed as float32 only when all of them are float32.  extrapolate: as icp_batch
+    (include/pcreg.h: pcreg_icp_batch_extrap; each window's results are then those of its own icp_batch call)."""
+    ex = _extrap_of(extrapolate, metric)
     if metric not in METRICS and metric != PLANE_TO_PLANE:
         raise ValueError("metric must be one of %s" % sorted(list(METRICS) + [PLANE_TO_PLANE]))
     if metric == PLANE_TO_PLANE and src_normals_list is None:
@@ -648,14 +670,20 @@ def icp_batch_windows(model: Model, src_list, T0_list, mode=ICP_PLAIN, iters=50,
     n_iter = np.empty(max(nh, 1), dtype=np.int32) if tolerance is not None else None
     converged = np.empty(max(nh, 1), dtype=np.int32) if tolerance is not None else None
     mcode = ICP_PLANE_TO_PLANE if metric == PLANE_TO_PLANE else METRICS[metric]
-    L.check(L.lib().pcreg_icp_batch_windows(model.handle, cat.ctypes.data_as(C.c_void_p), int(dt == np.float64), cat.shape[0],
-                                            _ptr(soff, L.c_i64p), _ptr(w, L.c_f64p),
-                                            sn.ctypes.data_as(C.c_void_p) if sn is not None else None, float(gicp_eps),
-                                            _ptr(hoff, L.c_i64p), nw, _ptr(T0, L.c_f64p), C.byref(o), mcode,
-                                            C.byref(stop) if stop is not None else None, _ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p),
-                                            _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p), _ptr(hist, L.c_f64p),
-                                            _ptr(best, L.c_i64p), _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p)),
-            "pcreg_icp_batch_windows")
+    n_extrap = np.empty(max(nh, 1), dtype=np.int32) if ex is not None else None
+    outs = (_ptr(T, L.c_f64p), _ptr(rmse, L.c_f64p), _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p), _ptr(idx, L.c_i32p),
+            _ptr(hist, L.c_f64p), _ptr(best, L.c_i64p), _ptr(n_iter, L.c_i32p), _ptr(converged, L.c_i32p))
+    if ex is not None:
+        L.check(L.lib().pcreg_icp_batch_extrap(model.handle, cat.ctypes.data_as(C.c_void_p), int(dt == np.float64), cat.shape[0],
+                                               _ptr(soff, L.c_i64p), _ptr(w, L.c_f64p), _ptr(hoff, L.c_i64p), nw, _ptr(T0, L.c_f64p),
+                                               C.byref(o), C.byref(stop) if stop is not None else None, C.byref(ex), *outs,
+                                               _ptr(n_extrap, L.c_i32p)), "pcreg_icp_batch_extrap")
+    else:
+        L.check(L.lib().pcreg_icp_batch_windows(model.handle, cat.ctypes.data_as(C.c_void_p), int(dt == np.float64), cat.shape[0],
+                                                _ptr(soff, L.c_i64p), _ptr(w, L.c_f64p),
+                                                sn.ctypes.data_as(C.c_void_p) if sn is not None else None, float(gicp_eps),
+                                                _ptr(hoff, L.c_i64p), nw, _ptr(T0, L.c_f64p), C.byref(o), mcode,
+                                                C.byref(stop) if stop is not None else None, *outs), "pcreg_icp_batch_windows")
     Ts = _T_from_abi(T, T.shape[0])
     out = []
     for k in range(nw):
@@ -664,6 +692,8 @@ def icp_batch_windows(model: Model, src_list, T0_list, mode=ICP_PLAIN, iters=50,
         if tolerance is not None:
             r["n_iter"] = n_iter[a:b].copy()
             r["converged"] = converged[a:b].copy()
+        if ex is not None:
+            r["n_extrap"] = n_extrap[a:b].copy()
         if return_idx:
             r["idx"] = idx[int(ioff[k]):int(ioff[k + 1])].reshape(b - a, int(ns[k])).copy()
         if return_hist:

@@ -34,10 +34,11 @@ struct Pose16 { double t[16]; };      // a row-major row-vector pose as a kernel
 // One block per hypothesis.
 // NT = threads per hypothesis: UPD_THREADS (the fused kernel's count, so that both sum in the same order and agree bit for
 // bit) for sources the fused kernel can take, 512 for large sources (C5: 65 536 correspondences per hypothesis).
-// STOP = the tolerance stop (a.stop_iter set); the STOP = false instantiations are the loop without it.
+// STOP = the tolerance stop (a.stop_iter set); the STOP = 0 instantiations are the loop without it; STOP = 2 (METRIC 0 only, a.ex_state
+// set as well) adds the pose extrapolation before the stop rule.
 // METRIC = 1: the point-to-plane metric (a.nrm set): 29 sums, the normals gathered with the model points; 2: plane-to-plane
 // (a.snx set as well): the same, and each correspondence's source normal read with the source point and rotated by the pose.
-template <int NT, bool STOP, int METRIC>
+template <int NT, int STOP, int METRIC>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __grid_constant__ IcpUpdateArgs a) {
     constexpr int NS = icp_nsums<METRIC>;
     constexpr bool MNRM = METRIC != ICP_M_POINT, SNRM = METRIC == ICP_M_GICP;
@@ -184,6 +185,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             if (k >= 0) hist_from = k + a.frozen[h];
             if (a.n_iter) a.n_iter[h] = k >= 0 ? k : a.hist_col;
             if (a.converged) a.converged[h] = k >= 0 && !a.frozen[h];
+            if (STOP == 2 && a.n_extrap) a.n_extrap[h] = (int32_t)a.ex_state[h * EXTRAP_STATE + 18];
         }
         if (a.rmse_hist) for (int c = hist_from; c <= a.hist_col; ++c) a.rmse_hist[h * a.hist_stride + c] = rmse;
         float moved = 0.f;
@@ -197,6 +199,8 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
                 a.frozen[h] = 1;
                 if (STOP) a.stop_iter[h] = a.hist_col;
             } else {
+                // extrapolation: Tn becomes the pose actually written, so the motion bound below and the stop rule see the jump
+                if constexpr (STOP == 2) icp_extrap_update(a.ex, s, a.pivot, a.ex_cen, Tc, Tn, a.hist_col + 1, a.ex_state + h * EXTRAP_STATE);
                 for (int k = 0; k < 16; ++k) a.T[h * 16 + k] = Tn[k];
                 if (a.delta) {
                     // upper bound of how far this update moves any source point:
@@ -266,6 +270,19 @@ __global__ void __launch_bounds__(1024) k_src_stats(const double* __restrict__ s
         stats[0] = cen[0]; stats[1] = cen[1]; stats[2] = cen[2];
         stats[3] = sqrt(m) * (1.0 + 1e-12);
     }
+}
+
+// Unweighted FP64 centroid of each window's source rows (the pose extrapolation's c), one block per window: block w sums rows
+// off[w] .. off[w + 1] - 1 of src (column stride ld) in a fixed order (thread t: rows t, t + 256, ...; then block_sum's tree), so
+// the result depends on the window's rows alone.
+__global__ void __launch_bounds__(256) k_src_centroid(const double* __restrict__ src, int64_t ld, const int64_t* __restrict__ off,
+                                                      double* __restrict__ cen /*[nwin][3]*/) {
+    __shared__ double red[3 * 32];
+    const int64_t r0 = off[blockIdx.x], ns = off[blockIdx.x + 1] - r0;
+    double s[3] = {0.0, 0.0, 0.0};
+    for (int64_t i = r0 + threadIdx.x; i < r0 + ns; i += 256) { s[0] += src[i]; s[1] += src[ld + i]; s[2] += src[2 * ld + i]; }
+    block_sum<3>(s, red);
+    if (threadIdx.x == 0) for (int k = 0; k < 3; ++k) cen[blockIdx.x * 3 + k] = ns > 0 ? s[k] / (double)ns : 0.0;
 }
 
 // first-index arg-min over hypotheses, NaN never wins (-1: none); one block per segment: block b takes rmse[seg[b] .. seg[b + 1] - 1]
@@ -447,9 +464,16 @@ void transpose16_launch(const double* d_in, double* d_out, int64_t n, cudaStream
 template <int METRIC>
 static void icp_update_launch_metric(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
     const bool stop = a.stop_iter != nullptr;
-    if (a.ns > 20000) { if (stop) k_icp_update<512, true, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, false, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); }
-    else if (stop)    k_icp_update<UPD_THREADS, true, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
-    else              k_icp_update<UPD_THREADS, false, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    if constexpr (METRIC == ICP_M_POINT) {
+        if (a.ex_state) {
+            if (a.ns > 20000) k_icp_update<512, 2, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a);
+            else              k_icp_update<UPD_THREADS, 2, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+            return;
+        }
+    }
+    if (a.ns > 20000) { if (stop) k_icp_update<512, 1, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); else k_icp_update<512, 0, METRIC><<<(unsigned)nhyp, 512, 0, st>>>(a); }
+    else if (stop)    k_icp_update<UPD_THREADS, 1, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+    else              k_icp_update<UPD_THREADS, 0, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
 }
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
     if (a.snx)      icp_update_launch_metric<ICP_M_GICP>(a, nhyp, st);
@@ -473,7 +497,8 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx,
                     double* d_rmse_hist, int64_t* d_best, cudaStream_t st,
                     const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr,
-                    int metric = ICP_M_POINT, const double* d_src_nrm = nullptr /*ICP_M_GICP: col-major ns x 3*/, double gicp_eps = 0.0) {
+                    int metric = ICP_M_POINT, const double* d_src_nrm = nullptr /*ICP_M_GICP: col-major ns x 3*/, double gicp_eps = 0.0,
+                    const IcpExtrapRule* ex = nullptr /*needs stop*/, const double* d_ex_cen = nullptr /*[3]*/, int32_t* d_n_extrap = nullptr) {
     PCREG_REQUIRE(m && d_src && d_T0_cm && d_T16_cm, "icp: null pointer");
     const bool plane = metric != ICP_M_POINT, gicp = metric == ICP_M_GICP;
     const ModelPointD* nrm = plane ? m->nrm.p : nullptr;
@@ -492,7 +517,9 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     const double t_enter = now_ms();
     double t_alloc = 0, t_sorted = 0, t_enq = 0;
 
-    const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop != nullptr, metric);
+    PCREG_REQUIRE(!ex || (stop && d_ex_cen && metric == ICP_M_POINT), "icp: extrapolation needs a stop rule, the centroid and point-to-point");
+    const int stop_mode = ex ? 2 : stop ? 1 : 0;
+    const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop_mode, metric);
     // chunk the hypotheses so that the per-correspondence scratch stays bounded
     const size_t total_b = c.total_mem;         // queried once at pcreg_init (cudaMemGetInfo costs up to tens of ms per call)
     const size_t per_hyp = (size_t)ns * (4 + 4 + 8 + (o.mode == PCREG_ICP_KNN ? 8 : 0) + (o.nn == PCREG_NN_GRID ? 8 + (m->has_vox ? 0 : 28 + 4 * 64 + 4 * 448 / 16) : 0));
@@ -522,6 +549,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     // tolerance stop, per-pass path: per-hypothesis stop state (the fused kernel keeps it in shared memory)
     DevBuf<int32_t> stop_iter(stop && !fused ? (size_t)nhyp : 0);
     DevBuf<double> stop_ring(stop && !fused ? (size_t)nhyp * 2 * ICP_STOP_WINDOW_MAX : 0);
+    DevBuf<double> ex_state(ex && !fused ? (size_t)nhyp * EXTRAP_STATE : 0);
     // profiling with the tolerance stop: the passes each hypothesis ran follow from n_iter and status
     DevBuf<int32_t> n_iter_tmp(stop && prof && !d_n_iter ? (size_t)nhyp : 0);
     if (n_iter_tmp.p) d_n_iter = n_iter_tmp.p;
@@ -582,6 +610,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     PCREG_CUDA(cudaMemsetAsync(frozen.p, 0, frozen.bytes(), st));
     PCREG_CUDA(cudaMemsetAsync(counters.p, 0, counters.bytes(), st));
     if (stop_iter.p) PCREG_CUDA(cudaMemsetAsync(stop_iter.p, 0xff, stop_iter.bytes(), st));      // -1: running
+    if (ex_state.p) PCREG_CUDA(cudaMemsetAsync(ex_state.p, 0, ex_state.bytes(), st));
     transpose16_launch(d_T0_cm, Twork.p, nhyp, st);
 
     std::vector<EventPair> evs;
@@ -642,8 +671,9 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         fa.counters = (prof && c.profiling_counters) ? counters.p : nullptr;
         fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
         fa.snx = snx; fa.sny = sny; fa.snz = snz; fa.gicp_eps = gicp_eps;
+        if (ex) { fa.ex = *ex; fa.ex_cen = d_ex_cen; fa.n_extrap = d_n_extrap; }
         ev_begin(0);
-        icp_fused_launch(fa, nhyp, stop != nullptr, st);
+        icp_fused_launch(fa, nhyp, stop_mode, st);
         ev_end();
         transpose16_launch(Twork.p, d_T16_cm, nhyp, st);
         if (d_status) PCREG_CUDA(cudaMemcpyAsync(d_status, frozen.p, (size_t)nhyp * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
@@ -740,6 +770,10 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     ua.stop_iter = stop_iter.p + h0; ua.stop_ring = stop_ring.p + h0 * 2 * ICP_STOP_WINDOW_MAX; ua.stop = rule;
                     ua.n_iter = d_n_iter ? d_n_iter + h0 : nullptr; ua.converged = d_converged ? d_converged + h0 : nullptr;
                 }
+                if (ex) {
+                    ua.ex = *ex; ua.ex_state = ex_state.p + h0 * EXTRAP_STATE; ua.ex_cen = d_ex_cen;
+                    ua.n_extrap = d_n_extrap ? d_n_extrap + h0 : nullptr;
+                }
                 ev_begin(1);
                 icp_update_launch(ua, hn, ls);
                 ev_end();
@@ -826,7 +860,7 @@ struct WindowLayout {
 
 // When a windowed call runs as one launch of the fused kernel.  The alternative is a loop over the windows through icp_run, each
 // window at least an NN and an update launch per pass plus host synchronisations (DESIGN.md section 3.3 has the measurements).
-static bool windows_use_fused(const pcreg_model* m, const WindowLayout& L, const pcreg_icp_opts& o, bool stop, int metric) {
+static bool windows_use_fused(const pcreg_model* m, const WindowLayout& L, const pcreg_icp_opts& o, int stop, int metric) {
     if (!icp_fused_windows_fit(m, L.ns_max, o, stop, metric)) return false;
     if (const char* e = getenv("PCREG_FUSED")) { if (e[0] == '0') return false; if (e[0] == '1') return true; }
     int64_t busy = 0;                          // windows with hypotheses
@@ -839,7 +873,8 @@ static bool windows_use_fused(const pcreg_model* m, const WindowLayout& L, const
 static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const double* d_src, const double* d_w, const double* d_src_nrm,
                             const double* d_T0_cm, const pcreg_icp_opts& o, const pcreg_icp_stop* stop, int metric, double gicp_eps,
                             double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist,
-                            int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, cudaStream_t st) {
+                            int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, cudaStream_t st,
+                            const IcpExtrapRule* ex = nullptr, int32_t* d_n_extrap = nullptr) {
     PCREG_REQUIRE(m && d_T16_cm && (L.nrows == 0 || d_src) && (L.nhyp == 0 || d_T0_cm), "icp windows: null pointer");
     const bool gicp = metric == ICP_M_GICP;
     const ModelPointD* nrm = metric != ICP_M_POINT ? m->nrm.p : nullptr;
@@ -857,7 +892,17 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
     PCREG_CUDA(cudaMemcpyAsync(d_soff, L.src_off.data(), (size_t)(L.nwin + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_hoff, L.hyp_off.data(), (size_t)(L.nwin + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_ioff, L.idx_off.data(), (size_t)L.nwin * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    const bool fused = nhyp > 0 && windows_use_fused(m, L, o, stop != nullptr, metric);
+    // pose extrapolation: it runs with the caller's stop rule, or with one that never stops (a tolerance of 0 changes no bit)
+    const pcreg_icp_stop never{0.0, 0.0, 1};
+    if (ex && !stop) { stop = &never; d_n_iter = nullptr; d_converged = nullptr; }
+    const int stop_mode = ex ? 2 : stop ? 1 : 0;
+    // the source centroid of every window, from the caller's rows in their order (both paths read it)
+    DevBuf<double> cen(ex ? (size_t)L.nwin * 3 : 0);
+    if (ex) {
+        k_src_centroid<<<(unsigned)L.nwin, 256, 0, st>>>(d_src, nrows, d_soff, cen.p);
+        PCREG_LAUNCHED();
+    }
+    const bool fused = nhyp > 0 && windows_use_fused(m, L, o, stop_mode, metric);
     // plane-to-plane: every window's source normals normalised and checked before any ICP kernel runs (in the windows' sorted order
     // on the fused path; the loop normalises each window again inside icp_run, from the caller's rows)
     DevBuf<int32_t> sperm(fused ? (size_t)nrows : 0), sinv(fused ? (size_t)nrows : 0);
@@ -898,7 +943,8 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
             icp_run(m, src_w.p, ns, d_w ? d_w + r0 : nullptr, d_T0_cm + h0 * 16, nh, o, d_T16_cm + h0 * 16, d_rmse ? d_rmse + h0 : nullptr,
                     d_n_used ? d_n_used + h0 : nullptr, d_status ? d_status + h0 : nullptr, d_idx ? d_idx + L.idx_off[w] : nullptr,
                     d_rmse_hist ? d_rmse_hist + h0 * hs : nullptr, d_best ? d_best + w : nullptr, st, stop,
-                    d_n_iter ? d_n_iter + h0 : nullptr, d_converged ? d_converged + h0 : nullptr, metric, gicp ? nrm_w.p : nullptr, gicp_eps);
+                    d_n_iter ? d_n_iter + h0 : nullptr, d_converged ? d_converged + h0 : nullptr, metric, gicp ? nrm_w.p : nullptr, gicp_eps,
+                    ex, ex ? cen.p + 3 * w : nullptr, d_n_extrap ? d_n_extrap + h0 : nullptr);
             if (prof) {
                 for (int k = 0; k < 26; ++k) prof_sum[k] += c.profile[k];
                 prof_sum[26] = std::max(prof_sum[26], c.profile[26]);
@@ -935,9 +981,10 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
     fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
     fa.snx = gicp ? snrm.p : nullptr; fa.sny = gicp ? snrm.p + nrows : nullptr; fa.snz = gicp ? snrm.p + 2 * nrows : nullptr; fa.gicp_eps = gicp_eps;
     fa.win_src = d_soff; fa.win_hyp = d_hoff; fa.win_idx = d_ioff; fa.nwin = (int32_t)L.nwin;
+    if (ex) { fa.ex = *ex; fa.ex_cen = cen.p; fa.n_extrap = d_n_extrap; }
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (prof) { e0 = pooled_event(0); e1 = pooled_event(1); PCREG_CUDA(cudaEventRecord(e0, st)); }
-    icp_fused_windows_launch(fa, nhyp, stop != nullptr, st);
+    icp_fused_windows_launch(fa, nhyp, stop_mode, st);
     if (prof) PCREG_CUDA(cudaEventRecord(e1, st));
     transpose16_launch(Twork.p, d_T16_cm, nhyp, st);
     if (d_status) PCREG_CUDA(cudaMemcpyAsync(d_status, frozen.p, (size_t)nhyp * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
@@ -1208,7 +1255,8 @@ static void check_windows(const pcreg_model* m, const int64_t* src_off, const in
 static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, const std::vector<double>& hs, const double* w_src,
                                    const std::vector<double>& hnrm, const double* T0_16, int64_t h0, int64_t h1, const pcreg_icp_opts& o,
                                    const pcreg_icp_stop* stop, int metric, double eps, double* T16, double* rmse, int32_t* n_used,
-                                   int32_t* status, int32_t* idx, double* rmse_hist, int32_t* n_iter, int32_t* converged) {
+                                   int32_t* status, int32_t* idx, double* rmse_hist, int32_t* n_iter, int32_t* converged,
+                                   const IcpExtrapRule* ex, int32_t* n_extrap) {
     PCREG_CUDA(cudaSetDevice(ctx().device));
     cudaStream_t st = 0;
     const int64_t wa = L.window_of(h0), wb = L.window_of(h1 - 1), nw = wb - wa + 1;
@@ -1223,7 +1271,7 @@ static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, 
     DevBuf<double> d_src((size_t)nr * 3), d_w(w_src ? (size_t)nr : 0), d_nrm(hnrm.empty() ? 0 : (size_t)nr * 3);
     DevBuf<double> d_T0((size_t)hn * 16), d_T((size_t)hn * 16), d_rmse((size_t)hn), d_hist(rmse_hist ? (size_t)hn * (o.iters + 1) : 0);
     DevBuf<int32_t> d_nu((size_t)hn), d_st((size_t)hn), d_idx(idx ? (size_t)ni : 0);
-    DevBuf<int32_t> d_nit(n_iter ? (size_t)hn : 0), d_conv(converged ? (size_t)hn : 0);
+    DevBuf<int32_t> d_nit(n_iter ? (size_t)hn : 0), d_conv(converged ? (size_t)hn : 0), d_nex(n_extrap ? (size_t)hn : 0);
     for (int a = 0; a < 3; ++a) {
         PCREG_CUDA(cudaMemcpyAsync(d_src.p + a * nr, hs.data() + a * L.nrows + ra, (size_t)nr * sizeof(double), cudaMemcpyHostToDevice, st));
         if (d_nrm.p) PCREG_CUDA(cudaMemcpyAsync(d_nrm.p + a * nr, hnrm.data() + a * L.nrows + ra, (size_t)nr * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -1231,7 +1279,7 @@ static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, 
     if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src + ra, d_w.bytes(), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
     icp_windows_run(m, S, d_src.p, d_w.p, d_nrm.p, d_T0.p, o, stop, metric, eps, d_T.p, d_rmse.p, d_nu.p, d_st.p, d_idx.p, d_hist.p,
-                    nullptr, d_nit.p, d_conv.p, st);
+                    nullptr, d_nit.p, d_conv.p, st, ex, d_nex.p);
     PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
@@ -1240,17 +1288,16 @@ static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, 
     if (rmse_hist) PCREG_CUDA(cudaMemcpyAsync(rmse_hist + h0 * (o.iters + 1), d_hist.p, d_hist.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_iter) PCREG_CUDA(cudaMemcpyAsync(n_iter + h0, d_nit.p, d_nit.bytes(), cudaMemcpyDeviceToHost, st));
     if (converged) PCREG_CUDA(cudaMemcpyAsync(converged + h0, d_conv.p, d_conv.bytes(), cudaMemcpyDeviceToHost, st));
+    if (n_extrap) PCREG_CUDA(cudaMemcpyAsync(n_extrap + h0, d_nex.p, d_nex.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaStreamSynchronize(st));
 }
 
-int pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+// pcreg_icp_batch_windows and pcreg_icp_batch_extrap (ex != nullptr) after the argument checks
+static int icp_windows_host(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
                             const double* w_src, const void* src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
                             const double* T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
                             double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
-                            int64_t* best, int32_t* n_iter, int32_t* converged) {
-    PCREG_API_BEGIN
-    require_init();
-    check_windows(m, src_offsets, hyp_offsets, nwin, opts, metric, src_nrm, gicp_eps, stop);
+                            int64_t* best, int32_t* n_iter, int32_t* converged, const IcpExtrapRule* ex, int32_t* n_extrap) {
     const WindowLayout L(src_offsets, hyp_offsets, nwin);
     PCREG_REQUIRE((L.nrows == 0 || src) && (L.nhyp == 0 || (T0_16 && T16)) && ld >= L.nrows, "pcreg_icp_batch_windows: null pointer or bad ld");
     const bool gicp = metric == PCREG_ICP_PLANE_TO_PLANE;
@@ -1274,7 +1321,7 @@ int pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double
             const int64_t h0 = k * per, h1 = std::min(L.nhyp, h0 + per);
             if (h1 <= h0) return;
             rc[k] = guarded([&]() { use_slot(k); icp_windows_host_slice(m->on_slot(k), L, hs, w_src, hnrm, T0_16, h0, h1, *opts, stop, metric, gicp_eps,
-                                                                      T16, rm, n_used, status, idx, rmse_hist, n_iter, converged); });
+                                                                      T16, rm, n_used, status, idx, rmse_hist, n_iter, converged, ex, n_extrap); });
         };
         for (int k = 1; k < nd; ++k) workers.emplace_back(run, k);
         run(0);
@@ -1291,6 +1338,18 @@ int pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double
         }
     }
     return PCREG_OK;
+}
+
+int pcreg_icp_batch_windows(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                            const double* w_src, const void* src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
+                            const double* T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
+                            double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                            int64_t* best, int32_t* n_iter, int32_t* converged) {
+    PCREG_API_BEGIN
+    require_init();
+    check_windows(m, src_offsets, hyp_offsets, nwin, opts, metric, src_nrm, gicp_eps, stop);
+    return icp_windows_host(m, src, is_double, ld, src_offsets, w_src, src_nrm, gicp_eps, hyp_offsets, nwin, T0_16, opts, metric, stop, T16,
+                            rmse, n_used, status, idx, rmse_hist, best, n_iter, converged, nullptr, nullptr);
     PCREG_API_END
 }
 
@@ -1306,6 +1365,52 @@ int pcreg_icp_batch_windows_dev(const pcreg_model* m, const double* d_src, const
     const WindowLayout L(src_offsets, hyp_offsets, nwin);
     icp_windows_run(m, L, d_src, d_w_src, d_src_nrm, d_T0_16, *opts, stop, metric, gicp_eps, d_T16, d_rmse, d_n_used, d_status, d_idx,
                     d_rmse_hist, d_best, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, (cudaStream_t)stream);
+    return PCREG_OK;
+    PCREG_API_END
+}
+
+void pcreg_icp_extrap_default(pcreg_icp_extrap* e) {
+    if (!e) return;
+    e->angle_deg = 10.0; e->vmax_scale = 25.0;
+}
+
+static void check_extrap(const pcreg_icp_extrap* e) {
+    if (!e) return;
+    PCREG_REQUIRE(e->angle_deg > 0.0 && e->angle_deg <= 180.0, "icp extrap: angle_deg must be in (0, 180]");
+    PCREG_REQUIRE(std::isfinite(e->vmax_scale) && e->vmax_scale > 0.0, "icp extrap: vmax_scale must be finite and > 0");
+}
+
+int pcreg_icp_batch_extrap(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                           const double* w_src, const int64_t* hyp_offsets, int64_t nwin, const double* T0_16,
+                           const pcreg_icp_opts* opts, const pcreg_icp_stop* stop, const pcreg_icp_extrap* ex,
+                           double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
+                           int64_t* best, int32_t* n_iter, int32_t* converged, int32_t* n_extrap) {
+    PCREG_API_BEGIN
+    require_init();
+    check_windows(m, src_offsets, hyp_offsets, nwin, opts, PCREG_ICP_POINT_TO_POINT, nullptr, 0.0, stop);
+    check_extrap(ex);
+    const IcpExtrapRule rule = ex ? IcpExtrapRule{ex->angle_deg, ex->vmax_scale} : IcpExtrapRule{};
+    return icp_windows_host(m, src, is_double, ld, src_offsets, w_src, nullptr, 0.0, hyp_offsets, nwin, T0_16, opts, PCREG_ICP_POINT_TO_POINT,
+                            stop, T16, rmse, n_used, status, idx, rmse_hist, best, n_iter, converged, ex ? &rule : nullptr,
+                            ex ? n_extrap : nullptr);
+    PCREG_API_END
+}
+
+int pcreg_icp_batch_extrap_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                               const int64_t* hyp_offsets, int64_t nwin, const double* d_T0_16, const pcreg_icp_opts* opts,
+                               const pcreg_icp_stop* stop, const pcreg_icp_extrap* ex, double* d_T16, double* d_rmse,
+                               int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
+                               int32_t* d_n_iter, int32_t* d_converged, int32_t* d_n_extrap, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    check_windows(m, src_offsets, hyp_offsets, nwin, opts, PCREG_ICP_POINT_TO_POINT, nullptr, 0.0, stop);
+    check_extrap(ex);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    const WindowLayout L(src_offsets, hyp_offsets, nwin);
+    const IcpExtrapRule rule = ex ? IcpExtrapRule{ex->angle_deg, ex->vmax_scale} : IcpExtrapRule{};
+    icp_windows_run(m, L, d_src, d_w_src, nullptr, d_T0_16, *opts, stop, PCREG_ICP_POINT_TO_POINT, 0.0, d_T16, d_rmse, d_n_used, d_status,
+                    d_idx, d_rmse_hist, d_best, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, (cudaStream_t)stream,
+                    ex ? &rule : nullptr, ex ? d_n_extrap : nullptr);
     return PCREG_OK;
     PCREG_API_END
 }

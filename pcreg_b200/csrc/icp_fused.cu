@@ -67,9 +67,20 @@ __device__ __noinline__ int fused_pose_update_stop(const double (&s)[icp_nsums<M
     for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
     return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
 }
+// The same with pose extrapolation between the Kabsch update and the stop rule (point-to-point; ex_state: shared, thread 0's).
+__device__ __noinline__ int fused_pose_update_extrap(const double (&s)[KABSCH_NSUMS], long long n_used, const double* pivot, bool reflection_fix,
+                                                     const IcpStopRule& rule, const IcpExtrapRule& ex, const double* cen, int it,
+                                                     double* ring, double* ex_state, double* Ts) {
+    double Tc[16], Tn[16];
+    for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
+    if (!icp_pose_update(s, n_used, pivot, reflection_fix, Tc, Tn)) return 0;
+    icp_extrap_update(ex, s, pivot, cen, Tc, Tn, it + 1, ex_state);
+    for (int k = 0; k < 16; ++k) Ts[k] = Tn[k];
+    return icp_stop_update(rule, Tc, Tn, it + 1, ring) ? 2 : 1;
+}
 
 // The source rows of a block's hypothesis: rows r0 .. r0 + ns - 1 of the source arrays, its idx_out block at idx_base (windowed calls).
-struct FusedWindow { int64_t r0, idx_base; int ns; };
+struct FusedWindow { int64_t r0, idx_base; int ns, w; };
 template <bool WIN, class Args>
 __device__ __forceinline__ FusedWindow fused_window(const Args& a, int64_t h) {
     if constexpr (WIN) {
@@ -77,20 +88,21 @@ __device__ __forceinline__ FusedWindow fused_window(const Args& a, int64_t h) {
         while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (a.win_hyp[mid] <= h) lo = mid; else hi = mid - 1; }
         const int64_t r0 = a.win_src[lo];
         const int ns = (int)(a.win_src[lo + 1] - r0);
-        return FusedWindow{r0, a.win_idx[lo] + (h - a.win_hyp[lo]) * (int64_t)ns, ns};
+        return FusedWindow{r0, a.win_idx[lo] + (h - a.win_hyp[lo]) * (int64_t)ns, ns, lo};
     } else {
-        return FusedWindow{0, 0, a.ns};
+        return FusedWindow{0, 0, a.ns, 0};
     }
 }
 
 // KNN = the trimmed mode (its selection scratch -- 18 KB of shared memory -- exists only in that instantiation).
 // STOP = the tolerance stop (pcreg_icp_batch_stop): a stop -- by the rule or by a degenerate update -- makes the block's next
-// pass its final scoring pass, after which the block exits.  The STOP = false instantiations are the loop without it.
+// pass its final scoring pass, after which the block exits.  The STOP = 0 instantiations are the loop without it; STOP = 2 (METRIC 0
+// only) adds the pose extrapolation (pcreg_icp_batch_extrap) before the stop rule.
 // METRIC = 0 point-to-point; 1 point-to-plane (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered
 // there; 2 plane-to-plane (pcreg_icp_batch_gicp): the same, and the source normal of each correspondence rotated by the pose.
 // WIN = a windowed call (pcreg_icp_batch_windows, FusedWinArgs): a prologue finds the block's window; from there on the block runs
 // exactly as in a call on that window alone (its rows, ns, perm / tie_order entries and idx_out block).
-template <bool KNN, bool STOP, int METRIC, bool WIN = false>
+template <bool KNN, int STOP, int METRIC, bool WIN = false>
 __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(const __grid_constant__ std::conditional_t<WIN, FusedWinArgs, FusedArgs> a) {
     constexpr int NS = icp_nsums<METRIC>;
     extern __shared__ __align__(16) unsigned char dyn[];
@@ -99,7 +111,8 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     __shared__ HistSelShared hsel;
     __shared__ int s_frozen;
     __shared__ int s_stop;                                  // STOP: the next pass is the final one
-    __shared__ double s_ring[2 * ICP_STOP_WINDOW_MAX];      // STOP: thread 0's window of update motions
+    __shared__ double s_ring[2 * ICP_STOP_WINDOW_MAX + (STOP == 2 ? EXTRAP_STATE : 0)];   // STOP: thread 0's window of update
+                                                                                          // motions; STOP = 2: then its extrapolation state
 
     const FusedWindow W = fused_window<WIN>(a, blockIdx.x);
     const int ns = W.ns;
@@ -119,6 +132,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
 
     if (tid < 16) Ts[tid] = a.T[h * 16 + tid];
     if (tid == 0) { s_frozen = a.frozen[h]; if (STOP) s_stop = 0; }
+    if (STOP == 2 && tid < EXTRAP_STATE) s_ring[2 * ICP_STOP_WINDOW_MAX + tid] = 0.0;
     if (KNN) for (int b = tid; b < SEL_BINS; b += UPD_THREADS) hsel.hist[b] = 0;     // block_hist_finish leaves it zero after
     __syncthreads();
     // trimmed mode: the K-th residual key of the last pass (0: none yet, or nothing selected); the next pass centres its
@@ -246,6 +260,11 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             if (!last && !s_frozen) {
                 if (!STOP) {
                     if (!fused_pose_update<METRIC>(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
+                } else if constexpr (STOP == 2) {
+                    const int r = fused_pose_update_extrap(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, a.ex, a.ex_cen + 3 * W.w, it,
+                                                           s_ring, s_ring + 2 * ICP_STOP_WINDOW_MAX, Ts);
+                    if (r == 0) s_frozen = 1;
+                    if (r != 1) s_stop = 1;
                 } else {
                     const int r = fused_pose_update_stop<METRIC>(s, n_used, a.pivot, a.reflection_fix != 0, a.stop, it, s_ring, Ts);
                     if (r == 0) s_frozen = 1;
@@ -259,6 +278,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
     }
     if (tid < 16) a.T[h * 16 + tid] = Ts[tid];
     if (tid == 0) a.frozen[h] = s_frozen;
+    if (STOP == 2 && tid == 0 && a.n_extrap) a.n_extrap[h] = (int32_t)s_ring[2 * ICP_STOP_WINDOW_MAX + 18];
     if (a.idx_out) {
         int32_t* __restrict__ out = a.idx_out + (WIN ? W.idx_base : h * (int64_t)ns);
         for (int r = tid; r < ns; r += UPD_THREADS) out[a.perm ? a.perm[W.r0 + r] : r] = idx_s[r];
@@ -287,9 +307,11 @@ size_t icp_fused_smem(int64_t ns, int mode) {
 }
 
 template <int METRIC, bool WIN = false>
-static const void* fused_kernel(bool knn, bool stop) {
-    return knn ? (stop ? (const void*)k_icp_fused<true, true, METRIC, WIN> : (const void*)k_icp_fused<true, false, METRIC, WIN>)
-               : (stop ? (const void*)k_icp_fused<false, true, METRIC, WIN> : (const void*)k_icp_fused<false, false, METRIC, WIN>);
+static const void* fused_kernel(bool knn, int stop) {
+    if constexpr (METRIC == ICP_M_POINT)
+        if (stop == 2) return knn ? (const void*)k_icp_fused<true, 2, METRIC, WIN> : (const void*)k_icp_fused<false, 2, METRIC, WIN>;
+    return knn ? (stop ? (const void*)k_icp_fused<true, 1, METRIC, WIN> : (const void*)k_icp_fused<true, 0, METRIC, WIN>)
+               : (stop ? (const void*)k_icp_fused<false, 1, METRIC, WIN> : (const void*)k_icp_fused<false, 0, METRIC, WIN>);
 }
 
 static bool fused_fits(const void* fn, int64_t ns, int mode) {
@@ -298,9 +320,10 @@ static bool fused_fits(const void* fn, int64_t ns, int mode) {
     return icp_fused_smem(ns, mode) + fa.sharedSizeBytes + 1024 <= ctx().smem_optin;
 }
 
-// Point-to-point calls keep the check they always had (the static shared memory of k_icp_fused<true, false, 0>); the other metrics
-// check the instantiation they launch (their reduction buffer is 29 instead of 17 doubles x 32).
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, int metric) {
+// Point-to-point calls without extrapolation keep the check they always had (the static shared memory of k_icp_fused<true, 0, 0>);
+// the others check the instantiation they launch (the other metrics' reduction buffer is 29 instead of 17 doubles x 32, the
+// extrapolation adds its state).
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, int stop, int metric) {
     if (!m->has_vox || o.nn != PCREG_NN_GRID) return false;
     if (const char* e = getenv("PCREG_FUSED")) { if (e[0] == '0') return false; if (e[0] == '1') nhyp = (int64_t)1 << 40; }
     // one block per hypothesis: a batch smaller than the SM count leaves SMs idle, the per-pass kernels (all SMs on every
@@ -308,12 +331,12 @@ bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pc
     if (nhyp < ctx().sm_count) return false;
     if (ns >= ((int64_t)1 << 30)) return false;
     const bool knn = o.mode == PCREG_ICP_KNN;
-    const void* fn = metric == ICP_M_POINT ? (const void*)k_icp_fused<true, false, ICP_M_POINT>
+    const void* fn = metric == ICP_M_POINT ? (stop == 2 ? fused_kernel<ICP_M_POINT>(knn, 2) : (const void*)k_icp_fused<true, 0, ICP_M_POINT>)
                    : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE>(knn, stop) : fused_kernel<ICP_M_GICP>(knn, stop);
     return fused_fits(fn, ns, o.mode);
 }
 
-bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, bool stop, int metric) {
+bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, int stop, int metric) {
     if (!m->has_vox || o.nn != PCREG_NN_GRID || ns_max >= ((int64_t)1 << 30)) return false;
     const bool knn = o.mode == PCREG_ICP_KNN;
     const void* fn = metric == ICP_M_POINT ? fused_kernel<ICP_M_POINT, true>(knn, stop)
@@ -321,23 +344,30 @@ bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp
     return fused_fits(fn, ns_max, o.mode);
 }
 
-template <bool KNN, bool STOP, int METRIC, bool WIN, class Args>
+template <bool KNN, int STOP, int METRIC, bool WIN, class Args>
 static void fused_launch_one(const Args& a, int64_t nhyp, size_t dyn, cudaStream_t st) {
     PCREG_CUDA(cudaFuncSetAttribute(k_icp_fused<KNN, STOP, METRIC, WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
     k_icp_fused<KNN, STOP, METRIC, WIN><<<(unsigned)nhyp, UPD_THREADS, dyn, st>>>(a);
 }
 
 template <int METRIC, bool WIN, class Args>
-static void fused_launch_metric(const Args& a, int64_t nhyp, bool stop, size_t dyn, cudaStream_t st) {
+static void fused_launch_metric(const Args& a, int64_t nhyp, int stop, size_t dyn, cudaStream_t st) {
     const bool knn = a.mode == PCREG_ICP_KNN;
-    if (knn && !stop)       fused_launch_one<true, false, METRIC, WIN>(a, nhyp, dyn, st);
-    else if (!knn && !stop) fused_launch_one<false, false, METRIC, WIN>(a, nhyp, dyn, st);
-    else if (knn)           fused_launch_one<true, true, METRIC, WIN>(a, nhyp, dyn, st);
-    else                    fused_launch_one<false, true, METRIC, WIN>(a, nhyp, dyn, st);
+    if constexpr (METRIC == ICP_M_POINT) {
+        if (stop == 2) {
+            if (knn) fused_launch_one<true, 2, METRIC, WIN>(a, nhyp, dyn, st);
+            else     fused_launch_one<false, 2, METRIC, WIN>(a, nhyp, dyn, st);
+            return;
+        }
+    }
+    if (knn && !stop)       fused_launch_one<true, 0, METRIC, WIN>(a, nhyp, dyn, st);
+    else if (!knn && !stop) fused_launch_one<false, 0, METRIC, WIN>(a, nhyp, dyn, st);
+    else if (knn)           fused_launch_one<true, 1, METRIC, WIN>(a, nhyp, dyn, st);
+    else                    fused_launch_one<false, 1, METRIC, WIN>(a, nhyp, dyn, st);
 }
 
 template <bool WIN, class Args>
-static void fused_launch(const Args& a, int64_t nhyp, bool stop, cudaStream_t st) {
+static void fused_launch(const Args& a, int64_t nhyp, int stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
     if (a.snx)      fused_launch_metric<ICP_M_GICP, WIN>(a, nhyp, stop, dyn, st);
     else if (a.nrm) fused_launch_metric<ICP_M_PLANE, WIN>(a, nhyp, stop, dyn, st);
@@ -345,7 +375,7 @@ static void fused_launch(const Args& a, int64_t nhyp, bool stop, cudaStream_t st
     PCREG_LAUNCHED();
 }
 
-void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st) { fused_launch<false>(a, nhyp, stop, st); }
-void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, bool stop, cudaStream_t st) { fused_launch<true>(a, nhyp, stop, st); }
+void icp_fused_launch(FusedArgs& a, int64_t nhyp, int stop, cudaStream_t st) { fused_launch<false>(a, nhyp, stop, st); }
+void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, int stop, cudaStream_t st) { fused_launch<true>(a, nhyp, stop, st); }
 
 }  // namespace pcreg

@@ -55,6 +55,9 @@ struct FusedArgs {
     const ModelPointD* nrm;                 // model normals (original order): the point-to-plane metric; null: point-to-point
     // plane-to-plane metric (null: the other two): unit source normals in the order of sx / sy / sz, and the covariance epsilon
     const double* snx; const double* sny; const double* snz; double gicp_eps;
+    // pose extrapolation (the k_icp_fused<*, 2, 0> instantiations only): the rule, the source centroid of each window ([nwin][3]; one
+    // window without WIN) and the optional [nhyp] count of extrapolated updates
+    IcpExtrapRule ex; const double* ex_cen; int32_t* n_extrap;
 };
 // Windowed calls (pcreg_icp_batch_windows; the k_icp_fused<*, *, *, true> instantiations): the source arrays, w_src, the source
 // normals, perm and tie_order are the concatenation of nwin windows (column stride of sx / sy / sz: the total row count), and
@@ -66,11 +69,12 @@ struct FusedWinArgs : FusedArgs {
     int32_t nwin;
 };
 size_t icp_fused_smem(int64_t ns, int mode);
-bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, bool stop, int metric);
-void icp_fused_launch(FusedArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
+// stop: 0 no tolerance stop, 1 the stop, 2 the stop with pose extrapolation (point-to-point only)
+bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pcreg_icp_opts& o, int stop, int metric);
+void icp_fused_launch(FusedArgs& a, int64_t nhyp, int stop, cudaStream_t st);
 // windowed calls: the instantiation they launch fits the largest window (ns_max) in shared memory on the model's voxel map
-bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, bool stop, int metric);
-void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, bool stop, cudaStream_t st);
+bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp_opts& o, int stop, int metric);
+void icp_fused_windows_launch(const FusedWinArgs& a, int64_t nhyp, int stop, cudaStream_t st);
 
 __device__ __forceinline__ void flush_counters(unsigned long long* counters, unsigned long long n_pts,
                                                unsigned long long n_cells, unsigned long long n_nodes, int i_pts = 0, int i_cells = 1,

@@ -158,4 +158,11 @@ __device__ __noinline__ static bool icp_stop_update(const IcpStopRule& r, const 
     return st / (double)w < r.tol_t && sr / (double)w < r.tol_r_deg;
 }
 
+// Pose extrapolation (pcreg_icp_extrap, include/pcreg.h; the rule is extrap_step in pcreg_math.cuh).  Update u took Tc = T_{u-1} to
+// Tn = K_u; on return Tn is the pose to write, T_u.  Both ICP paths call this one function, so their poses agree bit for bit.
+__device__ __noinline__ static void icp_extrap_update(const IcpExtrapRule& r, const double* s, const double* pivot, const double* cen,
+                                                      const double* Tc, double* Tn, int u, double* state) {
+    extrap_step(r.angle_deg, r.vmax_scale, s, pivot, cen, Tc, Tn, u, state, nullptr);
+}
+
 }  // namespace pcreg

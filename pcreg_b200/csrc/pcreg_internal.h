@@ -250,6 +250,8 @@ void nn_grid_launch(const pcreg_model* m, const double* d_sx, const double* d_sy
 // Tolerance stop of the ICP loop (pcreg_icp_stop; the rule is icp_stop_update in pcreg_icp.cuh)
 constexpr int ICP_STOP_WINDOW_MAX = 16;
 struct IcpStopRule { double tol_t, tol_r_deg; int window; };
+// Pose extrapolation of the point-to-point loop (pcreg_icp_extrap; the rule is extrap_step in pcreg_math.cuh)
+struct IcpExtrapRule { double angle_deg, vmax_scale; };
 
 // Select / weight / 17 sums / Kabsch / compose, one block per hypothesis.
 struct IcpUpdateArgs {
@@ -278,6 +280,11 @@ struct IcpUpdateArgs {
     const pcreg::ModelPointD* nrm;         // model normals (original order): the point-to-plane metric (k_icp_update<*, *, 1>)
     // plane-to-plane metric (k_icp_update<*, *, 2>; null otherwise): unit source normals in the order of sx / sy / sz, covariance epsilon
     const double* snx; const double* sny; const double* snz; double gicp_eps;
+    // pose extrapolation (ex_state == nullptr: none; else the k_icp_update<*, 2, 0> instantiations, which need stop_iter as well)
+    IcpExtrapRule ex;
+    double* ex_state;           // [nhyp][EXTRAP_STATE], zero before the first pass
+    const double* ex_cen;       // [3] source centroid
+    int32_t* n_extrap;          // [nhyp] optional, written by the final pass
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
 // d_seg (optional, device [nseg + 1]): one arg-min per segment of the rmse array, each relative to its segment

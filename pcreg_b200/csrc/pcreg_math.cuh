@@ -327,6 +327,158 @@ PCREG_HD void gicp_accumulate(double* s, double w, double d, const double* qt, c
     s[28] += w * d;
 }
 
+// ---- pose extrapolation of the point-to-point ICP (include/pcreg.h: pcreg_icp_extrap; Besl & McKay 1992, section IV) ----
+// Poses are row-vector 4x4 (rotation block R(r, c) = T[r * 4 + c], translation row T[12..14]).  A pose's state is
+// x(T) = (qR, qT) in R^7: qR = (w, x, y, z) the unit quaternion of R, qT = c R + t the image of the source centroid c.
+
+// Shepperd's conversion: the largest of (trace, R00, R11, R22) picks the component computed from a square root.
+PCREG_HD void rot_to_quat(const double* T, double* q) {
+    const double r00 = T[0], r01 = T[1], r02 = T[2], r10 = T[4], r11 = T[5], r12 = T[6], r20 = T[8], r21 = T[9], r22 = T[10];
+    const double tr = r00 + r11 + r22;
+    if (tr >= r00 && tr >= r11 && tr >= r22) {
+        const double w = 0.5 * sqrt(1.0 + tr), f = 0.25 / w;
+        q[0] = w; q[1] = (r21 - r12) * f; q[2] = (r02 - r20) * f; q[3] = (r10 - r01) * f;
+    } else if (r00 >= r11 && r00 >= r22) {
+        const double x = 0.5 * sqrt(1.0 + r00 - r11 - r22), f = 0.25 / x;
+        q[0] = (r21 - r12) * f; q[1] = x; q[2] = (r01 + r10) * f; q[3] = (r02 + r20) * f;
+    } else if (r11 >= r22) {
+        const double y = 0.5 * sqrt(1.0 - r00 + r11 - r22), f = 0.25 / y;
+        q[0] = (r02 - r20) * f; q[1] = (r01 + r10) * f; q[2] = y; q[3] = (r12 + r21) * f;
+    } else {
+        const double z = 0.5 * sqrt(1.0 - r00 - r11 + r22), f = 0.25 / z;
+        q[0] = (r10 - r01) * f; q[1] = (r02 + r20) * f; q[2] = (r12 + r21) * f; q[3] = z;
+    }
+}
+
+// The rotation block of T from a unit quaternion (the inverse of rot_to_quat); the other entries of T are left alone.
+PCREG_HD void quat_to_rot(const double* q, double* T) {
+    const double w = q[0], x = q[1], y = q[2], z = q[3];
+    T[0] = 1.0 - 2.0 * (y * y + z * z); T[1] = 2.0 * (x * y - z * w);       T[2] = 2.0 * (x * z + y * w);
+    T[4] = 2.0 * (x * y + z * w);       T[5] = 1.0 - 2.0 * (x * x + z * z); T[6] = 2.0 * (y * z - x * w);
+    T[8] = 2.0 * (x * z - y * w);       T[9] = 2.0 * (y * z + x * w);       T[10] = 1.0 - 2.0 * (x * x + y * y);
+}
+
+// x(T) for source centroid c.  Sign of qR: with qprev (a previous state's quaternion) the one with qR . qprev >= 0; without, w >= 0
+// and, at w = 0, the first nonzero component positive.
+PCREG_HD void pose_state(const double* T, const double* c, const double* qprev, double* x) {
+    rot_to_quat(T, x);
+    bool flip;
+    if (qprev) {
+        flip = x[0] * qprev[0] + x[1] * qprev[1] + x[2] * qprev[2] + x[3] * qprev[3] < 0.0;
+    } else {
+        int k = 0;
+        while (k < 3 && x[k] == 0.0) ++k;
+        flip = x[k] < 0.0;
+    }
+    if (flip) for (int k = 0; k < 4; ++k) x[k] = -x[k];
+    for (int b = 0; b < 3; ++b) x[4 + b] = c[0] * T[0 * 4 + b] + c[1] * T[1 * 4 + b] + c[2] * T[2 * 4 + b] + T[12 + b];
+}
+
+// Weighted mean-square error sum w |m - quickTF(s, T)|^2 / sum w of the correspondences behind the 17 sums s (taken at pose Tc,
+// relative to pivot p) at another pose T.  With E = Tc^-1 T = [RE 0; tE 1] a source point moves from q to q RE + tE; with centred
+// q^ = q - p - cq, m^ = m - p - cm (cq, cm the weighted centroids relative to p) and H = sum w q^ m^' the centred cross-covariance:
+//   sum w |e|^2 = (s16 - sw |cm - cq|^2) + 2 sum_ab (I - RE)_ab H_ab + sw |cm - cq RE - tau|^2,  tau = (tE + p RE) - p
+//               = (t - p) - (tc - p) RE.
+// Every term is small where the result is small, so a cloud far from the pivot loses no accuracy to cancellation.
+PCREG_HD double sums_mse_at(const double* s, const double* p, const double* Tc, const double* T) {
+    const double sw = s[0], inv = 1.0 / sw;
+    double cq[3], cm[3], RE[9];
+    for (int a = 0; a < 3; ++a) { cq[a] = s[1 + a] * inv; cm[a] = s[4 + a] * inv; }
+    for (int a = 0; a < 3; ++a)
+        for (int b = 0; b < 3; ++b) RE[a * 3 + b] = Tc[0 * 4 + a] * T[0 * 4 + b] + Tc[1 * 4 + a] * T[1 * 4 + b] + Tc[2 * 4 + a] * T[2 * 4 + b];
+    double e0 = 0.0, rot = 0.0, dl = 0.0;
+    for (int a = 0; a < 3; ++a) e0 += (cm[a] - cq[a]) * (cm[a] - cq[a]);
+    for (int a = 0; a < 3; ++a)
+        for (int b = 0; b < 3; ++b) {
+            const double H = s[7 + a * 3 + b] - s[1 + a] * cm[b];
+            rot += ((a == b ? 1.0 : 0.0) - RE[a * 3 + b]) * H;
+        }
+    for (int b = 0; b < 3; ++b) {
+        double tau = T[12 + b] - p[b], cqR = 0.0;
+        for (int a = 0; a < 3; ++a) { tau -= (Tc[12 + a] - p[a]) * RE[a * 3 + b]; cqR += cq[a] * RE[a * 3 + b]; }
+        const double r = cm[b] - cqR - tau;
+        dl += r * r;
+    }
+    return ((s[16] - sw * e0) + 2.0 * rot + sw * dl) * inv;
+}
+
+// Zero of the least-squares line through (v_i, D_i), i = 0..2 (NaN or infinite when the line is flat).
+PCREG_HD double extrap_line_zero(const double* v, const double* D) {
+    const double vm = (v[0] + v[1] + v[2]) / 3.0, Dm = (D[0] + D[1] + D[2]) / 3.0;
+    double sxy = 0.0, sxx = 0.0;
+    for (int i = 0; i < 3; ++i) { sxy += (v[i] - vm) * (D[i] - Dm); sxx += (v[i] - vm) * (v[i] - vm); }
+    return vm - Dm / (sxy / sxx);
+}
+
+// Vertex -b / (2a) of the parabola a v^2 + b v + c through the three points (Newton's divided differences).
+PCREG_HD double extrap_parabola_vertex(const double* v, const double* D) {
+    const double f01 = (D[1] - D[0]) / (v[1] - v[0]), f12 = (D[2] - D[1]) / (v[2] - v[1]);
+    const double a = (f12 - f01) / (v[2] - v[0]);
+    const double b = f01 - a * (v[0] + v[1]);
+    return -b / (2.0 * a);
+}
+
+// The step along the update direction (Besl & McKay's choice between the line zero v1, the parabola vertex v2 and the cap vmax).
+// Strict compares; NaN fails each.  Returns the branch: 1 = v2, 2 = v1, 3 = vmax, 0 = no step (*dv = 0).
+PCREG_HD int extrap_branch(double v1, double v2, double vmax, double* dv) {
+    if ((0.0 < v2 && v2 < v1 && v1 < vmax) || (0.0 < v2 && v2 < vmax && vmax < v1)) { *dv = v2; return 1; }
+    if ((0.0 < v1 && v1 < v2 && v2 < vmax) || (0.0 < v1 && v1 < vmax && vmax < v2) || (v2 < 0.0 && 0.0 < v1 && v1 < vmax)) { *dv = v1; return 2; }
+    if (v1 > vmax && v2 > vmax) { *dv = vmax; return 3; }
+    *dv = 0.0;
+    return 0;
+}
+
+// Per-hypothesis state of the extrapolation: x_{u-1} [0..6], Delta_{u-1} [7..13], n_{u-1} [14], theta_{u-1} [15] (NaN: undefined),
+// d_{u-1} [16], d_{u-2} [17], updates extrapolated so far [18].  All zero before the first update.
+constexpr int EXTRAP_STATE = 20;
+constexpr int EXTRAP_NTRACE = 5;       // theta_u, v1, v2, dv, branch of one update (host tests)
+
+// Update u >= 1 (not degenerate) of one hypothesis: Tc = T_{u-1}, Tn = K_u = T_{u-1} dT on entry, T_u on return; s = the update's
+// 17 sums (relative to pivot p), c = the source centroid.  Returns the branch (0: T_u = K_u).
+PCREG_HD int extrap_step(double angle_deg, double vmax_scale, const double* s, const double* p, const double* c, const double* Tc,
+                         double* Tn, int u, double* st, double* trace) {
+    const double nan_v = NAN;
+    if (u == 1) {
+        pose_state(Tc, c, nullptr, st);
+        for (int k = 7; k < 18; ++k) st[k] = nan_v;
+    }
+    double xk[7], dl[7], n2 = 0.0;
+    pose_state(Tn, c, st, xk);
+    for (int k = 0; k < 7; ++k) { dl[k] = xk[k] - st[k]; n2 += dl[k] * dl[k]; }
+    const double n = sqrt(n2), np = st[14];
+    double th = nan_v;
+    if (u >= 2 && n > 0.0 && np > 0.0) {
+        double dot = 0.0;
+        for (int k = 0; k < 7; ++k) dot += dl[k] * st[7 + k];
+        const double cs = fmin(fmax(dot / (n * np), -1.0), 1.0);
+        th = acos(cs) * (180.0 / 3.14159265358979323846);
+    }
+    const double dK = sums_mse_at(s, p, Tc, Tn);
+    double v1 = nan_v, v2 = nan_v, dv = 0.0;
+    int br = 0;
+    if (u >= 3 && th < angle_deg && st[15] < angle_deg) {
+        const double v[3] = {0.0, -n, -n - np}, D[3] = {dK, st[16], st[17]};
+        v1 = extrap_line_zero(v, D);
+        v2 = extrap_parabola_vertex(v, D);
+        br = extrap_branch(v1, v2, vmax_scale * n, &dv);
+    }
+    double dU = dK;
+    if (dv > 0.0) {
+        const double f = dv / n;
+        for (int k = 0; k < 7; ++k) xk[k] += f * dl[k];
+        const double qn = sqrt(xk[0] * xk[0] + xk[1] * xk[1] + xk[2] * xk[2] + xk[3] * xk[3]);
+        for (int k = 0; k < 4; ++k) xk[k] /= qn;
+        quat_to_rot(xk, Tn);
+        for (int b = 0; b < 3; ++b) Tn[12 + b] = xk[4 + b] - (c[0] * Tn[0 * 4 + b] + c[1] * Tn[1 * 4 + b] + c[2] * Tn[2 * 4 + b]);
+        dU = sums_mse_at(s, p, Tc, Tn);
+        st[18] += 1.0;
+    }
+    for (int k = 0; k < 7; ++k) { st[k] = xk[k]; st[7 + k] = dl[k]; }
+    st[14] = n; st[15] = th; st[17] = st[16]; st[16] = dU;
+    if (trace) { trace[0] = th; trace[1] = v1; trace[2] = v2; trace[3] = dv; trace[4] = (double)br; }
+    return br;
+}
+
 // MATLAB eps(x) for x >= 0: spacing of doubles at x.
 PCREG_HD double spacing(double x) {
     if (!(x > 0.0)) return 4.9406564584124654e-324;
