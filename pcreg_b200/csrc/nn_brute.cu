@@ -17,7 +17,8 @@
 //                on the original coordinates, and competes on (d2, original index).  E bounds the FP32
 //                error of d' against the true FP64 distance (derivation in DESIGN.md), so the true
 //                nearest neighbour -- and every exact tie of it -- is always inside the band: the
-//                returned index and d2 are the FP64 brute-force answers, bit for bit.
+//                returned index and d2 are the FP64 brute-force answers, bit for bit.  A query so far away
+//                that d' or E could overflow (2E > BRUTE_MAX_TWO_E) gets an infinite band: all points in FP64.
 //   bound        the band needs a good initial "best so far": the previous ICP iteration's
 //                correspondence when there is one, else a pure-min pass over a 1/8 sub-sample (the
 //                scan order is a random permutation, so the head of the array is a random sample).
@@ -41,6 +42,10 @@ namespace pcreg {
 constexpr int BRUTE_THREADS = 256;
 constexpr int BRUTE_G = 16;                 // group size of the fast path
 constexpr float BRUTE_ERR_COEF = 7.2e-7f;   // 12 * 2^-24: E = coef * (|q32| + max|m32|)^2
+// Largest band 2E a query may have.  Above it (a query some 1e18 model radii away, or beyond the float range) the scan
+// values |d'| <= 2 (|q32| + max|m32|)^2 could overflow, and with them the band: such a query scans with q32 = 0 and an
+// infinite band instead, so every model point is decided in FP64 (brute_prologue).
+constexpr float BRUTE_MAX_TWO_E = 1.0e30f;
 
 __device__ __forceinline__ float fmin3(float a, float b, float c) {
     float d;
@@ -71,6 +76,16 @@ __device__ __forceinline__ float brute_two_e(float ax, float ay, float az, float
     return __fmul_ru(__fmul_ru(2.02f * BRUTE_ERR_COEF, s), s);
 }
 
+// Scan coefficients (ax,ay,az) = -2 q32 of one query and its band 2E; a query whose band exceeds BRUTE_MAX_TWO_E gets zero
+// coefficients and an infinite band (its scan values are then |m|^2, finite, and every point lies inside the band).
+__device__ __forceinline__ float brute_prologue(double qx, double qy, double qz, const BruteArgs& a, float& ax, float& ay, float& az) {
+    ax = -2.f * __double2float_rn(qx - a.px); ay = -2.f * __double2float_rn(qy - a.py); az = -2.f * __double2float_rn(qz - a.pz);
+    const float twoE = brute_two_e(ax, ay, az, a.max_norm);
+    if (twoE <= BRUTE_MAX_TWO_E) return twoE;
+    ax = ay = az = 0.f;
+    return INFINITY;
+}
+
 // Re-scan one group for one query; exact FP64 evaluation of everything inside the band.  The exact
 // running winner (d2, original index) lives in the kernel's output arrays (global memory): the slow path is
 // rare, and keeping that state out of registers leaves the hot loop with 4 registers per query.
@@ -80,7 +95,7 @@ __device__ __noinline__ float nn_slow(const float4* __restrict__ grp, int64_t jb
     const int64_t h = g / a.ns, i = g - h * a.ns;
     double qx, qy, qz;
     quick_tf(a.T + h * 16, a.sx[i], a.sy[i], a.sz[i], qx, qy, qz);
-    const float twoE = brute_two_e(ax, ay, az, a.max_norm);
+    const float twoE = thr == INFINITY ? INFINITY : brute_two_e(ax, ay, az, a.max_norm);     // INFINITY: see brute_prologue
     double best64 = a.pd2[o];
     int32_t bidx = a.pidx[o];
 #pragma unroll 1
@@ -151,8 +166,7 @@ __global__ void __launch_bounds__(BRUTE_THREADS, 2) k_nn_brute(const __grid_cons
             const int64_t h = g / a.ns, i = g - h * a.ns;
             double qx, qy, qz;
             quick_tf(a.T + h * 16, a.sx[i], a.sy[i], a.sz[i], qx, qy, qz);
-            const float fx = __double2float_rn(qx - a.px), fy = __double2float_rn(qy - a.py), fz = __double2float_rn(qz - a.pz);
-            ax[k] = -2.f * fx; ay[k] = -2.f * fy; az[k] = -2.f * fz;
+            const float twoE = brute_prologue(qx, qy, qz, a, ax[k], ay[k], az[k]);
             if (!PURE_MIN) {
                 const int64_t o = (int64_t)blockIdx.y * a.nq + g;
                 a.pd2[o] = INFINITY;
@@ -172,7 +186,7 @@ __global__ void __launch_bounds__(BRUTE_THREADS, 2) k_nn_brute(const __grid_cons
                 } else if (a.bound_in) {
                     for (int b = 0; b < a.nbound; ++b) bound = fminf(bound, a.bound_in[(int64_t)b * a.nq + g]);
                 }
-                thr[k] = (bound < FLT_MAX) ? __fadd_ru(bound, brute_two_e(ax[k], ay[k], az[k], a.max_norm)) : FLT_MAX;
+                thr[k] = twoE == INFINITY ? INFINITY : (bound < FLT_MAX) ? __fadd_ru(bound, twoE) : FLT_MAX;
             }
         }
     }

@@ -130,16 +130,18 @@ __device__ __forceinline__ float box_lb(float qx, float qy, float qz, int x, int
     const float dx = axis_lb(qx, (float)x * edge, edge), dy = axis_lb(qy, (float)y * edge, edge), dz = axis_lb(qz, (float)z * edge, edge);
     return (dx * dx + dy * dy + dz * dz) * (1.f - 6e-7f);
 }
-// guaranteed upper bound of best (squared distance) in squared cell units, as a float
+// guaranteed upper bound of best (squared distance) in squared cell units, as a float.  Beyond the float range it is
+// +infinity, not FLT_MAX: the box bounds of a query some 1e19 cells away overflow to +infinity as well, and a finite bound
+// would prune every box -- the query would end without an answer.  With +infinity nothing is pruned (every box is visited).
 __device__ __forceinline__ float best_ub_cells(double best, double inv_cell2) {
     const double b = best * inv_cell2;
-    return (b < 3.0e38) ? __double2float_ru(b) * (1.f + 6e-7f) : FLT_MAX;
+    return (b < 3.0e38) ? __double2float_ru(b) * (1.f + 6e-7f) : INFINITY;
 }
 // same for the ball of radius (sqrt(best) + gap): everything inside it gets visited
 __device__ __forceinline__ float best_ub_cells_gap(double best, double inv_cell, float gap_cells) {
     const double r = sqrt(best) * inv_cell + (double)gap_cells;
     const double b = r * r;
-    return (b < 3.0e38) ? __double2float_ru(b) * (1.f + 6e-7f) : FLT_MAX;
+    return (b < 3.0e38) ? __double2float_ru(b) * (1.f + 6e-7f) : INFINITY;
 }
 
 struct Query {
