@@ -255,8 +255,17 @@ typedef struct {
     double R_w;             /* WEIGHTED: w = max(R_w - r, 0)                           */
     double thDist2;         /* > 0: reject correspondences with d^2 >= thDist2         */
     int    nn;              /* PCREG_NN_BRUTE / PCREG_NN_GRID                          */
-    int    reflection_fix;  /* 0 = reference                                           */
+    int    reflection_fix;  /* 0 = reference; see the rank rule below                  */
 } pcreg_icp_opts;
+/* Rank rule of the ICP update (the project's own: the reference has no ICP).  The update fits a rotation to the cross-covariance H
+ * of its correspondences (singular values S[0] >= S[1] >= S[2]).  When H is numerically of rank <= 2 -- S[2] <= tau S[0], or
+ * S[0] <= tau |sum w q~ m~'|_F (H is rounding noise: coincident correspondences) -- the rotation and the reflection fit them
+ * equally well (a flat region of the model, a ridge, a collinear source), and the update takes the PROPER solution whatever
+ * reflection_fix says.  Above that, reflection_fix = 0 reproduces R = V*U', reflections included (a patch mirrored in its tangent
+ * plane), and 1 always returns a rotation.  tau = 1e-8: the one-pass pivot-relative sums leave S[2] / S[0] of an exactly planar set
+ * at up to ~4e-15 (D / L)^2 for a patch of size L at distance D >= L from the model's pivot (4e-11 at D = 100 L), and a curved patch
+ * has S[2] / S[0] ~ (sag / L)^2, so only a patch flatter than a relative sag of 1e-4 counts as planar.  estimateTransform and
+ * RANSAC do not apply the rule. */
 void pcreg_icp_opts_default(pcreg_icp_opts* o);
 /* src: ns x 3 column-major; w_src[ns] optional; T0_16 [nhyp][16] initial poses.  Outputs (any
  * may be NULL except T16): T16 [nhyp][16], rmse [nhyp], n_used [nhyp], status [nhyp] (0 ok,
@@ -454,6 +463,9 @@ int  pcreg_icp_batch_windows_dev(const pcreg_model* m, const double* d_src, cons
  *   0 < v1 < vmax < v2 or (v2 < 0 and 0 < v1 < vmax); vmax if v1 > vmax and v2 > vmax; else 0 (strict compares, NaN fails each).
  *   With dv > 0: x' = x(K_u) + dv Delta_u / n_u, qR' renormalised, T_u = [R(qR') 0; qT' - c R' 1]; otherwise T_u = K_u.
  *   Stored: x_u = x' or x(K_u), d_u = d(T_u), Delta_u and n_u as before the jump; n_extrap counts the updates with dv > 0.
+ *   An update whose K_u or T_{u-1} is improper (reflection_fix = 0 on data that prefer a reflection) has no quaternion state: it is
+ *   not extrapolated (T_u = K_u, nothing stored) and the history restarts: the next update whose K_u and T_{u-1} are both proper
+ *   takes T_{u-1} as update 1 takes T_0 (canonical sign, no direction yet).  So a returned pose has the handedness of its Kabsch pose.
  * Correspondences, rejection, trimming, weights, rmse, the degenerate freeze and the winner are unchanged.  The tolerance stop
  * measures the motion from T_{u-1} to the pose written, T_u.  The rule is causal: a hypothesis stopped after k updates returns exactly
  * what the same call with iters = k returns.  Defaults {10, 25} are the paper's; angle_deg outside (0, 180] or a vmax_scale that is not

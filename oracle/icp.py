@@ -8,7 +8,8 @@ BASELINE.json's north_star describes:
   trimming (KNN)  keep round(k_frac*n) smallest residuals, stable sort  (AlignPoints_KNN.m:20-26)
   weights         w = max(R_w - r, 0)                                    (AlignPoints_weighted.m:16-18)
   rigid fit       estimateTransform.m:41-71 arranged as estimateTransform(pts1=model_j, pts2=q),
-                  weighted centroids + weighted cross-covariance, R = V*U' (no det fix by default)
+                  weighted centroids + weighted cross-covariance, R = V*U' (no det fix by default); the
+                  project's own rule: an H of numerical rank <= 2 gives the proper solution (RANK2_TAU)
   compose         T <- T * dT  (row-vector convention)
   winner          first-index arg-min of rmse (ransac.m:69-73 max() tie rule, mirrored)
 FP64 throughout.
@@ -47,15 +48,23 @@ def _weights(d2, mode, k_frac, R_w, thDist2, w_src):
     return w, int(np.sum(w > 0))
 
 
+RANK2_TAU = 1e-8       # include/pcreg.h: pcreg_icp_opts.reflection_fix (pcreg_math.cuh: ICP_RANK2_TAU)
+
+
 def _weighted_kabsch(m_pts, q_pts, w, reflection_fix):
-    """estimateTransform(pts1=m_pts, pts2=q_pts) with weights: returns dT with [q,1]*dT ~ [m,1]."""
+    """estimateTransform(pts1=m_pts, pts2=q_pts) with weights: returns dT with [q,1]*dT ~ [m,1].
+
+    The ICP update's rank rule: with S[2] <= RANK2_TAU * S[0], or S[0] <= RANK2_TAU * |sum w q m'|_F (H numerically of rank <= 2,
+    or rounding noise; the rotation and the reflection then fit equally well) the update is the proper solution whatever
+    reflection_fix says."""
     sw = w.sum()
     cd = (w[:, None] * m_pts).sum(axis=0) / sw     # estimateTransform.m:46 (d = pts1 = model side)
     cm = (w[:, None] * q_pts).sum(axis=0) / sw     # :47 (m = pts2 = query side)
     H = ((q_pts - cm) * w[:, None]).T @ (m_pts - cd)   # :58  H = m_c * d_c'
-    U, _, Vt = np.linalg.svd(H)                    # :60
+    U, S, Vt = np.linalg.svd(H)                    # :60
     V = Vt.T
-    if reflection_fix and np.linalg.det(V @ U.T) < 0:
+    rank2 = S[2] <= RANK2_TAU * S[0] or S[0] <= RANK2_TAU * np.linalg.norm((w[:, None] * q_pts).T @ m_pts)
+    if (reflection_fix or rank2) and np.linalg.det(V @ U.T) < 0:
         V = V.copy()
         V[:, 2] = -V[:, 2]
     R = V @ U.T                                    # :62

@@ -37,7 +37,8 @@ __device__ __forceinline__ void icp_accumulate(double (&s)[KABSCH_NSUMS], double
     s[16] += w * d;
 }
 
-// Thread 0 of a hypothesis after the block reduction: rigid fit from the sums and T <- T * dT.  Returns false (pose left
+// Thread 0 of a hypothesis after the block reduction: rigid fit from the sums (with the ICP rank rule of kabsch_from_sums) and
+// T <- T * dT.  Returns false (pose left
 // alone, hypothesis to be frozen) with fewer than 3 usable correspondences.  Tc: current pose (row-major), Tn: new pose.
 __device__ __forceinline__ bool icp_pose_update(const double (&s)[KABSCH_NSUMS], long long n_used, const double* pivot, bool reflection_fix,
                                                 const double* Tc, double* Tn) {
@@ -49,7 +50,7 @@ __device__ __forceinline__ bool icp_pose_update(const double (&s)[KABSCH_NSUMS],
     for (int k = 0; k < 9; ++k) ks.sqm[k] = s[7 + k];
     ks.swd2 = s[16];
     double dT[16];
-    kabsch_from_sums(ks, pivot, pivot, reflection_fix, dT);
+    kabsch_from_sums(ks, pivot, pivot, reflection_fix, dT, true);      // rank <= 2: the proper solution (ICP_RANK2_TAU)
     mul4(Tc, dT, Tn);
     return true;
 }

@@ -198,22 +198,38 @@ struct KabschSums {
 };
 constexpr int KABSCH_NSUMS = 17;
 
+// ICP updates (include/pcreg.h: pcreg_icp_opts.reflection_fix): the cross-covariance H is taken as of numerical rank <= 2 when
+// S[2] <= ICP_RANK2_TAU * S[0], or when it is rounding noise (S[0] <= ICP_RANK2_TAU * |sum w q~ m~'|_F, the uncentred sum it was
+// cancelled from: coincident correspondences); the update is then the proper solution whatever reflection_fix says.  There the
+// rotation and the reflection fit the correspondences equally well and the sign of det(V U') is set by how svd3 completes the null
+// direction, not by the data.  The bound: the one-pass pivot-relative sums leave S[2] / S[0] of an exactly planar set at up to
+// about 4e-15 (D / L)^2 (200 correspondences on a patch of size L at distance D >= L from the pivot; 4e-11 at D = 100 L,
+// tests/test_icp_degenerate_cpu.py), so tau keeps a factor 8 of margin up to D = 500 L, while a curved patch has
+// S[2] / S[0] ~ (sag / L)^2, 1e-8 only at a relative sag of 1e-4.
+constexpr double ICP_RANK2_TAU = 1e-8;
+
 // dT (row-major, row-vector convention) with [q,1]*dT ~ [m,1]  (estimateTransform(pts1 = m, pts2 = q)).
-// pivot_q / pivot_m: what was subtracted from the q side / the m side before summing.
-PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const double* pivot_m, bool reflection_fix, double* dT) {
+// pivot_q / pivot_m: what was subtracted from the q side / the m side before summing.  icp_rule: the ICP update's rank rule
+// (ICP_RANK2_TAU); estimateTransform / RANSAC pass false and keep R = V*U' (with reflection_fix alone deciding the flip).
+PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const double* pivot_m, bool reflection_fix, double* dT,
+                               bool icp_rule = false) {
     const double inv = 1.0 / s.sw;
     double cq[3], cm[3], H[9];
     for (int a = 0; a < 3; ++a) { cq[a] = s.sq[a] * inv; cm[a] = s.sm[a] * inv; }
     for (int a = 0; a < 3; ++a)
         for (int b = 0; b < 3; ++b) H[a * 3 + b] = s.sqm[a * 3 + b] - s.sq[a] * cm[b];   // estimateTransform.m:58
+    double f2 = 0.0;                                                                       // |sum w q~ m~'|_F^2 (ICP rank rule)
+    if (icp_rule)
+        for (int k = 0; k < 9; ++k) f2 += s.sqm[k] * s.sqm[k];
     double U[9], S[3], V[9];
     svd3(H, U, S, V);                                                                      // :60
+    const bool fix = reflection_fix || (icp_rule && (S[2] <= ICP_RANK2_TAU * S[0] || S[0] <= ICP_RANK2_TAU * sqrt(f2)));
     double R[9];
     for (int pass = 0; pass < 2; ++pass) {
         for (int r = 0; r < 3; ++r)
             for (int c = 0; c < 3; ++c)                                                   // R = V * U'  (:62)
                 R[r * 3 + c] = V[r * 3 + 0] * U[c * 3 + 0] + V[r * 3 + 1] * U[c * 3 + 1] + V[r * 3 + 2] * U[c * 3 + 2];
-        if (pass == 1 || !reflection_fix || det3(R) >= 0.0) break;
+        if (pass == 1 || !fix || det3(R) >= 0.0) break;
         for (int i = 0; i < 3; ++i) V[i * 3 + 2] = -V[i * 3 + 2];                        // flip the weakest direction
     }
     // t = cd - R*cm (:63) with cd = model centroid, cm = query centroid, pivot restored
@@ -429,18 +445,33 @@ PCREG_HD int extrap_branch(double v1, double v2, double vmax, double* dv) {
 }
 
 // Per-hypothesis state of the extrapolation: x_{u-1} [0..6], Delta_{u-1} [7..13], n_{u-1} [14], theta_{u-1} [15] (NaN: undefined),
-// d_{u-1} [16], d_{u-2} [17], updates extrapolated so far [18].  All zero before the first update.
+// d_{u-1} [16], d_{u-2} [17], updates extrapolated so far [18], 1 when the history restarts at the next update [19].  All zero
+// before the first update.
 constexpr int EXTRAP_STATE = 20;
 constexpr int EXTRAP_NTRACE = 5;       // theta_u, v1, v2, dv, branch of one update (host tests)
 
+// det of the rotation block of a row-major 4x4 pose
+PCREG_HD double det_rot4(const double* T) {
+    return T[0] * (T[5] * T[10] - T[6] * T[9]) - T[1] * (T[4] * T[10] - T[6] * T[8]) + T[2] * (T[4] * T[9] - T[5] * T[8]);
+}
+
 // Update u >= 1 (not degenerate) of one hypothesis: Tc = T_{u-1}, Tn = K_u = T_{u-1} dT on entry, T_u on return; s = the update's
 // 17 sums (relative to pivot p), c = the source centroid.  Returns the branch (0: T_u = K_u).
+// An improper K_u or T_{u-1} (reflection_fix = 0 reproducing R = V*U') has no quaternion state: that update is not extrapolated
+// (T_u = K_u) and the history restarts at the next update, which takes its T_{u-1} as update 1 takes T_0.  So every returned pose
+// has the handedness of its Kabsch pose.
 PCREG_HD int extrap_step(double angle_deg, double vmax_scale, const double* s, const double* p, const double* c, const double* Tc,
                          double* Tn, int u, double* st, double* trace) {
     const double nan_v = NAN;
-    if (u == 1) {
+    if (!(det_rot4(Tc) > 0.0 && det_rot4(Tn) > 0.0)) {
+        st[19] = 1.0;
+        if (trace) { trace[0] = nan_v; trace[1] = nan_v; trace[2] = nan_v; trace[3] = 0.0; trace[4] = 0.0; }
+        return 0;
+    }
+    if (u == 1 || st[19] != 0.0) {
         pose_state(Tc, c, nullptr, st);
         for (int k = 7; k < 18; ++k) st[k] = nan_v;
+        st[19] = 0.0;
     }
     double xk[7], dl[7], n2 = 0.0;
     pose_state(Tn, c, st, xk);

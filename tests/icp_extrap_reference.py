@@ -8,6 +8,8 @@ error d(T) is evaluated point by point, and the two fits are numpy.polyfit.  Par
   between Delta_{u-1} and Delta_u in degrees.  With u >= 3 and theta_u, theta_{u-1} < angle_deg: v = (0, -n_u, -n_u - n_{u-1}),
   D = (d(K_u), d_{u-1}, d_{u-2}); v1 = zero of the least-squares line, v2 = vertex of the parabola, vmax = vmax_scale n_u; the
   branch table picks dv; with dv > 0 the pose is built from x(K_u) + dv Delta_u / n_u (quaternion renormalised).
+  An update whose K_u or T_{u-1} is improper (reflection_fix = 0 on data that prefer a reflection) is not extrapolated (T_u = K_u)
+  and the history restarts: the next update with both poses proper takes its T_{u-1} as update 1 takes T_0.
 """
 from __future__ import annotations
 
@@ -87,7 +89,7 @@ def icp_single_extrap(model, src, T0, angle_deg=10.0, vmax_scale=25.0, extrapola
         iters = len(replay) - 1
     status, n_iter, converged, n_extrap = 0, iters, 0, 0
     hist, motion, trace = [], [], []
-    x_prev = pose_state(T, c)
+    x_prev, restart = None, True
     dl_prev, n_prev, th_prev, d_prev, d_prev2 = None, math.nan, math.nan, math.nan, math.nan
     for it in range(iters):
         if replay is not None:
@@ -106,7 +108,15 @@ def icp_single_extrap(model, src, T0, angle_deg=10.0, vmax_scale=25.0, extrapola
         K = T @ _weighted_kabsch(mj, q, w, reflection_fix)
         mse = lambda P: float((w * ((mj - quickTF(src, P)) ** 2).sum(axis=1)).sum() / sw)  # noqa: E731
         Tn = K
-        if extrapolate:
+        if extrapolate and not (np.linalg.det(T[:3, :3]) > 0 and np.linalg.det(K[:3, :3]) > 0):
+            restart = True
+            trace.append(dict(u=u, theta=math.nan, v1=math.nan, v2=math.nan, vmax=math.nan, dv=0.0, branch=BRANCH_NONE, margin=math.inf,
+                              T=Tn, skipped=True))
+        elif extrapolate:
+            if restart:
+                x_prev = pose_state(T, c)
+                dl_prev, n_prev, th_prev, d_prev, d_prev2 = None, math.nan, math.nan, math.nan, math.nan
+                restart = False
             xk = pose_state(K, c, x_prev[:4])
             dl = xk - x_prev
             n = float(np.linalg.norm(dl))
@@ -125,7 +135,7 @@ def icp_single_extrap(model, src, T0, angle_deg=10.0, vmax_scale=25.0, extrapola
                 a2, b2, _ = np.polyfit(v, D, 2)
                 v2 = -b2 / (2 * a2) if a2 != 0 else math.nan
                 dv, br = branch(v1, v2, vmax)
-            trace.append(dict(u=u, theta=th, v1=v1, v2=v2, vmax=vmax, dv=dv, branch=br,
+            trace.append(dict(u=u, theta=th, v1=v1, v2=v2, vmax=vmax, dv=dv, branch=br, skipped=False,
                               margin=decision_margin(th, th_prev, angle_deg, v1, v2, vmax) if u >= 3 else math.inf))
             if dv > 0:
                 xn = xk + dv * dl / n

@@ -1,7 +1,7 @@
 """FP64 reference of the ICP tolerance stop (include/pcreg.h: pcreg_icp_stop).  TEST INFRASTRUCTURE ONLY.
 
-The loop is oracle/icp.py's icp_single (same NN step, weights, rigid fit and compose; its helpers are reused) with the stop
-rule added.  The rule restates the documented 'Tolerance' of MATLAB's pcregistericp -- a translation and a rotation
+The loop is oracle/icp.py's icp_single (same NN step, weights, rigid fit and compose; its helpers are reused, so an update whose
+cross-covariance has numerical rank <= 2 is the proper solution, oracle.icp.RANK2_TAU) with the stop rule added.  The rule restates the documented 'Tolerance' of MATLAB's pcregistericp -- a translation and a rotation
 difference averaged over the most recent iterations -- and its parity with the toolbox is UNPINNED:
   after update u >= window, stop when mean(dt) < tol_t and mean(dr) < tol_r_deg over updates u-window+1 .. u
   (left-to-right FP64 sums divided by window, strict compares); the stopping update is applied.
