@@ -265,7 +265,9 @@ typedef struct {
  * plane), and 1 always returns a rotation.  tau = 1e-8: the one-pass pivot-relative sums leave S[2] / S[0] of an exactly planar set
  * at up to ~4e-15 (D / L)^2 for a patch of size L at distance D >= L from the model's pivot (4e-11 at D = 100 L), and a curved patch
  * has S[2] / S[0] ~ (sag / L)^2, so only a patch flatter than a relative sag of 1e-4 counts as planar.  estimateTransform and
- * RANSAC do not apply the rule. */
+ * RANSAC do not apply the rule.  The ICP update computes R = V*U' as the orthogonal polar factor of H' (a scaled Newton iteration)
+ * when det H alone proves S[2] >= 1e-6 S[0], S[0] is clear of the noise clause and reflection_fix would flip nothing; otherwise,
+ * and for estimateTransform and RANSAC, it takes the SVD, so rank-deficient, noise-level and flipped fits keep their bits. */
 void pcreg_icp_opts_default(pcreg_icp_opts* o);
 /* src: ns x 3 column-major; w_src[ns] optional; T0_16 [nhyp][16] initial poses.  Outputs (any
  * may be NULL except T16): T16 [nhyp][16], rmse [nhyp], n_used [nhyp], status [nhyp] (0 ok,

@@ -1,6 +1,6 @@
 // pcreg_math.cuh -- small FP64 linear algebra shared by every kernel (host + device).
 //
-// 3x3 one-sided Jacobi SVD, symmetric 3x3 Jacobi eigen-solver, Kabsch pose from the 16 weighted
+// 3x3 one-sided Jacobi SVD, 3x3 polar factor (Newton), symmetric 3x3 Jacobi eigen-solver, Kabsch pose from the 16 weighted
 // sums, row-vector 4x4 composition, the 6x6 LDL' solve and the Rodrigues rotation of the point-to-plane step.  Matrices are ROW-MAJOR double[9] / double[16] in here
 // (element (r,c) at [r*3+c] / [r*4+c]); the C ABI converts to MATLAB column-major at the edge.
 //
@@ -127,6 +127,58 @@ PCREG_HD void svd3(const double* A, double* U, double* S, double* V) {
     }
 }
 
+// 1 / sqrt(x) for the polar iteration's scaling, which sets only how fast it converges, not where to
+PCREG_HD double polar_rsqrt(double x) {
+#if defined(__CUDA_ARCH__)
+    return rsqrt(x);
+#else
+    return 1.0 / sqrt(x);
+#endif
+}
+
+constexpr int POLAR3_MAX_ITERS = 12;
+
+// Orthogonal polar factor Q of A^T (A^T = Q P, P symmetric positive definite) for a nonsingular 3x3 A: with A = U S V^T,
+// Q = V U^T, improper when det A < 0.  Scaled Newton iteration X <- (g X + X^-T / g) / 2 from X = A^T (Higham 1986), X^-T =
+// cof(X) / det X with one division, Frobenius scaling g = (|X^-1|_F / |X|_F)^(1/2) until a step moves X by less than 1e-2, then
+// unscaled steps.  Every step keeps the singular vectors and maps a singular value s to (g s + 1 / (g s)) / 2, so once the
+// singular values are 1 + e the next step leaves them at 1 + e^2 / 2: a step of at most 1e-8 (Frobenius) is followed by X
+// orthogonal to rounding, and that X is returned.  Returns the number of steps, or 0 (Q unusable) when the step did not reach
+// 1e-8 within POLAR3_MAX_ITERS or a value was not finite.  Random A with sigma_3 / sigma_1 from 1 down to 1e-6 take 2 to 7 steps
+// (tests/test_icp_polar_cpu.py).
+PCREG_HD int polar3(const double* A, double* Q) {
+    double X[9];
+    for (int r = 0; r < 3; ++r)
+        for (int c = 0; c < 3; ++c) X[r * 3 + c] = A[c * 3 + r];
+    bool scaled = true;
+    for (int it = 1; it <= POLAR3_MAX_ITERS; ++it) {
+        const double C[9] = {X[4] * X[8] - X[5] * X[7], X[5] * X[6] - X[3] * X[8], X[3] * X[7] - X[4] * X[6],
+                             X[2] * X[7] - X[1] * X[8], X[0] * X[8] - X[2] * X[6], X[1] * X[6] - X[0] * X[7],
+                             X[1] * X[5] - X[2] * X[4], X[2] * X[3] - X[0] * X[5], X[0] * X[4] - X[1] * X[3]};   // cof(X)
+        const double rdet = 1.0 / (X[0] * C[0] + X[1] * C[1] + X[2] * C[2]);
+        double f = 0.5, e = 0.5 * rdet;
+        if (scaled) {                   // g^2 = |cof X|_F |det X|^-1 |X|_F^-1
+            double a = 0.0, b = 0.0;
+            for (int k = 0; k < 9; ++k) { a += X[k] * X[k]; b += C[k] * C[k]; }
+            const double g2 = sqrt(b) * fabs(rdet) * polar_rsqrt(a), ginv = polar_rsqrt(g2);
+            f = 0.5 * g2 * ginv;
+            e *= ginv;
+        }
+        double d2 = 0.0;
+        for (int k = 0; k < 9; ++k) {
+            const double x = f * X[k] + e * C[k];
+            d2 += (x - X[k]) * (x - X[k]);
+            X[k] = x;
+        }
+        if (d2 <= 1e-16) {              // false for NaN; X is finite when it holds
+            for (int k = 0; k < 9; ++k) Q[k] = X[k];
+            return it;
+        }
+        if (d2 <= 1e-4) scaled = false;
+    }
+    return 0;
+}
+
 // Cyclic Jacobi eigen-decomposition of a symmetric 3x3 (only the upper triangle of A is trusted,
 // the matrix is symmetrised first).  Returns eigenvalues w (unsorted) and eigenvectors as the
 // COLUMNS of V (row-major storage).
@@ -207,10 +259,48 @@ constexpr int KABSCH_NSUMS = 17;
 // tests/test_icp_degenerate_cpu.py), so tau keeps a factor 8 of margin up to D = 500 L, while a curved patch has
 // S[2] / S[0] ~ (sag / L)^2, 1e-8 only at a relative sag of 1e-4.
 constexpr double ICP_RANK2_TAU = 1e-8;
+// The ICP update computes R = V*U' as polar3(H) where it can prove that neither clause of the rank rule holds and that
+// reflection_fix would flip nothing; every other H takes svd3 as estimateTransform does.  The certificate, from H alone:
+//  |det H| > ICP_POLAR_DET_C |H|_F^3: det H = S[0] S[1] S[2] <= S[0]^2 S[2] and |H|_F >= S[0], so S[2] / S[0] >= 1e-6, a factor
+//    100 above tau (the rounding of det3 and of svd3's S[2], a few ulp of S[0], is far below both); C3's updates have S[2] / S[0]
+//    >= 6e-4, and polar3 takes at most 7 steps down to 1e-6;
+//  |H|_F^2 >= ICP_POLAR_NOISE_F tau^2 f2: S[0]^2 >= |H|_F^2 / 3, so S[0] >= 1.15 tau sqrt(f2), 15 % above the noise clause (svd3's
+//    S[0] is good to a few ulp);
+//  with reflection_fix, det H > 0: then det(V U') = +1 and nothing is flipped.
+constexpr double ICP_POLAR_DET_C = 1e-6;
+constexpr double ICP_POLAR_NOISE_F = 4.0;
+
+// R = V*U' of the rigid fit to the cross-covariance H (row-major), flipped as reflection_fix and, with icp_rule, the ICP rank rule
+// say (f2 = |sum w q~ m~'|_F^2, read only with icp_rule).  Returns the polar3 step count when the ICP certificate above let polar3
+// compute R, 0 when svd3 did.
+PCREG_HD int kabsch_rotation(const double* H, double f2, bool reflection_fix, bool icp_rule, double* R) {
+    if (icp_rule) {
+        double h2 = 0.0;
+        for (int k = 0; k < 9; ++k) h2 += H[k] * H[k];
+        const double dH = det3(H);
+        if (dH * dH > (ICP_POLAR_DET_C * ICP_POLAR_DET_C) * (h2 * h2 * h2) && h2 >= ICP_POLAR_NOISE_F * (ICP_RANK2_TAU * ICP_RANK2_TAU) * f2 &&
+            (!reflection_fix || dH > 0.0)) {
+            const int it = polar3(H, R);
+            if (it > 0) return it;
+        }
+    }
+    double U[9], S[3], V[9];
+    svd3(H, U, S, V);                                                                      // :60
+    const bool fix = reflection_fix || (icp_rule && (S[2] <= ICP_RANK2_TAU * S[0] || S[0] <= ICP_RANK2_TAU * sqrt(f2)));
+    for (int pass = 0; pass < 2; ++pass) {
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c)                                                   // R = V * U'  (:62)
+                R[r * 3 + c] = V[r * 3 + 0] * U[c * 3 + 0] + V[r * 3 + 1] * U[c * 3 + 1] + V[r * 3 + 2] * U[c * 3 + 2];
+        if (pass == 1 || !fix || det3(R) >= 0.0) break;
+        for (int i = 0; i < 3; ++i) V[i * 3 + 2] = -V[i * 3 + 2];                        // flip the weakest direction
+    }
+    return 0;
+}
 
 // dT (row-major, row-vector convention) with [q,1]*dT ~ [m,1]  (estimateTransform(pts1 = m, pts2 = q)).
 // pivot_q / pivot_m: what was subtracted from the q side / the m side before summing.  icp_rule: the ICP update's rank rule
-// (ICP_RANK2_TAU); estimateTransform / RANSAC pass false and keep R = V*U' (with reflection_fix alone deciding the flip).
+// (ICP_RANK2_TAU) and its polar3 path; estimateTransform / RANSAC pass false and keep svd3's R = V*U' (with reflection_fix alone
+// deciding the flip).
 PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const double* pivot_m, bool reflection_fix, double* dT,
                                bool icp_rule = false) {
     const double inv = 1.0 / s.sw;
@@ -221,17 +311,8 @@ PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const
     double f2 = 0.0;                                                                       // |sum w q~ m~'|_F^2 (ICP rank rule)
     if (icp_rule)
         for (int k = 0; k < 9; ++k) f2 += s.sqm[k] * s.sqm[k];
-    double U[9], S[3], V[9];
-    svd3(H, U, S, V);                                                                      // :60
-    const bool fix = reflection_fix || (icp_rule && (S[2] <= ICP_RANK2_TAU * S[0] || S[0] <= ICP_RANK2_TAU * sqrt(f2)));
     double R[9];
-    for (int pass = 0; pass < 2; ++pass) {
-        for (int r = 0; r < 3; ++r)
-            for (int c = 0; c < 3; ++c)                                                   // R = V * U'  (:62)
-                R[r * 3 + c] = V[r * 3 + 0] * U[c * 3 + 0] + V[r * 3 + 1] * U[c * 3 + 1] + V[r * 3 + 2] * U[c * 3 + 2];
-        if (pass == 1 || !fix || det3(R) >= 0.0) break;
-        for (int i = 0; i < 3; ++i) V[i * 3 + 2] = -V[i * 3 + 2];                        // flip the weakest direction
-    }
+    kabsch_rotation(H, f2, reflection_fix, icp_rule, R);
     // t = cd - R*cm (:63) with cd = model centroid, cm = query centroid, pivot restored
     double t[3];
     for (int r = 0; r < 3; ++r) {
