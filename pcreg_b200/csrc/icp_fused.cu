@@ -37,7 +37,10 @@ namespace pcreg {
 #endif                          // Measured SLOWER (C4 polish, 16 384 poses: 592 vs 465 ms): the 34 accumulator registers push the NN loop
                                 // into spills.  Kept as a switch.
 
-__device__ __noinline__ void fused_walk(const GridArgs& a, double qx, double qy, double qz, int32_t warm, int32_t& bidx, double& best) {
+// Returned by value: reference outputs would make the NN loop's winners address-taken, stored to and reloaded from local memory
+// on every trip.
+struct WalkHit { int32_t bidx; double best; };
+__device__ __noinline__ WalkHit fused_walk(const GridArgs& a, double qx, double qy, double qz, int32_t warm) {
     Query Q;
     Q.qx = qx; Q.qy = qy; Q.qz = qz;
     setup_query_at(a.g, a.md, Q, 0.f, warm);
@@ -45,7 +48,7 @@ __device__ __noinline__ void fused_walk(const GridArgs& a, double qx, double qy,
     double thr2 = 0.0;
     unsigned long long n1 = 0, n2 = 0, n3 = 0;
     walk_search<false>(a, 0, Q, false, lc, ext_slot, thr2, 0.f, n1, n2, n3);
-    bidx = Q.bidx; best = Q.best;
+    return WalkHit{Q.bidx, Q.best};
 }
 template <int METRIC>
 __device__ __noinline__ bool fused_pose_update(const double (&s)[icp_nsums<METRIC>], long long n_used, const double* pivot, bool reflection_fix,
@@ -176,10 +179,10 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
             unsigned ng = 0;
             double w0c[3], w1c[3];                               // the winners' coordinates (modes without a trim: sums right here)
             if (ok0) { vox_scan<8, true>(V, pts, hd0, x0, y0, z0, q0x, q0y, q0z, b0, d0, ng, two_pass ? nullptr : w0c); c_read += hd0.y; c_gather += ng; }
-            else     { fused_walk(a.g, q0x, q0y, q0z, it > 0 ? idx_s[i0] : -1, b0, d0); ++c_walk; }
+            else     { const WalkHit r = fused_walk(a.g, q0x, q0y, q0z, it > 0 ? idx_s[i0] : -1); b0 = r.bidx; d0 = r.best; ++c_walk; }
             if (has1) {
                 if (ok1) { vox_scan<8, true>(V, pts, hd1, x1, y1, z1, q1x, q1y, q1z, b1, d1, ng, two_pass ? nullptr : w1c); c_read += hd1.y; c_gather += ng; }
-                else     { fused_walk(a.g, q1x, q1y, q1z, it > 0 ? idx_s[i1] : -1, b1, d1); ++c_walk; }
+                else     { const WalkHit r = fused_walk(a.g, q1x, q1y, q1z, it > 0 ? idx_s[i1] : -1); b1 = r.bidx; d1 = r.best; ++c_walk; }
             }
             idx_s[i0] = b0;
             if (has1) idx_s[i1] = b1;
