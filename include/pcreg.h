@@ -492,7 +492,50 @@ int  pcreg_icp_batch_extrap_dev(const pcreg_model* m, const double* d_src, const
                                 int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist, int64_t* d_best,
                                 int32_t* d_n_iter, int32_t* d_converged, int32_t* d_n_extrap, void* stream);
 
-/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev,_windows,_windows_dev,_extrap,_extrap_dev} or pcreg_nn_search call,
+/* ---- pose covariance and predicted target registration error ------------------------------------------------------------
+ * How well a returned pose is pinned down, without a ground truth: the linearised least-squares covariance of the point-to-plane
+ * objective at given poses, and the predicted RMS displacement of caller targets (a lesion, a drill entry) under it.  Parity with any
+ * toolbox is UNPINNED.
+ * Pass.  The entry evaluates the poses T16 and runs no update: it makes exactly the scoring pass pcreg_icp_batch makes at its final
+ * pose, with the same exact NN, rejection (thDist2), mode (PLAIN, KNN trim, WEIGHTED) and w_src.  So for an ICP result passed with the
+ * same opts, rmse, n_used and the correspondences equal that call's final pass bit for bit.  opts.iters and opts.reflection_fix are
+ * ignored.  It needs model normals (else PCREG_ERR_STATE), as POINT_TO_PLANE does.
+ * Sums.  For every correspondence with w > 0, with q = quickTF(s, T), m its model point, n its unit model normal and p the model's pivot:
+ *   q~ = q - p, m~ = m - p, a = (q~ x n, n), b = (m~ - q~) . n;  A = sum w a a', B = sum w b^2, S = sum w (FP64).
+ * Noise scale.  sigma2 = (B / S) n_used / (n_used - 6).
+ * Parametrisation.  A small perturbation of the pose moves a model-frame point x to x + omega x (x - ref) + tau; unknowns (omega, tau)
+ * in that order (as POINT_TO_PLANE); ref: double[3], NULL = the model-frame origin.  Sums and the L D L' factorisation stay about p;
+ * with M = [[I, 0], [-[ref - p]x, I]]:
+ *   cov36 = sigma2 M A^-1 M'  (6 x 6 row-major = column-major, symmetric; rad and model units),
+ *   info36 = M^-T A M^-1     (the unscaled Hessian, Open3D's "information matrix"; its eigenvectors of small eigenvalue are the
+ *                             directions the data leave free).  Written whenever n_used > 0, NaN otherwise.
+ * Degenerate case.  status 1 when n_used <= 6, S is not > 0 or a pivot of the L D L' factorisation is <= 1e-12 max A_kk (the flat-patch
+ * rule of POINT_TO_PLANE): cov36 and tre are NaN (info36 is still written; sigma2 is NaN only when n_used <= 6 or S is not > 0).
+ * Noise-free data on a plane leave info of rank 3 (the in-plane translations and the rotation about the normal are free), on a cylinder
+ * rank 4 (the axial translation and the rotation about the axis) and on a sphere rank 3 (every rotation about the centre).
+ * Target registration error.  targets: ntarget x 3 column-major doubles in the model frame, shared by every hypothesis (NULL with
+ * ntarget = 0); tre [nhyp][ntarget] (optional) = sqrt(trace(J_k cov J_k')), J_k = [-[x_k - ref]x, I]: the predicted RMS displacement of
+ * target k.  It does not depend on ref.
+ * Assumptions.  Independent residuals along the model normal with a common variance and fixed correspondences: cov describes the precision
+ * of the minimum of the linearised objective, not whether ICP reached it.  DESIGN.md section 3.3 gives the measured calibration.
+ * Layout.  The windows layout of pcreg_icp_batch_extrap (src_offsets / hyp_offsets, nwin = 1: one source for every pose); per-hypothesis
+ * outputs indexed by the global hypothesis.  cov36 [nhyp][36], sigma2 [nhyp] and status [nhyp] are required; info36, rmse, n_used and tre
+ * are optional.  PCREG_ERR_ARG: the errors of pcreg_icp_batch_windows, a null required output, a non-finite ref or target, or ntarget < 0.
+ * Sharded over the devices as the other ICP entries; results do not depend on the device count.  Paths (brute force, grid, voxel map,
+ * fused kernel) as pcreg_icp_batch_windows, and they agree bit for bit. */
+int  pcreg_icp_covariance(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                          const double* w_src, const int64_t* hyp_offsets, int64_t nwin, const double* T16, const pcreg_icp_opts* opts,
+                          const double* ref, const double* targets, int64_t ntarget, double* cov36, double* info36, double* sigma2,
+                          double* rmse, int32_t* n_used, int32_t* status, double* tre);
+/* The same on device arrays (src and w_src float64 column-major with ld = ns_total, T16 and every output on the device), synchronous with
+ * respect to `stream` as pcreg_icp_batch_windows_dev.  src_offsets, hyp_offsets, ref and targets are HOST arrays. */
+int  pcreg_icp_covariance_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                              const int64_t* hyp_offsets, int64_t nwin, const double* d_T16, const pcreg_icp_opts* opts, const double* ref,
+                              const double* targets, int64_t ntarget, double* d_cov36, double* d_info36, double* d_sigma2, double* d_rmse,
+                              int32_t* d_n_used, int32_t* d_status, double* d_tre, void* stream);
+
+/* Timing / accounting of the most recent pcreg_icp_batch{,_dev,_stop,_stop_dev,_metric,_metric_dev,_gicp,_gicp_dev,_windows,_windows_dev,_extrap,_extrap_dev},
+ * pcreg_icp_covariance{,_dev} or pcreg_nn_search call,
  * measured with CUDA events on the launching stream (bench.py's roofline numbers):
  *   out[0] = NN kernel launches, out[1] = total NN kernel ms, out[2] = NN queries (with the tolerance stop: the queries of
  *   the passes each hypothesis ran, except on the brute-force and map-less grid paths, which still search for stopped

@@ -136,6 +136,12 @@ SIGNATURES = {
                                              C.POINTER(IcpOpts), C.POINTER(IcpStop), C.POINTER(IcpExtrap), C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p]),
+    "pcreg_icp_covariance": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, c_i64p, c_f64p, c_i64p, C.c_int64, c_f64p,
+                                       C.POINTER(IcpOpts), c_f64p, c_f64p, C.c_int64, c_f64p, c_f64p, c_f64p, c_f64p, c_i32p, c_i32p,
+                                       c_f64p]),
+    "pcreg_icp_covariance_dev": (C.c_int, [C.c_void_p, C.c_void_p, c_i64p, C.c_void_p, c_i64p, C.c_int64, C.c_void_p,
+                                           C.POINTER(IcpOpts), c_f64p, c_f64p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pcreg_set_profiling": (C.c_int, [C.c_int]),
     "pcreg_last_profile": (C.c_int, [c_f64p]),
 }

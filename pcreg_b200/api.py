@@ -702,6 +702,71 @@ def icp_batch_windows(model: Model, src_list, T0_list, mode=ICP_PLAIN, iters=50,
     return out
 
 
+def icp_covariance(model: Model, src, T, mode=ICP_PLAIN, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src=None, nn=NN_BRUTE, ref=None,
+                   targets=None, return_info=False):
+    """Pose covariance of the point-to-plane objective at the poses T [H,4,4] (include/pcreg.h: pcreg_icp_covariance): one scoring pass
+    with icp_batch's correspondences, rejection, mode and weights, no update.  Needs the model's normals.
+    Returns dict(cov [H,6,6] (unknowns (omega, tau), rad and model units, about `ref` -- a model-frame point, default the origin),
+    sigma2 [H], rmse [H], n_used [H], status [H] (1: degenerate, cov and tre NaN), tre [H,K] (the predicted RMS displacement of each
+    model-frame target, targets [K,3]; [H,0] without targets), info [H,6,6]? (the unscaled Hessian, return_info=True)).
+    For an icp_batch result passed with the same options, rmse and n_used equal that call's bit for bit."""
+    return icp_covariance_windows(model, [src], [T], mode, k_frac, R_w, thDist2, None if w_src is None else [w_src], nn, ref, targets,
+                                  return_info)[0]
+
+
+def icp_covariance_windows(model: Model, src_list, T_list, mode=ICP_PLAIN, k_frac=0.85, R_w=3.5, thDist2=0.0, w_src_list=None,
+                           nn=NN_BRUTE, ref=None, targets=None, return_info=False):
+    """icp_covariance for many matching windows in ONE call: window w evaluates the poses T_list[w] [H_w,4,4] against its own source
+    src_list[w] (with w_src_list[w] when given); ref, targets and every other keyword are shared.  One dict per window, each what
+    icp_covariance(model, src_list[w], T_list[w], ...) returns."""
+    nw = len(src_list)
+    if len(T_list) != nw or (w_src_list is not None and len(w_src_list) != nw):
+        raise ValueError("one source, one pose array (and one w_src array, when given) per window")
+    srcs = [np.asarray(p).reshape(-1, 3) for p in src_list]
+    dt = np.float32 if all(p.dtype == np.float32 for p in srcs) else np.float64
+    ns = np.array([p.shape[0] for p in srcs], dtype=np.int64)
+    soff = np.zeros(nw + 1, dtype=np.int64)
+    np.cumsum(ns, out=soff[1:])
+    nt = int(soff[-1])
+    cat = np.asfortranarray(np.concatenate([p.astype(dt, copy=False) for p in srcs], axis=0)) if nt else np.zeros((1, 3), dtype=dt, order="F")
+    Ts = [np.asarray(t, dtype=np.float64).reshape(-1, 4, 4) for t in T_list]
+    hoff = np.zeros(nw + 1, dtype=np.int64)
+    np.cumsum([t.shape[0] for t in Ts], out=hoff[1:])
+    nh = int(hoff[-1])
+    T = _T_to_abi(np.concatenate(Ts, axis=0)) if nh else np.zeros((1, 4, 4))
+    w = None
+    if w_src_list is not None:
+        ws = [np.asarray(x, dtype=np.float64).reshape(-1) for x in w_src_list]
+        if any(x.shape[0] != n for x, n in zip(ws, ns)):
+            raise ValueError("w_src_list[w] must hold one weight per source point of window w")
+        w = np.ascontiguousarray(np.concatenate(ws)) if nt else np.zeros(1)
+    rf = None if ref is None else np.ascontiguousarray(np.asarray(ref, dtype=np.float64).reshape(3))
+    tg = np.zeros((0, 3)) if targets is None else np.asarray(targets, dtype=np.float64).reshape(-1, 3)
+    K = tg.shape[0]
+    tg_cm = np.asfortranarray(tg) if K else None
+    o = icp_opts(mode, 0, k_frac, R_w, thDist2, nn)
+    H1 = max(nh, 1)
+    cov = np.empty((H1, 36))
+    info = np.empty((H1, 36)) if return_info else None
+    sigma2, rmse = np.empty(H1), np.empty(H1)
+    n_used, status = np.empty(H1, dtype=np.int32), np.empty(H1, dtype=np.int32)
+    tre = np.empty((H1, max(K, 1)))
+    L.check(L.lib().pcreg_icp_covariance(model.handle, cat.ctypes.data_as(C.c_void_p), int(dt == np.float64), cat.shape[0],
+                                         _ptr(soff, L.c_i64p), _ptr(w, L.c_f64p), _ptr(hoff, L.c_i64p), nw, _ptr(T, L.c_f64p), C.byref(o),
+                                         _ptr(rf, L.c_f64p), _ptr(tg_cm, L.c_f64p), K, _ptr(cov, L.c_f64p), _ptr(info, L.c_f64p),
+                                         _ptr(sigma2, L.c_f64p), _ptr(rmse, L.c_f64p), _ptr(n_used, L.c_i32p), _ptr(status, L.c_i32p),
+                                         _ptr(tre, L.c_f64p) if K else None), "pcreg_icp_covariance")
+    out = []
+    for k in range(nw):
+        a, b = int(hoff[k]), int(hoff[k + 1])
+        r = dict(cov=cov[a:b].reshape(-1, 6, 6).copy(), sigma2=sigma2[a:b].copy(), rmse=rmse[a:b].copy(), n_used=n_used[a:b].copy(),
+                 status=status[a:b].copy(), tre=tre[a:b, :K].copy())
+        if return_info:
+            r["info"] = info[a:b].reshape(-1, 6, 6).copy()
+        out.append(r)
+    return out
+
+
 def set_profiling(enabled):
     """True / 1: event times + work counters; 2: event times only (no counter atomics in the kernels); False: off."""
     L.check(L.lib().pcreg_set_profiling(int(enabled)), "pcreg_set_profiling")

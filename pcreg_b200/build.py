@@ -70,7 +70,7 @@ def build_hostmath(force: bool = False) -> str:
     """Host-only build of pcreg_math.cuh behind a tiny C ABI (tests/hostmath): lets the CPU test
     suite check the 3x3 SVD / eigen / Kabsch code that the kernels inline, without a GPU."""
     root = os.path.dirname(HERE)
-    srcs = [os.path.join(root, "tests", "hostmath", f) for f in ("hostmath.cpp", "hostmath_plane.cpp", "hostmath_gicp.cpp", "hostmath_extrap.cpp", "hostmath_polar.cpp")]
+    srcs = [os.path.join(root, "tests", "hostmath", f) for f in ("hostmath.cpp", "hostmath_plane.cpp", "hostmath_gicp.cpp", "hostmath_extrap.cpp", "hostmath_polar.cpp", "hostmath_cov.cpp")]
     out = os.path.join(root, "tests", "hostmath", "libhostmath.so")
     deps = srcs + [os.path.join(CSRC, "pcreg_math.cuh")]
     if not force and os.path.exists(out) and os.path.getmtime(out) >= _newest(deps):

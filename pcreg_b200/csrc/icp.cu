@@ -37,7 +37,8 @@ struct Pose16 { double t[16]; };      // a row-major row-vector pose as a kernel
 // STOP = the tolerance stop (a.stop_iter set); the STOP = 0 instantiations are the loop without it; STOP = 2 (METRIC 0 only, a.ex_state
 // set as well) adds the pose extrapolation before the stop rule.
 // METRIC = 1: the point-to-plane metric (a.nrm set): 29 sums, the normals gathered with the model points; 2: plane-to-plane
-// (a.snx set as well): the same, and each correspondence's source normal read with the source point and rotated by the pose.
+// (a.snx set as well): the same, and each correspondence's source normal read with the source point and rotated by the pose;
+// 3 (STOP = 0 only, a.cov.cov set): the covariance pass of pcreg_icp_covariance, the final pass alone, writing a.cov instead of a pose.
 template <int NT, int STOP, int METRIC>
 __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __grid_constant__ IcpUpdateArgs a) {
     constexpr int NS = icp_nsums<METRIC>;
@@ -166,6 +167,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             double qx, qy, qz;
             quick_tf(Ts, xs[u], ys[u], zs[u], qx, qy, qz);
             if constexpr (SNRM) icp_accumulate_gicp(s, w, d, qx, qy, qz, mm[u], nv[u], snx[u], sny[u], snz[u], Ts, a.gicp_eps, px, py, pz);
+            else if constexpr (METRIC == ICP_M_COV) icp_accumulate_cov(s, w, d, qx, qy, qz, mm[u], nv[u], px, py, pz);
             else if constexpr (MNRM) icp_accumulate_plane(s, w, d, qx, qy, qz, mm[u], nv[u], px, py, pz);
             else icp_accumulate(s, w, d, qx, qy, qz, mm[u], px, py, pz);
         }
@@ -189,7 +191,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
         }
         if (a.rmse_hist) for (int c = hist_from; c <= a.hist_col; ++c) a.rmse_hist[h * a.hist_stride + c] = rmse;
         float moved = 0.f;
-        if (a.update && !a.frozen[h]) {
+        if (METRIC != ICP_M_COV && a.update && !a.frozen[h]) {
             double Tn[16], Tc[16];
             for (int k = 0; k < 16; ++k) Tc[k] = Ts[k];
             bool ok;
@@ -245,6 +247,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) k_icp_update(const __gr
             a.skip_thr[h] = thr;
         }
     }
+    if constexpr (METRIC == ICP_M_COV) icp_cov_write(a.cov, s, n_used, a.pivot, h, red);
 }
 
 // centroid and radius of the source cloud (for the per-update motion bound): one block
@@ -475,8 +478,15 @@ static void icp_update_launch_metric(const IcpUpdateArgs& a, int64_t nhyp, cudaS
     else if (stop)    k_icp_update<UPD_THREADS, 1, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
     else              k_icp_update<UPD_THREADS, 0, METRIC><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
 }
+// the covariance pass has no stop and no extrapolation
+template <>
+void icp_update_launch_metric<ICP_M_COV>(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
+    if (a.ns > 20000) k_icp_update<512, 0, ICP_M_COV><<<(unsigned)nhyp, 512, 0, st>>>(a);
+    else              k_icp_update<UPD_THREADS, 0, ICP_M_COV><<<(unsigned)nhyp, UPD_THREADS, 0, st>>>(a);
+}
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st) {
-    if (a.snx)      icp_update_launch_metric<ICP_M_GICP>(a, nhyp, st);
+    if (a.cov.cov)  icp_update_launch_metric<ICP_M_COV>(a, nhyp, st);
+    else if (a.snx) icp_update_launch_metric<ICP_M_GICP>(a, nhyp, st);
     else if (a.nrm) icp_update_launch_metric<ICP_M_PLANE>(a, nhyp, st);
     else            icp_update_launch_metric<ICP_M_POINT>(a, nhyp, st);
     PCREG_LAUNCHED();
@@ -498,7 +508,8 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     double* d_rmse_hist, int64_t* d_best, cudaStream_t st,
                     const pcreg_icp_stop* stop = nullptr, int32_t* d_n_iter = nullptr, int32_t* d_converged = nullptr,
                     int metric = ICP_M_POINT, const double* d_src_nrm = nullptr /*ICP_M_GICP: col-major ns x 3*/, double gicp_eps = 0.0,
-                    const IcpExtrapRule* ex = nullptr /*needs stop*/, const double* d_ex_cen = nullptr /*[3]*/, int32_t* d_n_extrap = nullptr) {
+                    const IcpExtrapRule* ex = nullptr /*needs stop*/, const double* d_ex_cen = nullptr /*[3]*/, int32_t* d_n_extrap = nullptr,
+                    const IcpCovOut* cov = nullptr /*metric ICP_M_COV, iters 0*/) {
     PCREG_REQUIRE(m && d_src && d_T0_cm && d_T16_cm, "icp: null pointer");
     const bool plane = metric != ICP_M_POINT, gicp = metric == ICP_M_GICP;
     const ModelPointD* nrm = plane ? m->nrm.p : nullptr;
@@ -518,6 +529,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
     double t_alloc = 0, t_sorted = 0, t_enq = 0;
 
     PCREG_REQUIRE(!ex || (stop && d_ex_cen && metric == ICP_M_POINT), "icp: extrapolation needs a stop rule, the centroid and point-to-point");
+    PCREG_REQUIRE((cov != nullptr) == (metric == ICP_M_COV) && (!cov || (o.iters == 0 && !stop)), "icp: the covariance pass runs alone");
     const int stop_mode = ex ? 2 : stop ? 1 : 0;
     const bool fused = icp_fused_eligible(m, ns, nhyp, o, stop_mode, metric);
     // chunk the hypotheses so that the per-correspondence scratch stays bounded
@@ -672,6 +684,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
         fa.stop = rule; fa.n_iter = d_n_iter; fa.converged = d_converged; fa.nrm = nrm;
         fa.snx = snx; fa.sny = sny; fa.snz = snz; fa.gicp_eps = gicp_eps;
         if (ex) { fa.ex = *ex; fa.ex_cen = d_ex_cen; fa.n_extrap = d_n_extrap; }
+        if (cov) fa.cov = *cov;
         ev_begin(0);
         icp_fused_launch(fa, nhyp, stop_mode, st);
         ev_end();
@@ -774,6 +787,7 @@ static void icp_run(const pcreg_model* m, const double* d_src /*col-major ns x 3
                     ua.ex = *ex; ua.ex_state = ex_state.p + h0 * EXTRAP_STATE; ua.ex_cen = d_ex_cen;
                     ua.n_extrap = d_n_extrap ? d_n_extrap + h0 : nullptr;
                 }
+                if (cov) ua.cov = cov_out_at(*cov, h0);
                 ev_begin(1);
                 icp_update_launch(ua, hn, ls);
                 ev_end();
@@ -874,7 +888,7 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
                             const double* d_T0_cm, const pcreg_icp_opts& o, const pcreg_icp_stop* stop, int metric, double gicp_eps,
                             double* d_T16_cm, double* d_rmse, int32_t* d_n_used, int32_t* d_status, int32_t* d_idx, double* d_rmse_hist,
                             int64_t* d_best, int32_t* d_n_iter, int32_t* d_converged, cudaStream_t st,
-                            const IcpExtrapRule* ex = nullptr, int32_t* d_n_extrap = nullptr) {
+                            const IcpExtrapRule* ex = nullptr, int32_t* d_n_extrap = nullptr, const IcpCovOut* cov = nullptr) {
     PCREG_REQUIRE(m && d_T16_cm && (L.nrows == 0 || d_src) && (L.nhyp == 0 || d_T0_cm), "icp windows: null pointer");
     const bool gicp = metric == ICP_M_GICP;
     const ModelPointD* nrm = metric != ICP_M_POINT ? m->nrm.p : nullptr;
@@ -940,11 +954,12 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
                 PCREG_CUDA(cudaMemcpyAsync(src_w.p + a * ns, d_src + a * nrows + r0, (size_t)ns * sizeof(double), cudaMemcpyDeviceToDevice, st));
                 if (gicp) PCREG_CUDA(cudaMemcpyAsync(nrm_w.p + a * ns, d_src_nrm + a * nrows + r0, (size_t)ns * sizeof(double), cudaMemcpyDeviceToDevice, st));
             }
+            const IcpCovOut cw = cov ? cov_out_at(*cov, h0) : IcpCovOut{};
             icp_run(m, src_w.p, ns, d_w ? d_w + r0 : nullptr, d_T0_cm + h0 * 16, nh, o, d_T16_cm + h0 * 16, d_rmse ? d_rmse + h0 : nullptr,
                     d_n_used ? d_n_used + h0 : nullptr, d_status ? d_status + h0 : nullptr, d_idx ? d_idx + L.idx_off[w] : nullptr,
                     d_rmse_hist ? d_rmse_hist + h0 * hs : nullptr, d_best ? d_best + w : nullptr, st, stop,
                     d_n_iter ? d_n_iter + h0 : nullptr, d_converged ? d_converged + h0 : nullptr, metric, gicp ? nrm_w.p : nullptr, gicp_eps,
-                    ex, ex ? cen.p + 3 * w : nullptr, d_n_extrap ? d_n_extrap + h0 : nullptr);
+                    ex, ex ? cen.p + 3 * w : nullptr, d_n_extrap ? d_n_extrap + h0 : nullptr, cov ? &cw : nullptr);
             if (prof) {
                 for (int k = 0; k < 26; ++k) prof_sum[k] += c.profile[k];
                 prof_sum[26] = std::max(prof_sum[26], c.profile[26]);
@@ -982,6 +997,7 @@ static void icp_windows_run(const pcreg_model* m, const WindowLayout& L, const d
     fa.snx = gicp ? snrm.p : nullptr; fa.sny = gicp ? snrm.p + nrows : nullptr; fa.snz = gicp ? snrm.p + 2 * nrows : nullptr; fa.gicp_eps = gicp_eps;
     fa.win_src = d_soff; fa.win_hyp = d_hoff; fa.win_idx = d_ioff; fa.nwin = (int32_t)L.nwin;
     if (ex) { fa.ex = *ex; fa.ex_cen = cen.p; fa.n_extrap = d_n_extrap; }
+    if (cov) fa.cov = *cov;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (prof) { e0 = pooled_event(0); e1 = pooled_event(1); PCREG_CUDA(cudaEventRecord(e0, st)); }
     icp_fused_windows_launch(fa, nhyp, stop_mode, st);
@@ -1250,13 +1266,20 @@ static void check_windows(const pcreg_model* m, const int64_t* src_off, const in
         throw StateError{"icp: the point-to-plane and plane-to-plane metrics need model normals (pcreg_model_set_normals / pcreg_model_compute_normals)"};
 }
 
+// Host outputs and inputs of pcreg_icp_covariance (the covariance pass; its status goes to the call's status array)
+struct CovHost {
+    double ref[3];
+    const double* targets; int64_t ntarget;     // [3][ntarget] column-major or null
+    double* cov; double* info; double* sigma2; double* tre;
+};
+
 // One device's share [h0, h1) of a windowed host call: the windows it touches (a share may start or end inside a window), their rows
 // and rebased offsets; every output lands in its own slice of the caller's arrays.
 static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, const std::vector<double>& hs, const double* w_src,
                                    const std::vector<double>& hnrm, const double* T0_16, int64_t h0, int64_t h1, const pcreg_icp_opts& o,
                                    const pcreg_icp_stop* stop, int metric, double eps, double* T16, double* rmse, int32_t* n_used,
                                    int32_t* status, int32_t* idx, double* rmse_hist, int32_t* n_iter, int32_t* converged,
-                                   const IcpExtrapRule* ex, int32_t* n_extrap) {
+                                   const IcpExtrapRule* ex, int32_t* n_extrap, const CovHost* cv) {
     PCREG_CUDA(cudaSetDevice(ctx().device));
     cudaStream_t st = 0;
     const int64_t wa = L.window_of(h0), wb = L.window_of(h1 - 1), nw = wb - wa + 1;
@@ -1278,8 +1301,24 @@ static void icp_windows_host_slice(const pcreg_model* m, const WindowLayout& L, 
     }
     if (w_src) PCREG_CUDA(cudaMemcpyAsync(d_w.p, w_src + ra, d_w.bytes(), cudaMemcpyHostToDevice, st));
     PCREG_CUDA(cudaMemcpyAsync(d_T0.p, T0_16 + h0 * 16, d_T0.bytes(), cudaMemcpyHostToDevice, st));
-    icp_windows_run(m, S, d_src.p, d_w.p, d_nrm.p, d_T0.p, o, stop, metric, eps, d_T.p, d_rmse.p, d_nu.p, d_st.p, d_idx.p, d_hist.p,
-                    nullptr, d_nit.p, d_conv.p, st, ex, d_nex.p);
+    const int64_t nt = cv ? cv->ntarget : 0;
+    DevBuf<double> c_cov(cv ? (size_t)hn * 36 : 0), c_info(cv && cv->info ? (size_t)hn * 36 : 0), c_sig(cv ? (size_t)hn : 0);
+    DevBuf<double> c_tre(cv && cv->tre ? (size_t)(hn * nt) : 0), c_tg((size_t)nt * 3);
+    IcpCovOut co{};
+    if (cv) {
+        co.cov = c_cov.p; co.info = c_info.p; co.sigma2 = c_sig.p; co.status = d_st.p; co.tre = c_tre.p;
+        co.targets = c_tg.p; co.ntarget = (int32_t)nt;
+        for (int k = 0; k < 3; ++k) co.ref[k] = cv->ref[k];
+        if (nt) PCREG_CUDA(cudaMemcpyAsync(c_tg.p, cv->targets, c_tg.bytes(), cudaMemcpyHostToDevice, st));
+    }
+    icp_windows_run(m, S, d_src.p, d_w.p, d_nrm.p, d_T0.p, o, stop, metric, eps, d_T.p, d_rmse.p, d_nu.p, cv ? nullptr : d_st.p, d_idx.p,
+                    d_hist.p, nullptr, d_nit.p, d_conv.p, st, ex, d_nex.p, cv ? &co : nullptr);
+    if (cv) {
+        PCREG_CUDA(cudaMemcpyAsync(cv->cov + h0 * 36, c_cov.p, c_cov.bytes(), cudaMemcpyDeviceToHost, st));
+        if (cv->info) PCREG_CUDA(cudaMemcpyAsync(cv->info + h0 * 36, c_info.p, c_info.bytes(), cudaMemcpyDeviceToHost, st));
+        PCREG_CUDA(cudaMemcpyAsync(cv->sigma2 + h0, c_sig.p, c_sig.bytes(), cudaMemcpyDeviceToHost, st));
+        if (c_tre.p) PCREG_CUDA(cudaMemcpyAsync(cv->tre + h0 * nt, c_tre.p, c_tre.bytes(), cudaMemcpyDeviceToHost, st));
+    }
     PCREG_CUDA(cudaMemcpyAsync(T16 + h0 * 16, d_T.p, d_T.bytes(), cudaMemcpyDeviceToHost, st));
     PCREG_CUDA(cudaMemcpyAsync(rmse + h0, d_rmse.p, d_rmse.bytes(), cudaMemcpyDeviceToHost, st));
     if (n_used) PCREG_CUDA(cudaMemcpyAsync(n_used + h0, d_nu.p, d_nu.bytes(), cudaMemcpyDeviceToHost, st));
@@ -1297,7 +1336,8 @@ static int icp_windows_host(const pcreg_model* m, const void* src, int is_double
                             const double* w_src, const void* src_nrm, double gicp_eps, const int64_t* hyp_offsets, int64_t nwin,
                             const double* T0_16, const pcreg_icp_opts* opts, int metric, const pcreg_icp_stop* stop,
                             double* T16, double* rmse, int32_t* n_used, int32_t* status, int32_t* idx, double* rmse_hist,
-                            int64_t* best, int32_t* n_iter, int32_t* converged, const IcpExtrapRule* ex, int32_t* n_extrap) {
+                            int64_t* best, int32_t* n_iter, int32_t* converged, const IcpExtrapRule* ex, int32_t* n_extrap,
+                            const CovHost* cv = nullptr) {
     const WindowLayout L(src_offsets, hyp_offsets, nwin);
     PCREG_REQUIRE((L.nrows == 0 || src) && (L.nhyp == 0 || (T0_16 && T16)) && ld >= L.nrows, "pcreg_icp_batch_windows: null pointer or bad ld");
     const bool gicp = metric == PCREG_ICP_PLANE_TO_PLANE;
@@ -1321,7 +1361,8 @@ static int icp_windows_host(const pcreg_model* m, const void* src, int is_double
             const int64_t h0 = k * per, h1 = std::min(L.nhyp, h0 + per);
             if (h1 <= h0) return;
             rc[k] = guarded([&]() { use_slot(k); icp_windows_host_slice(m->on_slot(k), L, hs, w_src, hnrm, T0_16, h0, h1, *opts, stop, metric, gicp_eps,
-                                                                      T16, rm, n_used, status, idx, rmse_hist, n_iter, converged, ex, n_extrap); });
+                                                                      T16, rm, n_used, status, idx, rmse_hist, n_iter, converged, ex, n_extrap,
+                                                                      cv); });
         };
         for (int k = 1; k < nd; ++k) workers.emplace_back(run, k);
         run(0);
@@ -1411,6 +1452,63 @@ int pcreg_icp_batch_extrap_dev(const pcreg_model* m, const double* d_src, const 
     icp_windows_run(m, L, d_src, d_w_src, nullptr, d_T0_16, *opts, stop, PCREG_ICP_POINT_TO_POINT, 0.0, d_T16, d_rmse, d_n_used, d_status,
                     d_idx, d_rmse_hist, d_best, stop ? d_n_iter : nullptr, stop ? d_converged : nullptr, (cudaStream_t)stream,
                     ex ? &rule : nullptr, ex ? d_n_extrap : nullptr);
+    return PCREG_OK;
+    PCREG_API_END
+}
+
+// pcreg_icp_covariance{,_dev}: the checks of the windows entry (metric 1: model normals needed), then the pass's own
+static pcreg_icp_opts check_cov(const pcreg_model* m, const int64_t* src_off, const int64_t* hyp_off, int64_t nwin, const pcreg_icp_opts* opts,
+                                const double* ref, const double* targets, int64_t ntarget, const void* cov36, const void* sigma2,
+                                const void* status, CovHost& cv) {
+    check_windows(m, src_off, hyp_off, nwin, opts, PCREG_ICP_POINT_TO_PLANE, nullptr, 0.0, nullptr);
+    PCREG_REQUIRE(cov36 && sigma2 && status, "pcreg_icp_covariance: cov36, sigma2 and status are required");
+    PCREG_REQUIRE(ntarget >= 0 && ntarget < ((int64_t)1 << 31) && (ntarget == 0 || targets), "pcreg_icp_covariance: bad targets");
+    for (int k = 0; k < 3; ++k) {
+        cv.ref[k] = ref ? ref[k] : 0.0;
+        PCREG_REQUIRE(std::isfinite(cv.ref[k]), "pcreg_icp_covariance: ref must be finite");
+    }
+    for (int64_t i = 0; i < 3 * ntarget; ++i) PCREG_REQUIRE(std::isfinite(targets[i]), "pcreg_icp_covariance: targets must be finite");
+    cv.targets = ntarget ? targets : nullptr; cv.ntarget = ntarget;
+    pcreg_icp_opts o = *opts;
+    o.iters = 0;
+    o.reflection_fix = 0;
+    return o;
+}
+
+int pcreg_icp_covariance(const pcreg_model* m, const void* src, int is_double, int64_t ld, const int64_t* src_offsets,
+                         const double* w_src, const int64_t* hyp_offsets, int64_t nwin, const double* T16, const pcreg_icp_opts* opts,
+                         const double* ref, const double* targets, int64_t ntarget, double* cov36, double* info36, double* sigma2,
+                         double* rmse, int32_t* n_used, int32_t* status, double* tre) {
+    PCREG_API_BEGIN
+    require_init();
+    CovHost cv{};
+    const pcreg_icp_opts o = check_cov(m, src_offsets, hyp_offsets, nwin, opts, ref, targets, ntarget, cov36, sigma2, status, cv);
+    cv.cov = cov36; cv.info = info36; cv.sigma2 = sigma2; cv.tre = ntarget ? tre : nullptr;
+    std::vector<double> T_out((size_t)std::max<int64_t>(1, hyp_offsets[nwin]) * 16);      // the pass leaves the poses alone
+    return icp_windows_host(m, src, is_double, ld, src_offsets, w_src, nullptr, 0.0, hyp_offsets, nwin, T16, &o, ICP_M_COV, nullptr,
+                            T_out.data(), rmse, n_used, status, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, &cv);
+    PCREG_API_END
+}
+
+int pcreg_icp_covariance_dev(const pcreg_model* m, const double* d_src, const int64_t* src_offsets, const double* d_w_src,
+                             const int64_t* hyp_offsets, int64_t nwin, const double* d_T16, const pcreg_icp_opts* opts, const double* ref,
+                             const double* targets, int64_t ntarget, double* d_cov36, double* d_info36, double* d_sigma2, double* d_rmse,
+                             int32_t* d_n_used, int32_t* d_status, double* d_tre, void* stream) {
+    PCREG_API_BEGIN
+    require_init();
+    CovHost cv{};
+    const pcreg_icp_opts o = check_cov(m, src_offsets, hyp_offsets, nwin, opts, ref, targets, ntarget, d_cov36, d_sigma2, d_status, cv);
+    PCREG_CUDA(cudaSetDevice(ctx().device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const WindowLayout L(src_offsets, hyp_offsets, nwin);
+    DevBuf<double> T_out((size_t)std::max<int64_t>(1, L.nhyp) * 16), d_tg((size_t)ntarget * 3);
+    if (ntarget) PCREG_CUDA(cudaMemcpyAsync(d_tg.p, targets, d_tg.bytes(), cudaMemcpyHostToDevice, st));
+    IcpCovOut co{};
+    co.cov = d_cov36; co.info = d_info36; co.sigma2 = d_sigma2; co.status = d_status; co.tre = ntarget ? d_tre : nullptr;
+    co.targets = d_tg.p; co.ntarget = (int32_t)ntarget;
+    for (int k = 0; k < 3; ++k) co.ref[k] = cv.ref[k];
+    icp_windows_run(m, L, d_src, d_w_src, nullptr, d_T16, o, nullptr, ICP_M_COV, 0.0, T_out.p, d_rmse, d_n_used, nullptr, nullptr, nullptr,
+                    nullptr, nullptr, nullptr, st, nullptr, nullptr, &co);
     return PCREG_OK;
     PCREG_API_END
 }

@@ -103,6 +103,8 @@ __device__ __forceinline__ FusedWindow fused_window(const Args& a, int64_t h) {
 // only) adds the pose extrapolation (pcreg_icp_batch_extrap) before the stop rule.
 // METRIC = 0 point-to-point; 1 point-to-plane (pcreg_icp_batch_metric): 29 sums in a pass of their own, model normals gathered
 // there; 2 plane-to-plane (pcreg_icp_batch_gicp): the same, and the source normal of each correspondence rotated by the pose.
+// METRIC = 3 (STOP = 0 only): the covariance pass of pcreg_icp_covariance -- iters = 0, the single pass accumulates as metric 1 with
+// sum w b^2 in place of g, and the block writes a.cov (icp_cov_write) instead of updating the pose.
 // WIN = a windowed call (pcreg_icp_batch_windows, FusedWinArgs): a prologue finds the block's window; from there on the block runs
 // exactly as in a call on that window alone (its rows, ns, perm / tie_order entries and idx_out block).
 template <bool KNN, int STOP, int METRIC, bool WIN = false>
@@ -242,6 +244,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 if constexpr (METRIC == ICP_M_GICP)
                     icp_accumulate_gicp(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], a.snx[W.r0 + i], a.sny[W.r0 + i], a.snz[W.r0 + i], Ts, a.gicp_eps, px, py, pz);
                 else if constexpr (METRIC == ICP_M_PLANE) icp_accumulate_plane(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
+                else if constexpr (METRIC == ICP_M_COV) icp_accumulate_cov(s, w, d, qx, qy, qz, m, a.nrm[j >= 0 ? j : 0], px, py, pz);
                 else icp_accumulate(s, w, d, qx, qy, qz, m, px, py, pz);
             }
         }
@@ -260,7 +263,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 if (a.n_iter) a.n_iter[h] = it - s_frozen;
                 if (a.converged) a.converged[h] = s_stop && !s_frozen;
             }
-            if (!last && !s_frozen) {
+            if (METRIC != ICP_M_COV && !last && !s_frozen) {
                 if (!STOP) {
                     if (!fused_pose_update<METRIC>(s, n_used, a.pivot, a.reflection_fix != 0, Ts)) s_frozen = 1;
                 } else if constexpr (STOP == 2) {
@@ -275,6 +278,7 @@ __global__ void __launch_bounds__(UPD_THREADS, FUSED_MIN_BLOCKS) k_icp_fused(con
                 }
             }
         }
+        if constexpr (METRIC == ICP_M_COV) if (last) icp_cov_write(a.cov, s, n_used, a.pivot, h, red);
         if (timing) { const long long t = clock64(); t_svd += t - t_mark; t_mark = t; }
         __syncthreads();
         if (STOP && last) break;
@@ -311,10 +315,14 @@ size_t icp_fused_smem(int64_t ns, int mode) {
 
 template <int METRIC, bool WIN = false>
 static const void* fused_kernel(bool knn, int stop) {
-    if constexpr (METRIC == ICP_M_POINT)
-        if (stop == 2) return knn ? (const void*)k_icp_fused<true, 2, METRIC, WIN> : (const void*)k_icp_fused<false, 2, METRIC, WIN>;
-    return knn ? (stop ? (const void*)k_icp_fused<true, 1, METRIC, WIN> : (const void*)k_icp_fused<true, 0, METRIC, WIN>)
-               : (stop ? (const void*)k_icp_fused<false, 1, METRIC, WIN> : (const void*)k_icp_fused<false, 0, METRIC, WIN>);
+    if constexpr (METRIC == ICP_M_COV) {            // no stop
+        return knn ? (const void*)k_icp_fused<true, 0, METRIC, WIN> : (const void*)k_icp_fused<false, 0, METRIC, WIN>;
+    } else {
+        if constexpr (METRIC == ICP_M_POINT)
+            if (stop == 2) return knn ? (const void*)k_icp_fused<true, 2, METRIC, WIN> : (const void*)k_icp_fused<false, 2, METRIC, WIN>;
+        return knn ? (stop ? (const void*)k_icp_fused<true, 1, METRIC, WIN> : (const void*)k_icp_fused<true, 0, METRIC, WIN>)
+                   : (stop ? (const void*)k_icp_fused<false, 1, METRIC, WIN> : (const void*)k_icp_fused<false, 0, METRIC, WIN>);
+    }
 }
 
 static bool fused_fits(const void* fn, int64_t ns, int mode) {
@@ -335,7 +343,8 @@ bool icp_fused_eligible(const pcreg_model* m, int64_t ns, int64_t nhyp, const pc
     if (ns >= ((int64_t)1 << 30)) return false;
     const bool knn = o.mode == PCREG_ICP_KNN;
     const void* fn = metric == ICP_M_POINT ? (stop == 2 ? fused_kernel<ICP_M_POINT>(knn, 2) : (const void*)k_icp_fused<true, 0, ICP_M_POINT>)
-                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE>(knn, stop) : fused_kernel<ICP_M_GICP>(knn, stop);
+                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE>(knn, stop)
+                   : metric == ICP_M_GICP ? fused_kernel<ICP_M_GICP>(knn, stop) : fused_kernel<ICP_M_COV>(knn, 0);
     return fused_fits(fn, ns, o.mode);
 }
 
@@ -343,7 +352,8 @@ bool icp_fused_windows_fit(const pcreg_model* m, int64_t ns_max, const pcreg_icp
     if (!m->has_vox || o.nn != PCREG_NN_GRID || ns_max >= ((int64_t)1 << 30)) return false;
     const bool knn = o.mode == PCREG_ICP_KNN;
     const void* fn = metric == ICP_M_POINT ? fused_kernel<ICP_M_POINT, true>(knn, stop)
-                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE, true>(knn, stop) : fused_kernel<ICP_M_GICP, true>(knn, stop);
+                   : metric == ICP_M_PLANE ? fused_kernel<ICP_M_PLANE, true>(knn, stop)
+                   : metric == ICP_M_GICP ? fused_kernel<ICP_M_GICP, true>(knn, stop) : fused_kernel<ICP_M_COV, true>(knn, 0);
     return fused_fits(fn, ns_max, o.mode);
 }
 
@@ -356,23 +366,29 @@ static void fused_launch_one(const Args& a, int64_t nhyp, size_t dyn, cudaStream
 template <int METRIC, bool WIN, class Args>
 static void fused_launch_metric(const Args& a, int64_t nhyp, int stop, size_t dyn, cudaStream_t st) {
     const bool knn = a.mode == PCREG_ICP_KNN;
-    if constexpr (METRIC == ICP_M_POINT) {
-        if (stop == 2) {
-            if (knn) fused_launch_one<true, 2, METRIC, WIN>(a, nhyp, dyn, st);
-            else     fused_launch_one<false, 2, METRIC, WIN>(a, nhyp, dyn, st);
-            return;
+    if constexpr (METRIC == ICP_M_COV) {               // no stop
+        if (knn) fused_launch_one<true, 0, METRIC, WIN>(a, nhyp, dyn, st);
+        else     fused_launch_one<false, 0, METRIC, WIN>(a, nhyp, dyn, st);
+    } else {
+        if constexpr (METRIC == ICP_M_POINT) {
+            if (stop == 2) {
+                if (knn) fused_launch_one<true, 2, METRIC, WIN>(a, nhyp, dyn, st);
+                else     fused_launch_one<false, 2, METRIC, WIN>(a, nhyp, dyn, st);
+                return;
+            }
         }
+        if (knn && !stop)       fused_launch_one<true, 0, METRIC, WIN>(a, nhyp, dyn, st);
+        else if (!knn && !stop) fused_launch_one<false, 0, METRIC, WIN>(a, nhyp, dyn, st);
+        else if (knn)           fused_launch_one<true, 1, METRIC, WIN>(a, nhyp, dyn, st);
+        else                    fused_launch_one<false, 1, METRIC, WIN>(a, nhyp, dyn, st);
     }
-    if (knn && !stop)       fused_launch_one<true, 0, METRIC, WIN>(a, nhyp, dyn, st);
-    else if (!knn && !stop) fused_launch_one<false, 0, METRIC, WIN>(a, nhyp, dyn, st);
-    else if (knn)           fused_launch_one<true, 1, METRIC, WIN>(a, nhyp, dyn, st);
-    else                    fused_launch_one<false, 1, METRIC, WIN>(a, nhyp, dyn, st);
 }
 
 template <bool WIN, class Args>
 static void fused_launch(const Args& a, int64_t nhyp, int stop, cudaStream_t st) {
     const size_t dyn = icp_fused_smem(a.ns, a.mode);
-    if (a.snx)      fused_launch_metric<ICP_M_GICP, WIN>(a, nhyp, stop, dyn, st);
+    if (a.cov.cov)  fused_launch_metric<ICP_M_COV, WIN>(a, nhyp, stop, dyn, st);
+    else if (a.snx) fused_launch_metric<ICP_M_GICP, WIN>(a, nhyp, stop, dyn, st);
     else if (a.nrm) fused_launch_metric<ICP_M_PLANE, WIN>(a, nhyp, stop, dyn, st);
     else            fused_launch_metric<ICP_M_POINT, WIN>(a, nhyp, stop, dyn, st);
     PCREG_LAUNCHED();

@@ -58,6 +58,7 @@ struct FusedArgs {
     // pose extrapolation (the k_icp_fused<*, 2, 0> instantiations only): the rule, the source centroid of each window ([nwin][3]; one
     // window without WIN) and the optional [nhyp] count of extrapolated updates
     IcpExtrapRule ex; const double* ex_cen; int32_t* n_extrap;
+    IcpCovOut cov;                          // the covariance pass (the k_icp_fused<*, 0, 3> instantiations; cov.cov null otherwise)
 };
 // Windowed calls (pcreg_icp_batch_windows; the k_icp_fused<*, *, *, true> instantiations): the source arrays, w_src, the source
 // normals, perm and tie_order are the concatenation of nwin windows (column stride of sx / sy / sz: the total row count), and

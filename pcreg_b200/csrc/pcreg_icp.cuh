@@ -123,9 +123,52 @@ __device__ __forceinline__ void icp_accumulate_gicp(double (&s)[PLANE_NSUMS], do
     gicp_accumulate(s, w, d, qt, mt, nq, nm, eps);
 }
 
+// Covariance pass (pcreg_icp_covariance): the point-to-plane accumulation of A in the same order, with sum w b^2 in the first slot
+// of g (s[COV_SUM_B2]) instead of g; s[23..27] stay zero.
+__device__ __forceinline__ void icp_accumulate_cov(double (&s)[PLANE_NSUMS], double w, double d, double qx, double qy, double qz,
+                                                   const ModelPointD& m, const ModelPointD& n, double px, double py, double pz) {
+    const double q0 = qx - px, q1 = qy - py, q2 = qz - pz;
+    const double b = ((m.x - px) - q0) * n.x + ((m.y - py) - q1) * n.y + ((m.z - pz) - q2) * n.z;
+    const double a[6] = {q1 * n.z - q2 * n.y, q2 * n.x - q0 * n.z, q0 * n.y - q1 * n.x, n.x, n.y, n.z};
+    s[0] += w;
+    int k = 1;
+#pragma unroll
+    for (int r = 0; r < 6; ++r) {
+        const double wa = w * a[r];
+#pragma unroll
+        for (int c = r; c < 6; ++c) s[k++] += wa * a[c];
+    }
+    s[COV_SUM_B2] += (w * b) * b;
+    s[28] += w * d;
+}
+
+// Thread 0's part of the covariance outputs of hypothesis h; cov goes to sh[0..35] as well.  Out of line: one thread runs it.
+__device__ __noinline__ static void icp_cov_thread0(const IcpCovOut& o, const double* s, long long n_used, const double* pivot, int64_t h,
+                                                    double* sh) {
+    double cov[36];
+    const int st = pose_cov_from_sums(s, n_used, pivot, o.ref, cov, o.info ? o.info + h * 36 : nullptr, o.sigma2 + h);
+    o.status[h] = st;
+    for (int k = 0; k < 36; ++k) { o.cov[h * 36 + k] = cov[k]; sh[k] = cov[k]; }
+}
+
+// Every thread of the block, after the block reduction (s: the reduced sums, valid in every thread; sh: >= 36 doubles of free shared
+// memory): the covariance outputs of hypothesis h, then tre over the targets (thread t: targets t, t + blockDim.x, ...).
+__device__ __forceinline__ void icp_cov_write(const IcpCovOut& o, const double (&s)[PLANE_NSUMS], long long n_used, const double* pivot,
+                                              int64_t h, double* sh) {
+    if (threadIdx.x == 0) icp_cov_thread0(o, s, n_used, pivot, h, sh);
+    __syncthreads();
+    if (o.tre) {
+        for (int k = threadIdx.x; k < o.ntarget; k += blockDim.x) {
+            const double x[3] = {o.targets[k], o.targets[o.ntarget + k], o.targets[2 * (int64_t)o.ntarget + k]};
+            o.tre[h * o.ntarget + k] = pose_cov_tre(sh, o.ref, x);
+        }
+    }
+    __syncthreads();
+}
+
 // ICP metrics of the kernels' METRIC template parameter: 0 point-to-point (17 sums, Kabsch), 1 point-to-plane and 2 plane-to-plane
-// (29 sums, the LDL' step); the last sum is sum w d^2 in all of them
-constexpr int ICP_M_POINT = 0, ICP_M_PLANE = 1, ICP_M_GICP = 2;
+// (29 sums, the LDL' step), 3 the covariance pass (29 sums, no update: pcreg_icp_covariance); the last sum is sum w d^2 in all of them
+constexpr int ICP_M_POINT = 0, ICP_M_PLANE = 1, ICP_M_GICP = 2, ICP_M_COV = 3;
 template <int METRIC> constexpr int icp_nsums = METRIC != ICP_M_POINT ? PLANE_NSUMS : KABSCH_NSUMS;
 template <int METRIC>
 __device__ __forceinline__ bool icp_pose_update_m(const double (&s)[icp_nsums<METRIC>], long long n_used, const double* pivot,

@@ -253,6 +253,27 @@ struct IcpStopRule { double tol_t, tol_r_deg; int window; };
 // Pose extrapolation of the point-to-point loop (pcreg_icp_extrap; the rule is extrap_step in pcreg_math.cuh)
 struct IcpExtrapRule { double angle_deg, vmax_scale; };
 
+// Outputs of the covariance pass (pcreg_icp_covariance; the ICP_M_COV kernels, selected by cov != nullptr), indexed by the
+// hypothesis of the launch; null pointers in every other call.
+struct IcpCovOut {
+    double* cov;                // [nhyp][36] row-major, about ref
+    double* info;               // [nhyp][36] or null
+    double* sigma2;             // [nhyp]
+    int32_t* status;            // [nhyp] 1: degenerate (cov and tre NaN)
+    double* tre;                // [nhyp][ntarget] or null
+    const double* targets;      // [3][ntarget] column-major model-frame points, device
+    int32_t ntarget;
+    double ref[3];
+};
+// the same outputs from hypothesis h0 on (a chunk or a window of the launch)
+inline IcpCovOut cov_out_at(const IcpCovOut& c, int64_t h0) {
+    IcpCovOut o = c;
+    o.cov += h0 * 36; o.sigma2 += h0; o.status += h0;
+    if (o.info) o.info += h0 * 36;
+    if (o.tre) o.tre += h0 * o.ntarget;
+    return o;
+}
+
 // Select / weight / 17 sums / Kabsch / compose, one block per hypothesis.
 struct IcpUpdateArgs {
     const pcreg::ModelPointD* md;
@@ -285,6 +306,7 @@ struct IcpUpdateArgs {
     double* ex_state;           // [nhyp][EXTRAP_STATE], zero before the first pass
     const double* ex_cen;       // [3] source centroid
     int32_t* n_extrap;          // [nhyp] optional, written by the final pass
+    IcpCovOut cov;              // the covariance pass (k_icp_update<*, 0, 3>; cov.cov null otherwise)
 };
 void icp_update_launch(const IcpUpdateArgs& a, int64_t nhyp, cudaStream_t st);
 // d_seg (optional, device [nseg + 1]): one arg-min per segment of the rmse array, each relative to its segment

@@ -331,17 +331,16 @@ PCREG_HD void kabsch_from_sums(const KabschSums& s, const double* pivot_q, const
 // g = sum w a b, sum w d^2
 constexpr int PLANE_NSUMS = 29;
 
-// A x = g for a symmetric 6x6 A given by its upper triangle (row-major, 21 entries): A = L D L' without pivoting, unknowns in
-// their natural order.  Returns false (x untouched) when some pivot D_k is not above 1e-12 * max_k A_kk (a flat patch leaves a
-// direction of the pose unconstrained).
-PCREG_HD bool ldlt6_solve(const double* Au, const double* g, double* x) {
+// A = L D L' for a symmetric 6x6 A given by its upper triangle (row-major, 21 entries), without pivoting, unknowns in their
+// natural order; L: its strict lower triangle (row-major 6x6).  Returns false when some pivot D_k is not above 1e-12 * max_k A_kk
+// (a flat patch leaves a direction of the pose unconstrained).
+PCREG_HD bool ldlt6_factor(const double* Au, double* L, double* D) {
     double A[36];
     for (int r = 0, k = 0; r < 6; ++r)
         for (int c = r; c < 6; ++c, ++k) { A[r * 6 + c] = Au[k]; A[c * 6 + r] = Au[k]; }
     double amax = 0.0;
     for (int k = 0; k < 6; ++k) amax = fmax(amax, A[k * 7]);
     const double tiny = 1e-12 * amax;
-    double L[36], D[6];
     for (int j = 0; j < 6; ++j) {
         double d = A[j * 7];
         for (int k = 0; k < j; ++k) d -= L[j * 6 + k] * L[j * 6 + k] * D[k];
@@ -353,6 +352,11 @@ PCREG_HD bool ldlt6_solve(const double* Au, const double* g, double* x) {
             L[i * 6 + j] = v / d;
         }
     }
+    return true;
+}
+
+// x = L'^-1 D^-1 L^-1 g for the factors of ldlt6_factor
+PCREG_HD void ldlt6_subst(const double* L, const double* D, const double* g, double* x) {
     double y[6];
     for (int i = 0; i < 6; ++i) {
         double v = g[i];
@@ -364,7 +368,104 @@ PCREG_HD bool ldlt6_solve(const double* Au, const double* g, double* x) {
         for (int k = i + 1; k < 6; ++k) v -= L[k * 6 + i] * x[k];
         x[i] = v;
     }
+}
+
+// A x = g by ldlt6_factor.  Returns false (x untouched) when the factorisation fails.
+PCREG_HD bool ldlt6_solve(const double* Au, const double* g, double* x) {
+    double L[36], D[6];
+    if (!ldlt6_factor(Au, L, D)) return false;
+    ldlt6_subst(L, D, g, x);
     return true;
+}
+
+// ---- pose covariance of the point-to-plane objective (include/pcreg.h: pcreg_icp_covariance) ----
+// s: the 29 sums of one covariance pass -- sw, the upper triangle of A = sum w a a' (as PLANE_NSUMS), B = sum w b^2 in s[COV_SUM_B2]
+// (the first slot of g, which the pass does not need), sum w d^2 last -- about the pivot p, over n_used correspondences.  With
+// d = ref - p and M = [[I, 0], [-[d]x, I]] (row-major 6x6, unknowns (omega, tau)):
+//   sigma2 = (B / sw) n_used / (n_used - 6),  cov = sigma2 M A^-1 M' (symmetrised),  info = M^-T A M^-1.
+// info is written whenever n_used > 0 (NaN otherwise), sigma2 when n_used > 6 and sw > 0 (NaN otherwise).  Returns 1 and a NaN cov
+// when n_used <= 6, sw is not > 0 or ldlt6_factor fails, else 0.
+constexpr int COV_SUM_B2 = 22;
+PCREG_HD int pose_cov_from_sums(const double* s, long long n_used, const double* pivot, const double* ref, double* cov, double* info,
+                                double* sigma2) {
+    const double nan_v = nan("");
+    const double d[3] = {ref[0] - pivot[0], ref[1] - pivot[1], ref[2] - pivot[2]};
+    const double dx[9] = {0.0, -d[2], d[1], d[2], 0.0, -d[0], -d[1], d[0], 0.0};      // [d]x, row-major
+    double A[36];
+    for (int r = 0, k = 1; r < 6; ++r)
+        for (int c = r; c < 6; ++c, ++k) { A[r * 6 + c] = s[k]; A[c * 6 + r] = s[k]; }
+    if (info) {
+        // M^-1 = [[I, 0], [[d]x, I]]; info = (M^-1)' (A M^-1)
+        double AM[36], Mi[36];
+        for (int i = 0; i < 36; ++i) Mi[i] = 0.0;
+        for (int i = 0; i < 6; ++i) Mi[i * 7] = 1.0;
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) Mi[(3 + r) * 6 + c] = dx[r * 3 + c];
+        for (int r = 0; r < 6; ++r)
+            for (int c = 0; c < 6; ++c) {
+                double v = 0.0;
+                for (int k = 0; k < 6; ++k) v += A[r * 6 + k] * Mi[k * 6 + c];
+                AM[r * 6 + c] = v;
+            }
+        for (int r = 0; r < 6; ++r)
+            for (int c = 0; c < 6; ++c) {
+                double v = 0.0;
+                for (int k = 0; k < 6; ++k) v += Mi[k * 6 + r] * AM[k * 6 + c];
+                info[r * 6 + c] = n_used > 0 ? v : nan_v;
+            }
+    }
+    const bool noise_ok = n_used > 6 && s[0] > 0.0;
+    const double s2 = noise_ok ? (s[COV_SUM_B2] / s[0]) * ((double)n_used / (double)(n_used - 6)) : nan_v;
+    *sigma2 = s2;
+    double L[36], D[6];
+    if (!noise_ok || !ldlt6_factor(s + 1, L, D)) {
+        for (int i = 0; i < 36; ++i) cov[i] = nan_v;
+        return 1;
+    }
+    double Ai[36];                                 // A^-1, column j = ldlt6_subst(e_j)
+    for (int j = 0; j < 6; ++j) {
+        double e[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, x[6];
+        e[j] = 1.0;
+        ldlt6_subst(L, D, e, x);
+        for (int i = 0; i < 6; ++i) Ai[i * 6 + j] = x[i];
+    }
+    double M[36], MA[36];
+    for (int i = 0; i < 36; ++i) M[i] = 0.0;
+    for (int i = 0; i < 6; ++i) M[i * 7] = 1.0;
+    for (int r = 0; r < 3; ++r)
+        for (int c = 0; c < 3; ++c) M[(3 + r) * 6 + c] = -dx[r * 3 + c];
+    for (int r = 0; r < 6; ++r)
+        for (int c = 0; c < 6; ++c) {
+            double v = 0.0;
+            for (int k = 0; k < 6; ++k) v += M[r * 6 + k] * Ai[k * 6 + c];
+            MA[r * 6 + c] = v;
+        }
+    for (int r = 0; r < 6; ++r)
+        for (int c = 0; c < 6; ++c) {
+            double v = 0.0;
+            for (int k = 0; k < 6; ++k) v += MA[r * 6 + k] * M[c * 6 + k];
+            cov[r * 6 + c] = s2 * v;
+        }
+    for (int r = 0; r < 6; ++r)
+        for (int c = r + 1; c < 6; ++c) { const double v = 0.5 * (cov[r * 6 + c] + cov[c * 6 + r]); cov[r * 6 + c] = v; cov[c * 6 + r] = v; }
+    return 0;
+}
+
+// Predicted RMS displacement of the model-frame point x under cov (pose_cov_from_sums, about ref): sqrt(trace(J cov J')) with
+// J = [-[x - ref]x, I] (3 x 6), the motion x + omega x (x - ref) + tau linearised.  NaN when cov is.
+PCREG_HD double pose_cov_tre(const double* cov, const double* ref, const double* x) {
+    const double e[3] = {x[0] - ref[0], x[1] - ref[1], x[2] - ref[2]};
+    const double J[18] = {0.0, e[2], -e[1], 1.0, 0.0, 0.0,
+                          -e[2], 0.0, e[0], 0.0, 1.0, 0.0,
+                          e[1], -e[0], 0.0, 0.0, 0.0, 1.0};
+    double t = 0.0;
+    for (int r = 0; r < 3; ++r)
+        for (int i = 0; i < 6; ++i) {
+            double v = 0.0;
+            for (int j = 0; j < 6; ++j) v += cov[i * 6 + j] * J[r * 6 + j];
+            t += J[r * 6 + i] * v;
+        }
+    return sqrt(t);
 }
 
 // Rodrigues: R = I + (sin t / t) [w]x + ((1 - cos t) / t^2) [w]x^2, t = |w|; R = I at t = 0.  Column-vector convention (R v =
@@ -543,7 +644,7 @@ PCREG_HD double det_rot4(const double* T) {
 // has the handedness of its Kabsch pose.
 PCREG_HD int extrap_step(double angle_deg, double vmax_scale, const double* s, const double* p, const double* c, const double* Tc,
                          double* Tn, int u, double* st, double* trace) {
-    const double nan_v = NAN;
+    const double nan_v = nan("");
     if (!(det_rot4(Tc) > 0.0 && det_rot4(Tn) > 0.0)) {
         st[19] = 1.0;
         if (trace) { trace[0] = nan_v; trace[1] = nan_v; trace[2] = nan_v; trace[3] = 0.0; trace[4] = 0.0; }

@@ -1,4 +1,4 @@
-// pcreg_mex_util.h -- argument helpers shared by the MEX gateways (pcreg_mex.cpp, pcreg_mex_windows.cpp).
+// pcreg_mex_util.h -- argument helpers shared by the MEX gateways (pcreg_mex.cpp, pcreg_mex_windows.cpp, pcreg_mex_cov.cpp).
 #pragma once
 #include <stdint.h>
 

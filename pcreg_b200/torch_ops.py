@@ -158,3 +158,48 @@ def icp_windows_device(model: Model, src_cm: torch.Tensor, src_offsets, w_src, T
                                                 C.c_void_p(st.cuda_stream)),
             "pcreg_icp_batch_windows_dev")
     return out
+
+
+class IcpCovDeviceBuffers:
+    """Output tensors of one icp_covariance_device call: cov / info [H,36] (row-major 6x6), sigma2, rmse, n_used, status [H] and
+    tre [H,ntarget]."""
+
+    def __init__(self, nhyp: int, ntarget: int, device, want_info=False):
+        f64, i32 = torch.float64, torch.int32
+        self.cov = torch.empty((nhyp, 36), dtype=f64, device=device)
+        self.info = torch.empty((nhyp, 36), dtype=f64, device=device) if want_info else None
+        self.sigma2 = torch.empty(nhyp, dtype=f64, device=device)
+        self.rmse = torch.empty(nhyp, dtype=f64, device=device)
+        self.n_used = torch.empty(nhyp, dtype=i32, device=device)
+        self.status = torch.empty(nhyp, dtype=i32, device=device)
+        self.tre = torch.empty((nhyp, ntarget), dtype=f64, device=device) if ntarget else None
+
+
+def icp_covariance_device(model: Model, src_cm: torch.Tensor, src_offsets, w_src, T_abi: torch.Tensor, hyp_offsets, opts,
+                          out: IcpCovDeviceBuffers, ref=None, targets=None, stream=None):
+    """Run pcreg_icp_covariance_dev on tensors already resident on the library's device: the pose covariance at the poses T_abi (layout
+    of icp_windows_device).  ref (3) and targets ([K,3], model frame) are host values; out.tre must hold K columns."""
+    if not (src_cm.is_cuda and T_abi.is_cuda):
+        raise L.PcregError("icp_covariance_device needs CUDA tensors (there is no CPU fallback)")
+    assert src_cm.dtype == torch.float64 and src_cm.is_contiguous() and src_cm.shape[0] == 3
+    assert T_abi.dtype == torch.float64 and T_abi.is_contiguous()
+    soff = np.ascontiguousarray(np.asarray(src_offsets, dtype=np.int64))
+    hoff = np.ascontiguousarray(np.asarray(hyp_offsets, dtype=np.int64))
+    nwin = soff.shape[0] - 1
+    if hoff.shape[0] != nwin + 1 or soff[-1] != src_cm.shape[1] or hoff[-1] != T_abi.shape[0]:
+        raise ValueError("src_offsets / hyp_offsets must be nwin + 1 offsets ending at ns_total / the number of poses")
+    tg = np.zeros((0, 3)) if targets is None else np.asarray(targets, dtype=np.float64).reshape(-1, 3)
+    K = tg.shape[0]
+    if K and (out.tre is None or tuple(out.tre.shape) != (T_abi.shape[0], K)):
+        raise ValueError("out.tre must be [H, ntarget]")
+    tg_cm = np.asfortranarray(tg) if K else None
+    rf = None if ref is None else np.ascontiguousarray(np.asarray(ref, dtype=np.float64).reshape(3))
+    st = stream if stream is not None else torch.cuda.current_stream()
+    f64p = L.c_f64p
+    L.check(L.lib().pcreg_icp_covariance_dev(model.handle, _p(src_cm), soff.ctypes.data_as(L.c_i64p), _p(w_src), hoff.ctypes.data_as(L.c_i64p),
+                                             nwin, _p(T_abi), C.byref(opts), rf.ctypes.data_as(f64p) if rf is not None else None,
+                                             tg_cm.ctypes.data_as(f64p) if K else None, K, _p(out.cov), _p(out.info), _p(out.sigma2),
+                                             _p(out.rmse), _p(out.n_used), _p(out.status), _p(out.tre) if K else None,
+                                             C.c_void_p(st.cuda_stream)),
+            "pcreg_icp_covariance_dev")
+    return out
